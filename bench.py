@@ -9,6 +9,10 @@ so ranks share nothing (weak scaling, no data-path collective).  Rank 0 prints O
 
 `--impl reference` times the reference path's CPU form (cv2 flip/resize, OpenCV-DNN on the ONNX
 export of the same weights, numpy NMS, cv2.solvePnP) on the box's host cores.
+
+`--dump-outputs DIR` writes what the timed path returned for rank 0's frames in its last step as
+DIR/<name>.npy (float32 / float64), so that two builds can be compared output for output: the inputs
+(frames and weights) are seeded and identical from run to run.
 """
 from __future__ import annotations
 
@@ -18,6 +22,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -135,11 +140,42 @@ def make_bayer_frames_device(n: int, seed: int, device):
     return out
 
 
+_SCRATCH = None
+
+
+def scratch_path(name: str) -> str:
+    """A path in this process's temporary directory (removed at exit): weight files and the ONNX export go
+    there, never into the source tree."""
+    global _SCRATCH
+    if _SCRATCH is None:
+        _SCRATCH = tempfile.TemporaryDirectory(prefix="irmv_bench_")
+    return os.path.join(_SCRATCH.name, name)
+
+
 def weights_file(seed: int = 0) -> str:
     from irmv_detection_b200 import weights
-    path = f"/tmp/irmv_bench_seed{seed}_{os.getpid()}.irmw"
+    path = scratch_path(f"seed{seed}.irmw")
     weights.write_random(path, seed)
     return path
+
+
+def dump_outputs(out_dir: str, eng, dets, n: int) -> None:
+    """What a caller of the timed path receives for the step's n frames: detections per frame (source-pixel
+    boxes, scores, class ids; zero past counts[f], max_det slots) and the fused PnP poses of those detections."""
+    md = eng.max_det
+    counts = np.array([len(d) for d in dets], np.float32)
+    boxes, scores, classes = np.zeros((n, md, 4), np.float32), np.zeros((n, md), np.float32), np.zeros((n, md), np.float32)
+    for f, frame in enumerate(dets):
+        for i, d in enumerate(frame):
+            boxes[f, i], scores[f, i], classes[f, i] = d.xyxy, d.score, int(d.class_id)
+    rv, tv, ok = eng.fetch_poses(n)
+    valid = np.arange(md)[None, :] < counts[:, None]
+    arrays = {"counts": counts, "boxes": boxes, "scores": scores, "class_ids": classes,
+              "rvecs": np.where(valid[..., None], rv, 0.0), "tvecs": np.where(valid[..., None], tv, 0.0),
+              "pose_ok": (ok & valid).astype(np.float32)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ---------------------------------------------------------------------------------- CPU reference
@@ -509,6 +545,8 @@ def run_ours(args):
     clocks = sampler.stop()
     dets = eng.fetch(B)
     n_dets = sum(len(d) for d in dets)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, dets, B)
     if world > 1:
         torch.distributed.barrier(device_ids=[local_rank])
     step_ms_local = dev_ms / args.steps
@@ -527,7 +565,7 @@ def run_ours(args):
         hosts.append(h.numpy())
     torch.cuda.synchronize()
     eng.detect_batch_arrays(hosts[0])
-    e2e_steps = max(2, args.steps)
+    e2e_steps = args.steps
     inflight = max(1, min(3, args.inflight))
     for _ in range(3):                            # warm the pipelined path (all three result sets, copy stream)
         eng.collect_arrays(eng.submit_batch(hosts[0]), poses=True)
@@ -712,7 +750,7 @@ def kpt_variant(local_rank: int):
     from irmv_detection_b200 import synth, weights
     out = {}
     for arch in getattr(weights, "KPT_ARCHS", ("yolov8n-pose",)):
-        path = f"/tmp/irmv_bench_{arch}_{os.getpid()}.irmw"
+        path = scratch_path(f"{arch}.irmw")
         if arch == "yolov8n-pose":
             weights.write_random(path, 0, pose=True)
         else:
@@ -749,7 +787,12 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the extra_keys measurements (PnP stress, reference protocol, ...)")
     ap.add_argument("--clock-warmup-s", type=float, default=1.0, help="untimed clock ramp before the --warmup steps")
     ap.add_argument("--inflight", type=int, default=3, help="batches in flight in the end-to-end loop (1..3)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     quiet_stdout()
     try:
         if args.impl == "reference":

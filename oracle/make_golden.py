@@ -9,8 +9,10 @@
   net_golden.npz   rm_test.jpg, seed-0 weights -> top-32 scores/boxes of the FP32 oracle
   armor_golden.npz seeded light-bar scenes -> armors of the reference's extract_armors written with
                    the cv2 calls themselves (oracle/armor_ref.extract_armors_cv2)
+  npp_random_golden.npz  a seeded random 1280x1024 frame -> the reference's NPP chain (oracle/_ref/npp_ref,
+                   needs a GPU): sha256 of the 8-bit output + a crop of the FP32 output
 
-Run:  python -m oracle.make_golden
+Run:  python -m oracle.make_golden            (npp_random_golden.npz: python -m oracle.make_golden npp)
 """
 import hashlib
 import os
@@ -101,6 +103,43 @@ def armor_golden():
     np.savez_compressed(os.path.join(OUT, "armor_golden.npz"), **rec)
 
 
+NPP_RANDOM_SEED = 21
+NPP_CROP = (slice(None), slice(288, 352), slice(288, 352))
+
+
+def npp_random_frame() -> np.ndarray:
+    """The seeded random frame of tests/test_gpu_parity.py::test_preprocess_matches_reference_npp_chain."""
+    return np.random.default_rng(NPP_RANDOM_SEED).integers(0, 256, (1024, 1280, 3), dtype=np.uint8)
+
+
+def run_npp_ref(img: np.ndarray, work_dir: str) -> np.ndarray:
+    """The reference's NPP chain (oracle/_ref/npp_ref, built by oracle/Makefile) on a GPU: f32 [3, 640, 640]."""
+    import subprocess
+    exe = os.path.join(ROOT, "oracle", "_ref", "npp_ref")
+    src, dst = os.path.join(work_dir, "npp_in.raw"), os.path.join(work_dir, "npp_out.f32")
+    img.tofile(src)
+    r = subprocess.run([exe, src, str(img.shape[1]), str(img.shape[0]), dst], capture_output=True, text=True)
+    if r.returncode != 0:
+        raise RuntimeError(f"npp_ref failed: {r.stderr}")
+    return np.fromfile(dst, np.float32).reshape(3, 640, 640)
+
+
+def npp_golden(out_dir: str = OUT):
+    """The NPP chain's output for npp_random_frame(): the full output is 4.9 MB, so the sha256 of its 8-bit
+    values (which pins every pixel) and an FP32 crop are stored."""
+    import tempfile
+    with tempfile.TemporaryDirectory() as d:
+        npp = run_npp_ref(npp_random_frame(), d)
+    u8 = np.rint(npp * 255.0).astype(np.uint8)
+    np.savez_compressed(os.path.join(out_dir, "npp_random_golden.npz"),
+                        sha=np.frombuffer(hashlib.sha256(np.ascontiguousarray(u8).tobytes()).digest(), np.uint8),
+                        crop=npp[NPP_CROP].copy())
+
+
 if __name__ == "__main__":
-    main()
-    armor_golden()
+    import sys
+    if sys.argv[1:] == ["npp"]:
+        npp_golden()
+    else:
+        main()
+        armor_golden()

@@ -58,32 +58,32 @@ def test_preprocess_bayer_bit_exact(frames, chan):
         assert np.array_equal(rot[i], ref_rot)
 
 
-def test_preprocess_matches_reference_npp_chain(base_image):
-    """The reference's own NPP calls (oracle/_ref/npp_ref, run on this GPU) and the golden capture
-    of them: the CUDA kernel must reproduce their 8-bit result exactly."""
+def test_preprocess_matches_reference_npp_chain(base_image, tmp_path):
+    """The reference's own NPP calls (oracle/npp_ref.cpp) on rm_test.jpg and on a seeded random frame, as
+    captured on a B200 (tests/golden/npp_*_golden.npz, oracle/make_golden.py), and live when the harness
+    oracle/_ref/npp_ref is built: the CUDA kernel must reproduce their 8-bit result exactly."""
     import hashlib
     import os
-    import subprocess
     import irmv_detection_b200 as irmv
+    from oracle import make_golden as MG
     _cuda()
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    sha256 = lambda a: np.frombuffer(hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest(), np.uint8)
     got = irmv.preprocess(base_image[None])[0, :, :, :3].astype(np.float32).transpose(2, 0, 1)
     u8 = np.rint(got * 255.0).astype(np.uint8)
     g = np.load(os.path.join(root, "tests", "golden", "npp_rm_golden.npz"))
-    sha = np.frombuffer(hashlib.sha256(np.ascontiguousarray(u8).tobytes()).digest(), np.uint8)
     assert np.array_equal(u8[:, 288:352, 288:352], g["crop"])
-    assert np.array_equal(sha, g["sha"])
-    exe = os.path.join(root, "oracle", "_ref", "npp_ref")
-    if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/npp_ref not built")
-    rnd = np.random.default_rng(21).integers(0, 256, base_image.shape, dtype=np.uint8)
-    rnd.tofile("/tmp/_npp_in.raw")
-    r = subprocess.run([exe, "/tmp/_npp_in.raw", "1280", "1024", "/tmp/_npp_out.f32"], capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr
-    npp = np.fromfile("/tmp/_npp_out.f32", np.float32).reshape(3, 640, 640)
+    assert np.array_equal(sha256(u8), g["sha"])
+    rnd = MG.npp_random_frame()
     ours = irmv.preprocess(rnd[None])[0, :, :, :3].astype(np.float32).transpose(2, 0, 1)
-    assert np.array_equal(np.rint(ours * 255.0), np.rint(npp * 255.0))
-    assert np.abs(ours - npp).max() < 1e-3           # FP16 storage of k/255
+    g = np.load(os.path.join(root, "tests", "golden", "npp_random_golden.npz"))
+    assert np.array_equal(sha256(np.rint(ours * 255.0).astype(np.uint8)), g["sha"])
+    assert np.array_equal(np.rint(ours[MG.NPP_CROP] * 255.0), np.rint(g["crop"] * 255.0))
+    assert np.abs(ours[MG.NPP_CROP] - g["crop"]).max() < 1e-3           # FP16 storage of k/255
+    if os.path.exists(os.path.join(root, "oracle", "_ref", "npp_ref")):
+        npp = MG.run_npp_ref(rnd, str(tmp_path))
+        assert np.array_equal(np.rint(ours * 255.0), np.rint(npp * 255.0))
+        assert np.abs(ours - npp).max() < 1e-3
 
 
 def test_preprocess_odd_source_size():
