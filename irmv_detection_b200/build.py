@@ -32,6 +32,7 @@ def needs_build() -> bool:
     t = os.path.getmtime(LIB)
     deps = [os.path.join(CSRC, s) for s in SOURCES] + [
         os.path.join(CSRC, "common.cuh"),
+        os.path.join(CSRC, "result_layout.h"),
         os.path.join(os.path.dirname(HERE), "include", "irmv_cabi.h"),
     ]
     return any(os.path.getmtime(d) > t for d in deps)

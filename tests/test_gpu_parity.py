@@ -1219,6 +1219,50 @@ def test_engine_armor_stage_payload(weights_seed0):
     eng.close()
 
 
+def test_multi_replay_results_land_at_their_frames(weights_seed0, tmp_path):
+    """Every result field of a batch replayed as 2 + 2 + 1 frames on two lanes (detections, kept indices, poses,
+    armor poses, armors, keypoints) lands at the same frame offsets as from one 5-frame replay: bit-identical,
+    synchronous and pipelined."""
+    import torch
+    import irmv_detection_b200 as irmv
+    from irmv_detection_b200 import synth, weights as W
+    from oracle import armor_ref as A, pnp_ref as P, preprocess_ref as PR
+    _cuda()
+    wp = str(tmp_path / "pose_seed0.irmw")
+    W.write_random(wp, 0, pose=True)
+    scenes = [PR.rot180(A.synth_armor_scene(10, s)[0]) for s in (7, 8)]
+    fr = np.concatenate([synth.frames_from_base(synth.load_base(), 3, seed=4), np.stack(scenes)])
+    pinned = torch.from_numpy(fr).pin_memory().numpy()
+    n = len(fr)
+    same = lambda a, b: a.shape == b.shape and a.tobytes() == b.tobytes()
+    # the extractor writes a whole record where it finds an armor and only `valid` elsewhere
+    armors = lambda a: [a["valid"], a[a["valid"] != 0]]
+
+    def run(sub_batch, num_lanes):
+        eng = irmv.YoloEngine(wp, (1280, 1024), max_batch=n, sub_batch=sub_batch, num_lanes=num_lanes)
+        eng.enable_armors(binary_threshold=20, light_min_ratio=0.01, light_max_ratio=10.0, light_max_angle=90.0,
+                          min_small_center_distance=0.0, max_large_center_distance=1e9)
+        eng.enable_pnp(P.K_DEFAULT, P.D_DEFAULT, (np.float32(0.5), np.float32(480 / 1024)))
+        counts, dets = (a.copy() for a in eng.detect_batch_arrays(fr))
+        sync = {"dets": [counts, *(dets[f, :counts[f]] for f in range(n))], "kept": [eng.kept_indices(f) for f in range(n)],
+                "poses": list(eng.fetch_poses(n)), "armor_poses": [eng.fetch_armor_poses(n)],
+                "armors": armors(eng.fetch_armors(n)), "kpts": [eng.fetch_keypoints(n)]}
+        t = eng.submit_batch(pinned)
+        c, d, rv, tv, ok = (a.copy() for a in eng.collect_arrays(t, poses=True))
+        piped = {"dets": [c, *(d[f, :c[f]] for f in range(n))], "poses": [rv, tv, ok],
+                 "armor_poses": [eng.fetch_armor_poses(n, ticket=t)], "armors": armors(eng.fetch_armors(n, ticket=t)),
+                 "kpts": [eng.fetch_keypoints(n, ticket=t)]}
+        eng.close()
+        return sync, piped
+
+    (sync_a, piped_a), (sync_b, piped_b) = run(2, 2), run(n, 1)
+    assert sync_a["armor_poses"][0]["ok"].any(), "no armor was solved: the comparison would not cover the armor poses"
+    # A against B, and the pipelined results against the synchronous ones
+    for x, y in ((sync_a, sync_b), (piped_a, piped_b), (piped_a, sync_a)):
+        for key, xs in x.items():
+            assert len(xs) == len(y[key]) and all(same(a, b) for a, b in zip(xs, y[key])), key
+
+
 # ------------------------------------------------------- host-path hygiene
 def test_per_frame_calls_do_not_allocate(base_image, weights_seed0):
     """After construction and one warm call, detect(), get_rotated_image(), detect_batch(), the pipelined
