@@ -230,6 +230,16 @@ int irmv_engine_enable_armors(irmv_engine *e, const irmv_armor_params *prm);
  * pipelined batch (its ticket). */
 int irmv_engine_fetch_armors(irmv_engine *e, int ticket, int nframes, irmv_armor *out);
 
+/* Raw-domain colour stage for Bayer sources: lut = [3][256] bytes (R, G, B sites) or NULL (off, the default).
+ * Applied by every kernel that reads the raw frame: stem / preprocess, rotated view, fused armor stage.
+ * A raw sample s at sensor position (y, x) -- frame coordinates as the camera wrote them, before rot180 -- is read
+ * as lut[c][s], c = the colour of that site under the engine's pattern (both green sites use lut[1]): the engine
+ * with table L on frames F returns what it returns without a table on the frames L(F).  One table covers black
+ * level, white-balance gains and a tone curve; the caller's frames are never written.  Non-zero (irmv_last_error)
+ * for a packed RGB/BGR source or while pipelined batches are in flight.  The first non-NULL call allocates the
+ * device table, later calls rewrite it; switching between off and on drops the captured graphs. */
+int irmv_engine_set_raw_lut(irmv_engine *e, const uint8_t *lut);
+
 /* Pipelined hand-off for host-resident batches -- the B200 form of the overlap the reference gets
  * from its TripleBuffer (camera thread fills the next slot while detect() runs on the previous one,
  * reference README.md:60-63, src/irm_detector.cpp:68-72).  submit queues H2D copy (dedicated copy

@@ -86,6 +86,7 @@ SYMBOLS = {
     "irmv_extract_armors_last_profile": (C.c_int, [C.POINTER(C.c_uint64 * 8)]),
     "irmv_engine_enable_armors": (C.c_int, [_P, C.POINTER(ArmorParams)]),
     "irmv_engine_fetch_armors": (C.c_int, [_P, C.c_int, C.c_int, _P]),
+    "irmv_engine_set_raw_lut": (C.c_int, [_P, _P]),
     "irmv_engine_profile_stages": (C.c_int, [_P, _P, C.c_int, C.POINTER(C.c_float * 5)]),
     "irmv_engine_submit_batch": (C.c_int, [_P, _P, C.c_int, C.POINTER(C.c_int)]),
     "irmv_engine_collect": (C.c_int, [_P, C.c_int, _P, _P, _P, _P, _P]),

@@ -85,15 +85,25 @@ __device__ __forceinline__ int reflect101(int i, int n) {
 // buffer the reference holds (memory channel 0 takes the blue weight, whatever the channel really
 // is: src/irm_detector.cpp:310; a Bayer source is demosaiced to RGB like the vendor ISP does).
 // Branch-free, so that the loads of several pixels can be in flight together.
-template <bool BAYER>
-__device__ __forceinline__ int gray_at(const uint8_t *__restrict__ frame, int W, int H, int red_y, int red_x, int rot, int X, int Y) {
+// LUT (Bayer only): every raw sample first goes through the raw-domain colour table lut[y & 1][x & 1][s]
+// (ArmorParams::raw_lut, staged in shared memory); reflect-101 keeps a mirrored neighbour on its colour site, so
+// the neighbours of (sx, sy) use the tables of parity (sx ^ 1) and (sy ^ 1).
+template <bool BAYER, bool LUT>
+__device__ __forceinline__ int gray_at(const uint8_t *__restrict__ frame, const uint8_t *lut, int W, int H, int red_y, int red_x,
+                                       int rot, int X, int Y) {
   const int sx = rot ? W - 1 - X : X, sy = rot ? H - 1 - Y : Y;
   int c0, c1, c2;
   if (BAYER) {
     const int ym = reflect101(sy - 1, H), yp = reflect101(sy + 1, H);
     const int xm = reflect101(sx - 1, W), xp = reflect101(sx + 1, W);
     const uint8_t *r0 = frame + (size_t)ym * W, *r1 = frame + (size_t)sy * W, *r2 = frame + (size_t)yp * W;
-    const int nw = r0[xm], n = r0[sx], ne = r0[xp], w = r1[xm], c = r1[sx], e = r1[xp], sw = r2[xm], s = r2[sx], se = r2[xp];
+    int nw = r0[xm], n = r0[sx], ne = r0[xp], w = r1[xm], c = r1[sx], e = r1[xp], sw = r2[xm], s = r2[sx], se = r2[xp];
+    if (LUT) {
+      const uint8_t *tc = lut + (((sy & 1) << 9) | ((sx & 1) << 8));                       // own site
+      const uint8_t *th = tc + ((sx & 1) ? -256 : 256), *tv = tc + ((sy & 1) ? -512 : 512), *td = th + ((sy & 1) ? -512 : 512);
+      c = tc[c]; w = th[w]; e = th[e]; n = tv[n]; s = tv[s];
+      nw = td[nw]; ne = td[ne]; sw = td[sw]; se = td[se];
+    }
     const int cross = (n + s + w + e + 2) >> 2, diag = (nw + ne + sw + se + 2) >> 2;
     const int horiz = (w + e + 1) >> 1, vert = (n + s + 1) >> 1;
     const bool red_row = ((sy & 1) == red_y), red_col = ((sx & 1) == red_x);
@@ -111,8 +121,8 @@ __device__ __forceinline__ int gray_at(const uint8_t *__restrict__ frame, int W,
 // ROI -> 1-bit-per-pixel threshold bitmap, padded by one background pixel all round: a warp builds one
 // word per ballot, eight words per round with their loads issued together (clamped coordinates keep
 // the fetch branch-free).
-template <bool BAYER>
-__device__ __forceinline__ void build_bitmap(uint32_t *fg, const uint8_t *__restrict__ frame, int W, int H, int chan, int rot,
+template <bool BAYER, bool LUT>
+__device__ __forceinline__ void build_bitmap(uint32_t *fg, const uint8_t *__restrict__ frame, const uint8_t *lut, int W, int H, int chan, int rot,
                                              int rx, int ry, int rw, int rh, int wpr, int words, int thr, int warp, int lane) {
   int red_y = 0, red_x = 0;
   if (chan == 3) { red_y = 1; red_x = 1; }
@@ -127,7 +137,7 @@ __device__ __forceinline__ void build_bitmap(uint32_t *fg, const uint8_t *__rest
       const int row = w / wpr, wi = w - row * wpr;
       const int x = wi * 32 + lane - 1, y = row - 1;
       const bool in = x >= 0 && x < rw && y >= 0 && y < rh;
-      g[u] = gray_at<BAYER>(frame, W, H, red_y, red_x, rot, rx + min(max(x, 0), rw - 1), ry + min(max(y, 0), rh - 1));
+      g[u] = gray_at<BAYER, LUT>(frame, lut, W, H, red_y, red_x, rot, rx + min(max(x, 0), rw - 1), ry + min(max(y, 0), rh - 1));
       if (!in) g[u] = -1;
     }
 #pragma unroll
@@ -353,8 +363,9 @@ __device__ __forceinline__ void process_border(Shared &sh, const WarpBuf &wb, co
 
 // One detection: bitmap -> exterior flood -> border walks -> lights -> armor.  LARGE selects where
 // the per-ROI state lives, so that the small path compiles to shared-memory instructions.
-template <bool LARGE>
-__device__ __forceinline__ void roi_body(Shared &sh, const ArmorParams &p, uint32_t *slot, const uint8_t *frame, int W, int H,
+// LUT: Bayer frames go through the raw-domain colour table `lut` (shared memory)
+template <bool LARGE, bool LUT>
+__device__ __forceinline__ void roi_body(Shared &sh, const ArmorParams &p, uint32_t *slot, const uint8_t *frame, const uint8_t *lut, int W, int H,
                                          bool bayer, int rx, int ry, int rw, int rh, float min_x, float min_y, int item,
                                          ArmorOut *out, int tid, int lane, int warp) {
   const int PW = rw + 2, PH = rh + 2, wpr = (PW + 31) >> 5, words = PH * wpr;
@@ -378,8 +389,8 @@ __device__ __forceinline__ void roi_body(Shared &sh, const ArmorParams &p, uint3
   int rounds = 0;
   if (p.prof && tid == 0) t0 = clock64();
   // 1. threshold bitmap
-  if (bayer) build_bitmap<true>(fg, frame, W, H, p.chan_order, p.rotate180, rx, ry, rw, rh, wpr, words, p.binary_threshold, warp, lane);
-  else build_bitmap<false>(fg, frame, W, H, p.chan_order, p.rotate180, rx, ry, rw, rh, wpr, words, p.binary_threshold, warp, lane);
+  if (bayer) build_bitmap<true, LUT>(fg, frame, lut, W, H, p.chan_order, p.rotate180, rx, ry, rw, rh, wpr, words, p.binary_threshold, warp, lane);
+  else build_bitmap<false, false>(fg, frame, nullptr, W, H, p.chan_order, p.rotate180, rx, ry, rw, rh, wpr, words, p.binary_threshold, warp, lane);
   __syncthreads();
   if (p.prof && tid == 0) t1 = clock64();
   // 2. exterior background.  Seeds on the padding, spread along runs inside each word; then rounds of
@@ -574,10 +585,15 @@ __device__ __forceinline__ void roi_body(Shared &sh, const ArmorParams &p, uint3
   }
 }
 
+// LUT: Bayer frames with a raw-domain colour table; the table (1 KB) follows Shared in dynamic shared memory
+// and is visible after the barrier that precedes the first ROI
+template <bool LUT>
 __global__ void __launch_bounds__(kThreads, 3) extract_armors_kernel(ArmorParams p) {
   extern __shared__ __align__(16) uint8_t smem_raw[];
   Shared &sh = *reinterpret_cast<Shared *>(smem_raw);
+  uint8_t *lut = smem_raw + sizeof(Shared);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if (LUT) reinterpret_cast<uint32_t *>(lut)[tid] = reinterpret_cast<const uint32_t *>(p.raw_lut)[tid];   // kThreads == 256 words
   const int W = p.src_w, H = p.src_h;
   const bool bayer = p.chan_order >= 2;
   const size_t frame_bytes = (size_t)W * H * (bayer ? 1 : 3);
@@ -614,10 +630,10 @@ __global__ void __launch_bounds__(kThreads, 3) extract_armors_kernel(ArmorParams
     __syncthreads();
     const uint8_t *frame = base + (size_t)f * frame_bytes;
     if (large) {
-      roi_body<true>(sh, p, p.scratch + (size_t)sh.slot * p.scratch_words_per_cta, frame, W, H, bayer, rx, ry, rw, rh, min_x,
+      roi_body<true, LUT>(sh, p, p.scratch + (size_t)sh.slot * p.scratch_words_per_cta, frame, lut, W, H, bayer, rx, ry, rw, rh, min_x,
                      min_y, item, out, tid, lane, warp);
     } else {
-      roi_body<false>(sh, p, nullptr, frame, W, H, bayer, rx, ry, rw, rh, min_x, min_y, item, out, tid, lane, warp);
+      roi_body<false, LUT>(sh, p, nullptr, frame, lut, W, H, bayer, rx, ry, rw, rh, min_x, min_y, item, out, tid, lane, warp);
     }
     __syncthreads();
   }
@@ -654,16 +670,22 @@ int armors_grid(int num_sms) { return num_sms * 3; }
 size_t armors_scratch_words_per_cta(int src_w, int src_h) { return slot_words(src_w, src_h); }
 size_t armors_scratch_total_words(int src_w, int src_h, int grid) { return 64 + (size_t)grid * slot_words(src_w, src_h); }
 
+// armors_grid() runs 3 CTAs per SM: the table must leave room for them (228 KB per SM, 1 KB reserved per CTA)
+static_assert(3 * (sizeof(Shared) + 1024 + 1024) <= 228 * 1024, "raw lookup table costs the armor stage a CTA per SM");
+
 cudaError_t launch_extract_armors(const ArmorParams &p, cudaStream_t s) {
   if (p.src_h > kMaxRows - 2 || p.src_w > 32766) return cudaErrorInvalidValue;
+  if (p.raw_lut && p.chan_order < 2) return cudaErrorInvalidValue;    // the table is defined for Bayer sources only
+  auto kernel = p.raw_lut ? extract_armors_kernel<true> : extract_armors_kernel<false>;
+  const size_t smem = sizeof(Shared) + (p.raw_lut ? 1024 : 0);
   {   // per device and cheap: no process-wide "already configured" flag (several engines / devices per process)
-    cudaError_t e = cudaFuncSetAttribute(extract_armors_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Shared));
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
   }
   const int total = p.n * p.max_det;
   if (total <= 0) return cudaSuccess;
   const int grid = total < p.grid ? total : p.grid;
-  extract_armors_kernel<<<grid, kThreads, sizeof(Shared), s>>>(p);
+  kernel<<<grid, kThreads, smem, s>>>(p);
   return cudaGetLastError();
 }
 

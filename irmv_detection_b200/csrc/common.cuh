@@ -57,6 +57,9 @@ struct PreprocessParams {
   // filled by letterbox_geometry(): the resized image is new_w x new_h at (pad_x, pad_y) of the
   // 640 x 640 network input (stretch modes: 640 x 640 at (0, 0))
   int pad_x, pad_y, new_w, new_h;
+  // Raw-domain colour stage of a Bayer source (irmv_engine_set_raw_lut): [2][2][256] bytes, sample s at sensor
+  // position (y, x) reads as raw_lut[y & 1][x & 1][s] before anything else uses it; null = off
+  const uint8_t *raw_lut;
 };
 // Resize geometry of a src_w x src_h frame.  LETTERBOX (resize_mode 1) follows ultralytics'
 // LetterBox: r = min(640/w, 640/h), new = round(size * r), centred, pad value 114, pixel-centre
@@ -291,6 +294,7 @@ struct ArmorParams {
   size_t scratch_words_per_cta;         // words per slot
   int grid;
   unsigned long long *prof;             // debug: cycles summed over ROIs {bitmap, flood, walks, armor, rois, flood rounds}; null in production
+  const uint8_t *raw_lut;               // [2][2][256] raw-domain colour stage of a Bayer source (PreprocessParams::raw_lut), or null
 };
 int armors_grid(int num_sms);
 size_t armors_scratch_words_per_cta(int src_w, int src_h);

@@ -558,6 +558,8 @@ struct irmv_engine {
   bool fused_stem = true;               // preprocess + conv0 in one kernel (input never materialised)
   float *d_stem_w = nullptr, *d_stem_b = nullptr;
   uint32_t *d_stem_tab = nullptr;        // table block of the camera-case stem (stem_bayer.cu), or null
+  uint8_t *d_raw_lut = nullptr;          // [2][2][256] raw-domain colour table (irmv_engine_set_raw_lut), allocated on first use
+  bool raw_lut_on = false;               // the kernels that read the raw frame apply d_raw_lut
   PnpConsts pnp_c{};
   float net_sx = 1.f, net_sy = 1.f, net_px = 0.f, net_py = 0.f;   // network -> source pixels: (v - p) * s (parse_output)
   float pnp_sx = 1.f, pnp_sy = 1.f, pnp_px = 0.f, pnp_py = 0.f;
@@ -1035,6 +1037,7 @@ int issue_replay(irmv_engine *e, Lane &ln, int n, cudaStream_t st, int *launches
   pp.n = n; pp.src_w = e->cfg.src_width; pp.src_h = e->cfg.src_height; pp.frame0 = 0;
   pp.chan_order = e->cfg.chan_order; pp.rotate180 = e->cfg.rotate180;
   pp.resize_mode = e->cfg.resize_mode; pp.quantize_u8 = e->cfg.quantize_u8;
+  pp.raw_lut = e->raw_lut_on ? e->d_raw_lut : nullptr;
   const bool fused = e->fused_stem && e->cfg.conv_impl != IRMV_CONV_DIRECT;
   if (fused) IRMV_CUDA(launch_stem(pp, e->d_stem_w, e->d_stem_b, e->d_stem_tab, ln.stem_out.parity_only ? nullptr : ln.stem_out.p, ln.stem_out.pstride, ln.stem_out.pp, ln.stem_out.pp_stride, st));
   else IRMV_CUDA(launch_preprocess(pp, st));
@@ -1135,6 +1138,7 @@ int issue_replay(irmv_engine *e, Lane &ln, int n, cudaStream_t st, int *launches
     ap.out = ln.armors; ap.slot_locks = reinterpret_cast<int *>(ln.armor_scratch); ap.scratch = ln.armor_scratch + 64;
     ap.scratch_words_per_cta = armors_scratch_words_per_cta(e->cfg.src_width, e->cfg.src_height);
     ap.grid = armors_grid(e->num_sms);
+    ap.raw_lut = pp.raw_lut;
     IRMV_CUDA(launch_extract_armors(ap, st)); ++cnt;
     if (e->pnp_on) {
       const int total = n * e->cfg.max_det;
@@ -1299,6 +1303,7 @@ int refresh_rotated(irmv_engine *e, int slot) {
   pp.src = e->slot_dev; pp.rotated = e->rot_dev; pp.n = 1;
   pp.src_w = e->cfg.src_width; pp.src_h = e->cfg.src_height; pp.chan_order = e->cfg.chan_order;
   pp.rotate180 = e->cfg.rotate180;
+  pp.raw_lut = e->raw_lut_on ? e->d_raw_lut : nullptr;
   IRMV_CUDA(launch_rotate(pp, e->main_stream));
   IRMV_CUDA(cudaMemcpyAsync(e->rot_host[slot], e->rot_dev, (size_t)e->cfg.src_width * e->cfg.src_height * 3,
                             cudaMemcpyDeviceToHost, e->main_stream));
@@ -1634,6 +1639,7 @@ void irmv_engine_destroy(irmv_engine *e) {
   if (e->rot_dev) cudaFree(e->rot_dev);
   cudaFree(e->slot_dev);
   cudaFree(e->d_stem_w); cudaFree(e->d_stem_b); cudaFree(e->d_stem_tab);
+  if (e->d_raw_lut) cudaFree(e->d_raw_lut);
   if (e->batch_dev) cudaFree(e->batch_dev);
   for (int i = 1; i < kSets; ++i)
     if (e->sets[i].batch_dev) cudaFree(e->sets[i].batch_dev);
@@ -2019,6 +2025,43 @@ int irmv_engine_enable_armors(irmv_engine *e, const irmv_armor_params *prm) {
     ln.graphs.clear();
   }
   e->armors_on = true;
+  return 0;
+}
+
+// The caller's [3][256] table (R, G, B sites) is expanded to [2][2][256] by sensor position parity (y & 1, x & 1), so
+// the kernels never look at the pattern.  The device table is allocated once; an update rewrites it in place after
+// the engine's queued work has finished, and the graphs read it through their captured pointer.
+int irmv_engine_set_raw_lut(irmv_engine *e, const uint8_t *lut) {
+  if (!e) { set_error("bad argument"); return 1; }
+  if (e->cfg.chan_order < IRMV_CH_BAYER_RGGB || e->cfg.chan_order > IRMV_CH_BAYER_GBRG) {
+    set_error("irmv_engine_set_raw_lut: the raw lookup table applies to Bayer sources only");
+    return 2;
+  }
+  if (pipeline_busy(e)) return 5;
+  IRMV_CUDA(cudaSetDevice(e->cfg.device));
+  IRMV_CUDA(cudaDeviceSynchronize());
+  const bool on = lut != nullptr;
+  if (on) {
+    // red site (red_y, red_x), as bayer_rgb (preprocess.cu) and gray_at (armors.cu)
+    const int co = e->cfg.chan_order;
+    const int red_y = (co == IRMV_CH_BAYER_BGGR || co == IRMV_CH_BAYER_GBRG) ? 1 : 0;
+    const int red_x = (co == IRMV_CH_BAYER_BGGR || co == IRMV_CH_BAYER_GRBG) ? 1 : 0;
+    uint8_t tab[2][2][256];
+    for (int py = 0; py < 2; ++py)
+      for (int px = 0; px < 2; ++px) {
+        const int c = (py == red_y && px == red_x) ? 0 : (py != red_y && px != red_x) ? 2 : 1;
+        memcpy(tab[py][px], lut + c * 256, 256);
+      }
+    if (!e->d_raw_lut) IRMV_CUDA(dev_malloc((void **)&e->d_raw_lut, sizeof tab));
+    IRMV_CUDA(cudaMemcpy(e->d_raw_lut, tab, sizeof tab, cudaMemcpyHostToDevice));
+  }
+  if (on != e->raw_lut_on) {
+    for (auto &ln : e->lanes) {           // the kernels the replay launches changed: drop captured graphs
+      for (auto &g : ln.graphs) cudaGraphExecDestroy(g.second);
+      ln.graphs.clear();
+    }
+    e->raw_lut_on = on;
+  }
   return 0;
 }
 

@@ -57,6 +57,7 @@ struct Region {
   int src_pitch;          // bytes per source row
   int shift0, dshift;     // (address of staged row 0) & 15, and src_pitch & 15: row r starts at
                           // smem offset r*pitch_s + ((shift0 + r*dshift) & 15)
+  int nrows, nbytes;      // staged rows, needed bytes per row
 };
 
 // byte of source row `sy`, byte column `bx` (already inside the staged window)
@@ -212,11 +213,26 @@ __device__ __forceinline__ Region stage_window(const PreprocessParams &p, const 
     }
   }
   const int shift0 = (int)((size_t)(frame + (size_t)sy_lo * src_pitch + col_byte_lo) & 15);
-  return Region{frame, smem, sy_lo, pitch_s, col_byte_lo, src_pitch, shift0, src_pitch & 15};
+  return Region{frame, smem, sy_lo, pitch_s, col_byte_lo, src_pitch, shift0, src_pitch & 15, nrows, nbytes};
 }
 
 __device__ __forceinline__ void stage_wait() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
+// Raw-domain colour stage of a Bayer source (PreprocessParams::raw_lut), in place on the staged window after
+// stage_wait() + a barrier: the sample of source row sy, column sx becomes lut[sy & 1][sx & 1][sample].  The caller
+// adds a barrier before the window is read.
+__device__ __forceinline__ void apply_raw_lut(const Region &r, const uint8_t *__restrict__ lut, int nthreads) {
+  uint8_t *smem = const_cast<uint8_t *>(r.smem);
+  for (int i = threadIdx.x; i < r.nrows * r.nbytes; i += nthreads) {
+    const int rr = i / r.nbytes, k = i - rr * r.nbytes;
+    const int sy = r.row_lo + rr, sx = r.col_byte_lo + k;
+    uint8_t &b = smem[rr * r.pitch_s + ((r.shift0 + rr * r.dshift) & 15) + k];
+    b = __ldg(lut + ((sy & 1) * 2 + (sx & 1)) * 256 + b);
+  }
+}
+
+// LUT: Bayer source with a raw-domain colour table (p.raw_lut)
+template <bool LUT>
 __global__ void __launch_bounds__(NT)
 preprocess_kernel(PreprocessParams p, int rows_cap, int pitch_s) {
   extern __shared__ __align__(16) uint8_t smem[];
@@ -242,6 +258,10 @@ preprocess_kernel(PreprocessParams p, int rows_cap, int pitch_s) {
                             scale_x, scale_y, hp, NT);
   stage_wait();
   __syncthreads();
+  if (LUT) {
+    apply_raw_lut(reg, p.raw_lut, NT);
+    __syncthreads();
+  }
   (void)rows_cap;
 
   int red_y = 0, red_x = 0;
@@ -282,6 +302,7 @@ __device__ __forceinline__ float silu_fast(float x) {
   return fmaf(h, t, h);
 }
 
+template <bool LUT>
 __global__ void __launch_bounds__(ST * ST)
 stem_kernel(PreprocessParams p, const float *__restrict__ w, const float *__restrict__ bias, __half *out,
             long long out_pstride, __half *out2, long long out2_pstride, int pitch_s, int fast_x) {
@@ -322,6 +343,10 @@ stem_kernel(PreprocessParams p, const float *__restrict__ w, const float *__rest
   else if (threadIdx.x < 2 * SI) xtap[threadIdx.x - SI] = axis_taps_lb(min(max(2 * ox0 - 1 + (int)threadIdx.x - SI, 0), kNet - 1), p.pad_x, p.new_w, scale_x, W, hp);
   stage_wait();
   __syncthreads();
+  if (LUT) {
+    apply_raw_lut(reg, p.raw_lut, ST * ST);
+    __syncthreads();
+  }
   int red_y = 0, red_x = 0;
   if (p.chan_order == 3) { red_y = 1; red_x = 1; }
   else if (p.chan_order == 4) { red_y = 0; red_x = 1; }
@@ -491,6 +516,8 @@ stem_kernel(PreprocessParams p, const float *__restrict__ w, const float *__rest
 
 // Optional: materialise the rotated RGB frame (what get_rotated_image() exposes in the reference,
 // include/irmv_detection/yolo_engine.hpp:34) for consumers of the rotated source image.
+// LUT: Bayer source with a raw-domain colour table (p.raw_lut), applied to each of the nine raw reads.
+template <bool LUT>
 __global__ void rotate_kernel(PreprocessParams p) {
   const bool bayer = p.chan_order >= 2;
   const int H = p.src_h, W = p.src_w, bpp = bayer ? 1 : 3;
@@ -508,7 +535,10 @@ __global__ void rotate_kernel(PreprocessParams p) {
     if (bayer) {
       Region reg{frame, frame, 0, W, 0, W, 0, 0};
       // direct global reads: shift term must vanish, so index manually
-      auto g = [&](int yy, int xx) { return (int)frame[(size_t)yy * W + xx]; };
+      auto g = [&](int yy, int xx) {
+        const int v = frame[(size_t)yy * W + xx];
+        return LUT ? (int)__ldg(p.raw_lut + ((yy & 1) * 2 + (xx & 1)) * 256 + v) : v;
+      };
       int red_y = 0, red_x = 0;
       if (p.chan_order == 3) { red_y = 1; red_x = 1; }
       else if (p.chan_order == 4) { red_y = 0; red_x = 1; }
@@ -547,7 +577,8 @@ cudaError_t launch_rotate(const PreprocessParams &p, cudaStream_t s) {
   size_t total = (size_t)p.n * p.src_h * p.src_w;
   int blocks = (int)((total + 255) / 256);
   if (blocks > 148 * 16) blocks = 148 * 16;
-  rotate_kernel<<<blocks, 256, 0, s>>>(p);
+  if (p.raw_lut) rotate_kernel<true><<<blocks, 256, 0, s>>>(p);
+  else rotate_kernel<false><<<blocks, 256, 0, s>>>(p);
   return cudaGetLastError();
 }
 
@@ -563,23 +594,17 @@ cudaError_t launch_preprocess(const PreprocessParams &p_in, cudaStream_t s) {
   int pitch_s = ((cols_cap * bpp + 15) / 16 + 2) * 16;   // +1 chunk for the alignment shift
   size_t smem = (size_t)rows_cap * pitch_s;
   if (smem > 200 * 1024) return cudaErrorInvalidValue;
+  if (p.raw_lut && !bayer) return cudaErrorInvalidValue;       // the table is defined for Bayer sources only
+  auto kernel = p.raw_lut ? preprocess_kernel<true> : preprocess_kernel<false>;
   if (smem > 48 * 1024) {                 // per device, cheap: no process-wide flag
-    cudaError_t e = cudaFuncSetAttribute(preprocess_kernel,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
   }
   dim3 grid((kNet + TW - 1) / TW, (kNet + TH - 1) / TH, p.n);
-  preprocess_kernel<<<grid, NT, smem, s>>>(p, rows_cap, pitch_s);
+  kernel<<<grid, NT, smem, s>>>(p, rows_cap, pitch_s);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return e;
-  if (p.rotated) {
-    size_t total = (size_t)p.n * p.src_h * p.src_w;
-    int blocks = (int)((total + 255) / 256);
-    if (blocks > 148 * 16) blocks = 148 * 16;
-    rotate_kernel<<<blocks, 256, 0, s>>>(p);
-    e = cudaGetLastError();
-  }
-  return e;
+  return launch_rotate(p, s);
 }
 
 
@@ -591,16 +616,10 @@ cudaError_t launch_stem(const PreprocessParams &p_in, const float *w, const floa
   static const bool no_fast = getenv("IRMV_NO_STEM_FAST") != nullptr;
   if (!no_fast && fast_tab && stem_bayer2x_applies(p)) {
     cudaError_t e = launch_stem_bayer2x(p, p.frame0, fast_tab, out, out_pstride, out2, out2_pstride, s);
-    if (e == cudaSuccess && p.rotated) {
-      size_t total = (size_t)p.n * p.src_h * p.src_w;
-      int blocks = (int)((total + 255) / 256);
-      if (blocks > 148 * 16) blocks = 148 * 16;
-      rotate_kernel<<<blocks, 256, 0, s>>>(p);
-      e = cudaGetLastError();
-    }
-    return e;
+    return e == cudaSuccess ? launch_rotate(p, s) : e;
   }
   const bool bayer = p.chan_order >= 2;
+  if (p.raw_lut && !bayer) return cudaErrorInvalidValue;
   const int bpp = bayer ? 1 : 3;
   const float sx = (float)p.src_w / p.new_w, sy = (float)p.src_h / p.new_h;
   int rows_cap = (int)(SI * sy) + 4 + (bayer ? 4 : 0);
@@ -608,23 +627,17 @@ cudaError_t launch_stem(const PreprocessParams &p_in, const float *w, const floa
   int pitch_s = ((cols_cap * bpp + 15) / 16 + 2) * 16;
   size_t smem = (size_t)rows_cap * pitch_s;
   if (smem > 160 * 1024) return cudaErrorInvalidValue;
+  auto kernel = p.raw_lut ? stem_kernel<true> : stem_kernel<false>;
   if (smem > 30 * 1024) {
-    cudaError_t e = cudaFuncSetAttribute(stem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
   }
   dim3 grid(kNet / 2 / ST, kNet / 2 / ST, p.n);
   // integer horizontal scale without half-pixel centres: every second x tap has weight exactly 0
   const int fast_x = (p.src_w % kNet == 0) && p.resize_mode == 0;
-  stem_kernel<<<grid, ST * ST, smem, s>>>(p, w, bias, out, out_pstride, out2, out2_pstride, pitch_s, fast_x);
+  kernel<<<grid, ST * ST, smem, s>>>(p, w, bias, out, out_pstride, out2, out2_pstride, pitch_s, fast_x);
   cudaError_t e = cudaGetLastError();
-  if (e == cudaSuccess && p.rotated) {
-    size_t total = (size_t)p.n * p.src_h * p.src_w;
-    int blocks = (int)((total + 255) / 256);
-    if (blocks > 148 * 16) blocks = 148 * 16;
-    rotate_kernel<<<blocks, 256, 0, s>>>(p);
-    e = cudaGetLastError();
-  }
-  return e;
+  return e == cudaSuccess ? launch_rotate(p, s) : e;
 }
 
 }  // namespace irmv

@@ -23,6 +23,7 @@
 // (16-byte cp.async, always aligned), the tile is [2*OROWS+1][641 px][3] halves, conv0 runs as
 // mma.sync m16n8k16 with K ordered (ky, 3 px x 3 ch + 1 pad) so that every A fragment register is one
 // aligned, bank-conflict-free 32-bit shared-memory load.
+#include <cstdio>
 #include <cstring>
 #include <vector>
 
@@ -57,6 +58,7 @@ struct StemBayerArgs {
   const uint32_t *tab;                   // device tables built by stem_bayer2x_tables()
   __half *out; long long out_ps;         // normal layout (may be null)
   __half *out2; long long out2_ps;       // parity-split twin (may be null)
+  const uint8_t *raw_lut;                // [2][2][256] raw-domain colour stage (PreprocessParams::raw_lut), LUT instantiations only
 };
 
 // Device table block (built once per engine, stem_bayer2x_tables):
@@ -99,8 +101,10 @@ __device__ __forceinline__ Px3 unpack(const uint32_t *rowj) {
   return o;
 }
 
-// OUT1 / OUT2: write the normal layout / the parity-split twin (at least one of them)
-template <bool ROT, int FMT, bool OUT1, bool OUT2>
+// OUT1 / OUT2: write the normal layout / the parity-split twin (at least one of them).
+// LUT (Bayer formats only): the staged rows go through the raw-domain colour table before the demosaic; the
+// [2][2][256]-byte table sits in shared memory between the lerp table and the staged rows.
+template <bool ROT, int FMT, bool OUT1, bool OUT2, bool LUT>
 __global__ void __launch_bounds__(NTHREADS, 2) stem_bayer2x_kernel(const __grid_constant__ StemBayerArgs a) {
   constexpr int OROWS = orows_for(FMT), NIR = 2 * OROWS + 1, RP = row_pitch(FMT), STRIP_WORDS = strip_words(OROWS);
   constexpr bool PACKED = FMT >= FMT_RGB, RED_COL = FMT == FMT_BAYER_REDCOL;
@@ -108,7 +112,8 @@ __global__ void __launch_bounds__(NTHREADS, 2) stem_bayer2x_kernel(const __grid_
   extern __shared__ __align__(16) uint8_t smem[];
   uint32_t *tile_w = reinterpret_cast<uint32_t *>(smem);                       // [NIR][PITCHW]
   uint8_t *lut = smem + (size_t)NIR * PITCHW * 4;                              // [lut_n] halves
-  uint8_t *raw = smem + (((size_t)NIR * PITCHW * 4 + (size_t)a.lut_n * 2 + 15) & ~(size_t)15);   // [nr][RP]
+  uint8_t *rlut = smem + (((size_t)NIR * PITCHW * 4 + (size_t)a.lut_n * 2 + 15) & ~(size_t)15);  // [2][2][256] (LUT)
+  uint8_t *raw = rlut + (LUT ? 1024 : 0);                                                        // [nr][RP]
   __shared__ __align__(16) RowTab rowtab[NIR];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int H = a.H;
@@ -141,6 +146,7 @@ __global__ void __launch_bounds__(NTHREADS, 2) stem_bayer2x_kernel(const __grid_
     uint32_t *sl = reinterpret_cast<uint32_t *>(lut);
     for (int i = tid; i < (a.lut_n + 1) / 2; i += NTHREADS) sl[i] = gl[i];
   }
+  if (LUT && tid < 256) reinterpret_cast<uint32_t *>(rlut)[tid] = reinterpret_cast<const uint32_t *>(a.raw_lut)[tid];
   if (tid < NIR) {
     reinterpret_cast<uint4 *>(rowtab)[tid] = reinterpret_cast<const uint4 *>(strip + 4)[tid];
     // conv padding of the tile: column 0 (ix = -1) and the pad half behind the last pixel
@@ -150,6 +156,23 @@ __global__ void __launch_bounds__(NTHREADS, 2) stem_bayer2x_kernel(const __grid_
   }
   asm volatile("cp.async.wait_all;" ::: "memory");
   __syncthreads();
+  if (LUT) {
+    // raw-domain colour stage, in place: a sample of sensor row y, column x becomes rlut[y & 1][x & 1][s].  The
+    // parity is that of the row and column actually read; reflect-101 keeps a mirrored sample on its colour site
+    // (column -1 holds column 1, column SW holds column SW - 2).
+    for (int r = warp; r < nr; r += NWARPS) {
+      const uint8_t *te = rlut + (min(reflect101(vlo + r, H), H - 1) & 1) * 512, *to = te + 256;   // even / odd columns
+      uint8_t *d = raw + (size_t)r * RP + 16;
+      uint32_t *dw = reinterpret_cast<uint32_t *>(d);
+      for (int c = lane; c < SW / 4; c += 32) {
+        const uint32_t v = dw[c];
+        dw[c] = (uint32_t)te[v & 0xffu] | ((uint32_t)to[(v >> 8) & 0xffu] << 8) | ((uint32_t)te[(v >> 16) & 0xffu] << 16) |
+                ((uint32_t)to[v >> 24] << 24);
+      }
+      if (lane == 0) { d[-1] = to[d[-1]]; d[SW] = te[d[SW]]; }
+    }
+    __syncthreads();
+  }
 
   // ---- sampling: a warp owns 32 units (= 64 network-input columns) and every second input row
   {
@@ -328,20 +351,50 @@ __global__ void __launch_bounds__(NTHREADS, 2) stem_bayer2x_kernel(const __grid_
 }
 
 
-template <bool ROT, int FMT, bool OUT1, bool OUT2>
+template <bool ROT, int FMT, bool OUT1, bool OUT2, bool LUT>
 cudaError_t launch_o(const StemBayerArgs &a, size_t smem, cudaStream_t s) {
-  cudaError_t e = cudaFuncSetAttribute(stem_bayer2x_kernel<ROT, FMT, OUT1, OUT2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(stem_bayer2x_kernel<ROT, FMT, OUT1, OUT2, LUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   dim3 grid(OWID / orows_for(FMT), a.n);
-  stem_bayer2x_kernel<ROT, FMT, OUT1, OUT2><<<grid, NTHREADS, smem, s>>>(a);
+  stem_bayer2x_kernel<ROT, FMT, OUT1, OUT2, LUT><<<grid, NTHREADS, smem, s>>>(a);
   return cudaGetLastError();
+}
+
+// The table's 1 KB must not cost the kernel a CTA per SM (it is sized for two at the camera's 1024 rows, where
+// about 2.5 KB per CTA are left): refuse the launch rather than silently run at half the occupancy.
+template <bool ROT, int FMT, bool OUT1, bool OUT2>
+cudaError_t launch_lut(const StemBayerArgs &a, size_t smem, cudaStream_t s) {
+  auto on = stem_bayer2x_kernel<ROT, FMT, OUT1, OUT2, true>;
+  auto off = stem_bayer2x_kernel<ROT, FMT, OUT1, OUT2, false>;
+  cudaError_t e = cudaFuncSetAttribute(on, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem + 1024));
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(off, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  int ctas_on = 0, ctas_off = 0;
+  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_on, on, NTHREADS, smem + 1024);
+  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_off, off, NTHREADS, smem);
+  if (e != cudaSuccess) return e;
+  if (ctas_on < ctas_off) {
+    fprintf(stderr, "irmv: camera-case stem with a raw lookup table: %d CTAs per SM instead of %d (shared memory %zu B)\n",
+            ctas_on, ctas_off, smem + 1024);
+    return cudaErrorLaunchOutOfResources;
+  }
+  return launch_o<ROT, FMT, OUT1, OUT2, true>(a, smem + 1024, s);
 }
 
 template <bool ROT, int FMT>
 cudaError_t launch_t(const StemBayerArgs &a, size_t smem, cudaStream_t s) {
-  if (a.out && a.out2) return launch_o<ROT, FMT, true, true>(a, smem, s);
-  if (a.out2) return launch_o<ROT, FMT, false, true>(a, smem, s);
-  if (a.out) return launch_o<ROT, FMT, true, false>(a, smem, s);
+  if constexpr (FMT < FMT_RGB) {
+    if (a.raw_lut) {
+      if (a.out && a.out2) return launch_lut<ROT, FMT, true, true>(a, smem, s);
+      if (a.out2) return launch_lut<ROT, FMT, false, true>(a, smem, s);
+      if (a.out) return launch_lut<ROT, FMT, true, false>(a, smem, s);
+      return cudaErrorInvalidValue;
+    }
+  } else {
+    if (a.raw_lut) return cudaErrorInvalidValue;       // the table is defined for Bayer sources only
+  }
+  if (a.out && a.out2) return launch_o<ROT, FMT, true, true, false>(a, smem, s);
+  if (a.out2) return launch_o<ROT, FMT, false, true, false>(a, smem, s);
+  if (a.out) return launch_o<ROT, FMT, true, false, false>(a, smem, s);
   return cudaErrorInvalidValue;
 }
 
@@ -460,9 +513,10 @@ cudaError_t launch_stem_bayer2x(const PreprocessParams &p, int frame0, const uin
   a.Q = Q; a.lut_n = 2 * Q * 255 + Q + 1;
   a.tab_strip = TAB_LUT + (a.lut_n + 7) / 8 * 4;
   a.tab = tab; a.out = out; a.out_ps = out_ps; a.out2 = out2; a.out2_ps = out2_ps;
+  a.raw_lut = p.raw_lut;
   const size_t smem = (((size_t)(2 * orows_for(fmt) + 1) * PITCHW * 4 + (size_t)a.lut_n * 2 + 15) & ~(size_t)15) +
                       (size_t)nr_max_for(P, Q, fmt) * row_pitch(fmt);
-  if (smem > 227 * 1024) return cudaErrorInvalidValue;
+  if (smem + (p.raw_lut ? 1024 : 0) > 227 * 1024) return cudaErrorInvalidValue;
   return p.rotate180 ? launch_f<true>(fmt, a, smem, s) : launch_f<false>(fmt, a, smem, s);
 }
 

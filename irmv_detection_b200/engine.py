@@ -243,6 +243,19 @@ class YoloEngine:
         prm = armor_params(**params)
         L.check(self._lib.irmv_engine_enable_armors(self._h, C.byref(prm)), "irmv_engine_enable_armors")
 
+    def set_raw_lut(self, lut: Optional[np.ndarray]) -> None:
+        """Raw-domain colour stage of a Bayer engine: `lut` is a (3, 256) uint8 table (rows: red, green, blue
+        sites) that every raw sample goes through before the demosaic, or None to switch it off.  The engine
+        with table L on frames F returns what it returns without a table on raw_lut.apply_raw_lut(F, L)."""
+        if lut is None:
+            L.check(self._lib.irmv_engine_set_raw_lut(self._h, None), "irmv_engine_set_raw_lut")
+            return
+        lut = np.asarray(lut)
+        if lut.shape != (3, 256) or lut.dtype != np.uint8:
+            raise ValueError("set_raw_lut needs a (3, 256) uint8 table or None")
+        lut = np.ascontiguousarray(lut)
+        L.check(self._lib.irmv_engine_set_raw_lut(self._h, lut.ctypes.data), "irmv_engine_set_raw_lut")
+
     def fetch_armors(self, n: int, ticket: int = -1) -> np.ndarray:
         """Armors of the last synchronous call (or of a collected ticket): structured [n, max_det]."""
         out = np.zeros((n, self.max_det), ARMOR_DTYPE)
