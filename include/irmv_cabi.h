@@ -53,7 +53,8 @@ enum {
  * 8-bit Bayer codes :733-736, packed RGB8 / BGR8 :771-772) -> IRMV_CH_* for a raw sensor frame handed to the
  * engine instead of the vendor ISP's RGB8 output (reference src/mv_camera.cpp:64,96).  The vendor names a
  * pattern by the first two pixels of the first row: BAYRG = R G / G B = RGGB, BAYGR = GRBG, BAYGB = GBRG,
- * BAYBG = BGGR.  Returns -1 for formats the engine does not ingest (10/12/16-bit Bayer, mono, YUV, planar). */
+ * BAYBG = BGGR.  Covers the 8-bit formats: returns -1 for everything else, including the 10/12-bit Bayer formats
+ * the engine ingests through raw_format (irmv_source_format_from_media_type maps those). */
 #define IRMV_MV_MEDIA_TYPE_BAYGR8 0x01080008u
 #define IRMV_MV_MEDIA_TYPE_BAYRG8 0x01080009u
 #define IRMV_MV_MEDIA_TYPE_BAYGB8 0x0108000Au
@@ -61,6 +62,31 @@ enum {
 #define IRMV_MV_MEDIA_TYPE_RGB8 0x02180014u
 #define IRMV_MV_MEDIA_TYPE_BGR8 0x02180015u
 int irmv_chan_order_from_media_type(uint32_t mv_media_type);
+
+/* Format of the raw samples of a Bayer source (irmv_engine_config.raw_format).  Frames are row-major without line
+ * padding.  RAW_8: one byte per sample (W*H bytes, the default).  RAW_10 / RAW_12: one little-endian uint16 per
+ * sample, the value in the low 10 / 12 bits; the bits above are ignored (W*H*2 bytes).  RAW_12_PACKED: two
+ * horizontally adjacent samples in three bytes, B0 = p0[11:4], B1 = p1[3:0] << 4 | p0[3:0], B2 = p1[11:4]
+ * (W*H*3/2 bytes, W even) -- the GigE Vision "BayerXX12Packed" layout the vendor's media-type numbering follows,
+ * taken from that definition and not checked against bytes from a real camera. */
+enum { IRMV_RAW_8 = 0, IRMV_RAW_10 = 1, IRMV_RAW_12 = 2, IRMV_RAW_12_PACKED = 3 };
+/* The vendor header's MONO | occupancy | id codes of the 10-bit, 12-bit and 12-bit packed Bayer formats. */
+#define IRMV_MV_MEDIA_TYPE_BAYGR10 0x0110000Cu
+#define IRMV_MV_MEDIA_TYPE_BAYRG10 0x0110000Du
+#define IRMV_MV_MEDIA_TYPE_BAYGB10 0x0110000Eu
+#define IRMV_MV_MEDIA_TYPE_BAYBG10 0x0110000Fu
+#define IRMV_MV_MEDIA_TYPE_BAYGR12 0x01100010u
+#define IRMV_MV_MEDIA_TYPE_BAYRG12 0x01100011u
+#define IRMV_MV_MEDIA_TYPE_BAYGB12 0x01100012u
+#define IRMV_MV_MEDIA_TYPE_BAYBG12 0x01100013u
+#define IRMV_MV_MEDIA_TYPE_BAYGR12_PACKED 0x010C002Au
+#define IRMV_MV_MEDIA_TYPE_BAYRG12_PACKED 0x010C002Bu
+#define IRMV_MV_MEDIA_TYPE_BAYGB12_PACKED 0x010C002Cu
+#define IRMV_MV_MEDIA_TYPE_BAYBG12_PACKED 0x010C002Du
+/* Media type -> (IRMV_CH_*, IRMV_RAW_*) for every format the engine ingests: the 8-bit Bayer formats, RGB8 and BGR8
+ * (raw_format IRMV_RAW_8) and the 10-bit, 12-bit and 12-bit packed Bayer formats.  Returns 0 and fills both outputs,
+ * non-zero for anything else (10-bit packed, 16-bit, mono, YUV, planar). */
+int irmv_source_format_from_media_type(uint32_t mv_media_type, int32_t *chan_order, int32_t *raw_format);
 
 /* STRETCH = the reference: independent x/y scale, NPP's measured corner-aligned bilinear map
  * (src = dst * src_size/640, no half-pixel offset; pinned in tests/golden/npp_rm_golden.npz).
@@ -93,7 +119,7 @@ typedef struct irmv_engine_config {
   float score_thr;          /* 0.25 */
   float iou_thr;            /* 0.45 */
   int32_t use_graph;        /* 1 = replay captured CUDA graphs (reference behaviour) */
-  int32_t reserved[8];      /* reserved[0] != 0: run preprocess and conv0 as separate kernels (the network
+  int32_t reserved[7];      /* reserved[0] != 0: run preprocess and conv0 as separate kernels (the network
                              * input tensor is then materialised and readable as tap "input");
                              * reserved[1] != 0: do not fuse 1x1 convs into their producers (every module
                              * output is then materialised and readable through irmv_engine_read_tensor);
@@ -101,6 +127,10 @@ typedef struct irmv_engine_config {
                              * kernel per unit;
                              * reserved[3] != 0: the neck's 1x1 convs over concat(upsample(a), b) as ONE gather-kernel
                              * launch each instead of two raster-kernel launches (W_a at a's resolution + W_b) */
+  int32_t raw_format;       /* IRMV_RAW_*; anything but IRMV_RAW_8 (0, the default) needs a Bayer chan_order, and
+                             * IRMV_RAW_12_PACKED an even src_width.  A 10/12-bit engine decodes every frame into an
+                             * 8-bit mosaic through its raw table (irmv_engine_set_raw_lut) before anything else reads
+                             * it: one extra kernel per replay, counted in the preprocess stage. */
 } irmv_engine_config;
 
 /* One armor as IrmDetector::extract_armors builds it (src/irm_detector.cpp:292-355): slot i of a frame
@@ -151,7 +181,8 @@ int irmv_engine_config_default(irmv_engine_config *cfg);
 int irmv_engine_create(const char *weights_path, const irmv_engine_config *cfg, irmv_engine **out);
 void irmv_engine_destroy(irmv_engine *e);
 
-/* Borrowed, address-stable pinned-host frame slot the camera writes (src_w*src_h*channels bytes). */
+/* Borrowed, address-stable pinned-host frame slot the camera writes (one frame: src_w*src_h*3 bytes for packed RGB,
+ * otherwise the raw_format's frame size). */
 uint8_t *irmv_engine_src_buffer(irmv_engine *e, int slot);
 /* get_rotated_image() (include/irmv_detection/yolo_engine.hpp:34; the node calls it every frame,
  * src/irm_detector.cpp:183): *view = address-stable pinned buffer holding the rotated packed-RGB frame
@@ -230,14 +261,19 @@ int irmv_engine_enable_armors(irmv_engine *e, const irmv_armor_params *prm);
  * pipelined batch (its ticket). */
 int irmv_engine_fetch_armors(irmv_engine *e, int ticket, int nframes, irmv_armor *out);
 
-/* Raw-domain colour stage for Bayer sources: lut = [3][256] bytes (R, G, B sites) or NULL (off, the default).
+/* Raw-domain colour stage for Bayer sources: lut = [3][2^b] bytes (R, G, B sites) for a b-bit raw_format -- [3][256]
+ * for IRMV_RAW_8, [3][1024] for IRMV_RAW_10, [3][4096] for IRMV_RAW_12 and IRMV_RAW_12_PACKED -- or NULL.
  * Applied by every kernel that reads the raw frame: stem / preprocess, rotated view, fused armor stage.
  * A raw sample s at sensor position (y, x) -- frame coordinates as the camera wrote them, before rot180 -- is read
  * as lut[c][s], c = the colour of that site under the engine's pattern (both green sites use lut[1]): the engine
  * with table L on frames F returns what it returns without a table on the frames L(F).  One table covers black
  * level, white-balance gains and a tone curve; the caller's frames are never written.  Non-zero (irmv_last_error)
- * for a packed RGB/BGR source or while pipelined batches are in flight.  The first non-NULL call allocates the
- * device table, later calls rewrite it; switching between off and on drops the captured graphs. */
+ * for a packed RGB/BGR source or while pipelined batches are in flight.
+ * 8-bit engines: NULL = off, the default.  The first non-NULL call allocates the device table, later calls rewrite
+ * it; switching between off and on drops the captured graphs.
+ * 10/12-bit engines: the table maps a b-bit sample to the 8-bit value the rest of the pipeline sees; NULL (and the
+ * default) is the shift s >> (b - 8).  Every call rewrites the table allocated at create: no allocation, the
+ * captured graphs stay. */
 int irmv_engine_set_raw_lut(irmv_engine *e, const uint8_t *lut);
 
 /* Pipelined hand-off for host-resident batches -- the B200 form of the overlap the reference gets

@@ -16,6 +16,7 @@ NUM_ANCHORS = 8400
 CH_PASSTHROUGH, CH_SWAP_RB, CH_BAYER_RGGB, CH_BAYER_BGGR, CH_BAYER_GRBG, CH_BAYER_GBRG = range(6)
 RESIZE_STRETCH, RESIZE_LETTERBOX, RESIZE_STRETCH_HALF_PIXEL = 0, 1, 2
 CONV_TCGEN05, CONV_DIRECT = 0, 1
+RAW_8, RAW_10, RAW_12, RAW_12_PACKED = range(4)
 
 
 class Bbox(C.Structure):
@@ -46,7 +47,7 @@ class EngineConfig(C.Structure):
         ("max_batch", C.c_int32), ("sub_batch", C.c_int32), ("num_lanes", C.c_int32),
         ("num_slots", C.c_int32), ("device", C.c_int32), ("conv_impl", C.c_int32),
         ("max_det", C.c_int32), ("score_thr", C.c_float), ("iou_thr", C.c_float),
-        ("use_graph", C.c_int32), ("reserved", C.c_int32 * 8),
+        ("use_graph", C.c_int32), ("reserved", C.c_int32 * 7), ("raw_format", C.c_int32),
     ]
 
 
@@ -56,6 +57,7 @@ SYMBOLS = {
     "irmv_last_error": (C.c_char_p, []),
     "irmv_version": (C.c_int, []),
     "irmv_chan_order_from_media_type": (C.c_int, [C.c_uint32]),
+    "irmv_source_format_from_media_type": (C.c_int, [C.c_uint32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "irmv_engine_config_default": (C.c_int, [C.POINTER(EngineConfig)]),
     "irmv_engine_create": (C.c_int, [C.c_char_p, C.POINTER(EngineConfig), C.POINTER(_P)]),
     "irmv_engine_destroy": (None, [_P]),

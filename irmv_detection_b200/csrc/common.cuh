@@ -92,6 +92,21 @@ std::vector<uint32_t> stem_bayer2x_tables(const float *w, const float *bias, int
 cudaError_t launch_stem_bayer2x(const PreprocessParams &p, int frame0, const uint32_t *tab, __half *out,
                                 long long out_ps, __half *out2, long long out2_ps, cudaStream_t s);
 
+// ---------------------------------------------------------------- raw decode (raw_decode.cu)
+// 10- / 12-bit and 12-bit packed Bayer frames -> the 8-bit mosaic every other kernel reads.  Frames are row-major
+// without line padding: one little-endian u16 per sample (value in the low `bits` bits, the bits above are ignored),
+// or two samples in three bytes (packed: B0 = p0[11:4], B1 = p1[3:0] << 4 | p0[3:0], B2 = p1[11:4]).
+struct RawDecodeParams {
+  const uint8_t *src;                  // [n] frames; used when src_indirect == null; any alignment
+  const uint8_t *const *src_indirect;  // device word holding the frame base pointer (batch path)
+  uint8_t *dst;                        // [n][H][W] 8-bit mosaic, 16-byte aligned
+  const uint8_t *lut;                  // [2][2][1 << bits]: sample s at sensor position (y, x) -> lut[y & 1][x & 1][s]
+  int n, src_w, src_h;
+  int bits;                            // 10 or 12
+  int packed;                          // 1: 12-bit packed (src_w even)
+};
+cudaError_t launch_raw_decode(const RawDecodeParams &p, int num_sms, cudaStream_t s);
+
 // ---------------------------------------------------------------- convolution
 struct ConvSeg {
   const __half *ptr;    // pixel 0 of the first plane of the slice read

@@ -393,6 +393,7 @@ struct Lane {
   uint8_t *results = nullptr;              // everything a replay hands back: irmv_engine::lane_res
   DetOut det{};                            // the detection fields of `results`
   const uint8_t **src_word = nullptr;      // device word: base pointer of the frames of this replay
+  uint8_t *raw8 = nullptr;                 // [S][H][W] 8-bit mosaic decoded from 10/12-bit frames (raw_decode.cu), or null
   uint8_t *rotated = nullptr;
   std::map<int, cudaGraphExec_t> graphs;   // keyed by frames in the replay
   static constexpr int kSide = 9, kSig = 6;
@@ -560,6 +561,9 @@ struct irmv_engine {
   uint32_t *d_stem_tab = nullptr;        // table block of the camera-case stem (stem_bayer.cu), or null
   uint8_t *d_raw_lut = nullptr;          // [2][2][256] raw-domain colour table (irmv_engine_set_raw_lut), allocated on first use
   bool raw_lut_on = false;               // the kernels that read the raw frame apply d_raw_lut
+  int raw_bits = 8;                      // bits per raw sample (cfg.raw_format); > 8: every replay decodes first
+  uint8_t *d_decode_lut = nullptr;       // [2][2][1 << raw_bits] table of the decode kernel (raw_bits > 8), allocated at create
+  uint8_t *slot8_dev = nullptr;          // decoded slot_dev, what refresh_rotated rotates (raw_bits > 8)
   PnpConsts pnp_c{};
   float net_sx = 1.f, net_sy = 1.f, net_px = 0.f, net_py = 0.f;   // network -> source pixels: (v - p) * s (parse_output)
   float pnp_sx = 1.f, pnp_sy = 1.f, pnp_px = 0.f, pnp_py = 0.f;
@@ -992,6 +996,7 @@ bool build_lane(irmv_engine *e, Lane &ln) {
       !lane_alloc(ln, (void **)&ln.nms.counts, (size_t)S * 4))
     return false;
   if (!lane_alloc(ln, (void **)&ln.src_word, sizeof(void *))) return false;
+  if (e->raw_bits > 8 && !lane_alloc(ln, (void **)&ln.raw8, (size_t)S * e->cfg.src_width * e->cfg.src_height)) return false;
   const size_t slots = (size_t)S * e->cfg.max_det;
   // Everything a replay hands back lives in ONE device block per lane, laid out like the pinned result set.
   // When a replay covers the whole batch the copies back then merge into two or three cudaMemcpyAsync calls
@@ -1032,8 +1037,20 @@ int issue_replay(irmv_engine *e, Lane &ln, int n, cudaStream_t st, int *launches
     return 0;
   };
   if (mark(0)) return 1;
+  // 10/12-bit engines: the frames are decoded into the lane's 8-bit mosaic first, and every later reader of the raw
+  // frame reads that instead (counted in the preprocess stage)
+  const uint8_t *src = nullptr;
+  const uint8_t *const *src_indirect = ln.src_word;
+  if (e->raw_bits > 8) {
+    RawDecodeParams d{};
+    d.src_indirect = ln.src_word; d.dst = ln.raw8; d.lut = e->d_decode_lut;
+    d.n = n; d.src_w = e->cfg.src_width; d.src_h = e->cfg.src_height;
+    d.bits = e->raw_bits; d.packed = e->cfg.raw_format == IRMV_RAW_12_PACKED;
+    IRMV_CUDA(launch_raw_decode(d, e->num_sms, st)); ++cnt;
+    src = ln.raw8; src_indirect = nullptr;
+  }
   PreprocessParams pp{};
-  pp.src = nullptr; pp.src_indirect = ln.src_word; pp.dst = ln.in8.p; pp.rotated = ln.rotated;
+  pp.src = src; pp.src_indirect = src_indirect; pp.dst = ln.in8.p; pp.rotated = ln.rotated;
   pp.n = n; pp.src_w = e->cfg.src_width; pp.src_h = e->cfg.src_height; pp.frame0 = 0;
   pp.chan_order = e->cfg.chan_order; pp.rotate180 = e->cfg.rotate180;
   pp.resize_mode = e->cfg.resize_mode; pp.quantize_u8 = e->cfg.quantize_u8;
@@ -1124,7 +1141,7 @@ int issue_replay(irmv_engine *e, Lane &ln, int n, cudaStream_t st, int *launches
     // reference message_callback: extract_armors(get_rotated_image(), bboxes), then solvePnP per armor
     // (src/irm_detector.cpp:183,204-208)
     ArmorParams ap{};
-    ap.src = nullptr; ap.src_indirect = ln.src_word;
+    ap.src = src; ap.src_indirect = src_indirect;
     ap.n = n; ap.src_w = e->cfg.src_width; ap.src_h = e->cfg.src_height;
     ap.chan_order = e->cfg.chan_order; ap.rotate180 = e->cfg.rotate180;
     ap.num = ln.det.num_dets; ap.boxes = ln.det.boxes; ap.scores = ln.det.scores; ap.classes = ln.det.classes;
@@ -1297,10 +1314,20 @@ bool pipeline_busy(irmv_engine *e) {
   return false;
 }
 
-// Refresh the rotated frame of `slot` from the device copy of the frame (slot_dev) on the main stream.
+// Refresh the rotated frame of `slot` from the device copy of the frame (slot_dev) on the main stream.  A 10/12-bit
+// frame is decoded into slot8_dev first: the lane buffers may hold a later batch by now.
 int refresh_rotated(irmv_engine *e, int slot) {
   PreprocessParams pp{};
-  pp.src = e->slot_dev; pp.rotated = e->rot_dev; pp.n = 1;
+  pp.src = e->slot_dev;
+  if (e->raw_bits > 8) {
+    RawDecodeParams d{};
+    d.src = e->slot_dev; d.dst = e->slot8_dev; d.lut = e->d_decode_lut;
+    d.n = 1; d.src_w = e->cfg.src_width; d.src_h = e->cfg.src_height;
+    d.bits = e->raw_bits; d.packed = e->cfg.raw_format == IRMV_RAW_12_PACKED;
+    IRMV_CUDA(launch_raw_decode(d, e->num_sms, e->main_stream));
+    pp.src = e->slot8_dev;
+  }
+  pp.rotated = e->rot_dev; pp.n = 1;
   pp.src_w = e->cfg.src_width; pp.src_h = e->cfg.src_height; pp.chan_order = e->cfg.chan_order;
   pp.rotate180 = e->cfg.rotate180;
   pp.raw_lut = e->raw_lut_on ? e->d_raw_lut : nullptr;
@@ -1330,6 +1357,32 @@ int irmv_chan_order_from_media_type(uint32_t t) {
     default: return -1;
   }
 }
+
+int irmv_source_format_from_media_type(uint32_t t, int32_t *chan_order, int32_t *raw_format) {
+  if (!chan_order || !raw_format) { set_error("null argument"); return 1; }
+  int co = irmv_chan_order_from_media_type(t), rf = IRMV_RAW_8;
+  if (co < 0) {
+    switch (t) {
+      case IRMV_MV_MEDIA_TYPE_BAYRG10: co = IRMV_CH_BAYER_RGGB; rf = IRMV_RAW_10; break;
+      case IRMV_MV_MEDIA_TYPE_BAYGR10: co = IRMV_CH_BAYER_GRBG; rf = IRMV_RAW_10; break;
+      case IRMV_MV_MEDIA_TYPE_BAYGB10: co = IRMV_CH_BAYER_GBRG; rf = IRMV_RAW_10; break;
+      case IRMV_MV_MEDIA_TYPE_BAYBG10: co = IRMV_CH_BAYER_BGGR; rf = IRMV_RAW_10; break;
+      case IRMV_MV_MEDIA_TYPE_BAYRG12: co = IRMV_CH_BAYER_RGGB; rf = IRMV_RAW_12; break;
+      case IRMV_MV_MEDIA_TYPE_BAYGR12: co = IRMV_CH_BAYER_GRBG; rf = IRMV_RAW_12; break;
+      case IRMV_MV_MEDIA_TYPE_BAYGB12: co = IRMV_CH_BAYER_GBRG; rf = IRMV_RAW_12; break;
+      case IRMV_MV_MEDIA_TYPE_BAYBG12: co = IRMV_CH_BAYER_BGGR; rf = IRMV_RAW_12; break;
+      case IRMV_MV_MEDIA_TYPE_BAYRG12_PACKED: co = IRMV_CH_BAYER_RGGB; rf = IRMV_RAW_12_PACKED; break;
+      case IRMV_MV_MEDIA_TYPE_BAYGR12_PACKED: co = IRMV_CH_BAYER_GRBG; rf = IRMV_RAW_12_PACKED; break;
+      case IRMV_MV_MEDIA_TYPE_BAYGB12_PACKED: co = IRMV_CH_BAYER_GBRG; rf = IRMV_RAW_12_PACKED; break;
+      case IRMV_MV_MEDIA_TYPE_BAYBG12_PACKED: co = IRMV_CH_BAYER_BGGR; rf = IRMV_RAW_12_PACKED; break;
+      default: set_error("media type not ingested by the engine"); return 2;
+    }
+  }
+  *chan_order = co;
+  *raw_format = rf;
+  return 0;
+}
+
 int irmv_version(void) { return 100; }
 
 int irmv_engine_config_default(irmv_engine_config *c) {
@@ -1348,6 +1401,13 @@ int irmv_engine_create(const char *weights_path, const irmv_engine_config *cfg, 
   IRMV_ABI_TRY
   if (cfg->max_batch < 1 || cfg->src_width < 2 || cfg->src_height < 2 || cfg->max_det < 1 || cfg->max_det > 1024) {
     set_error("bad engine config"); return 2;
+  }
+  if (cfg->raw_format < IRMV_RAW_8 || cfg->raw_format > IRMV_RAW_12_PACKED) { set_error("unknown raw_format"); return 2; }
+  if (cfg->raw_format != IRMV_RAW_8 && (cfg->chan_order < IRMV_CH_BAYER_RGGB || cfg->chan_order > IRMV_CH_BAYER_GBRG)) {
+    set_error("raw_format other than IRMV_RAW_8 needs a Bayer chan_order"); return 2;
+  }
+  if (cfg->raw_format == IRMV_RAW_12_PACKED && (cfg->src_width & 1)) {
+    set_error("IRMV_RAW_12_PACKED needs an even src_width"); return 2;
   }
   int ndev = 0;
   IRMV_CUDA(cudaGetDeviceCount(&ndev));
@@ -1569,7 +1629,18 @@ int irmv_engine_create(const char *weights_path, const irmv_engine_config *cfg, 
   }
 
   const bool bayer = cfg->chan_order >= 2;
-  e->frame_bytes = (size_t)cfg->src_width * cfg->src_height * (bayer ? 1 : 3);
+  const size_t px = (size_t)cfg->src_width * cfg->src_height;
+  e->raw_bits = cfg->raw_format == IRMV_RAW_10 ? 10 : (cfg->raw_format == IRMV_RAW_8 ? 8 : 12);
+  e->frame_bytes = cfg->raw_format == IRMV_RAW_12_PACKED ? px / 2 * 3 : px * (e->raw_bits > 8 ? 2 : (bayer ? 1 : 3));
+  if (e->raw_bits > 8) {
+    // the decode kernel always runs with a table: the shift s >> (bits - 8) until irmv_engine_set_raw_lut
+    const size_t T = (size_t)1 << e->raw_bits;
+    std::vector<uint8_t> tab(4 * T);
+    for (size_t i = 0; i < tab.size(); ++i) tab[i] = (uint8_t)((i & (T - 1)) >> (e->raw_bits - 8));
+    IRMV_CUDA(dev_malloc((void **)&e->d_decode_lut, tab.size()));
+    IRMV_CUDA(cudaMemcpy(e->d_decode_lut, tab.data(), tab.size(), cudaMemcpyHostToDevice));
+    IRMV_CUDA(dev_malloc((void **)&e->slot8_dev, px));
+  }
   // defaults from the bench sweeps: replays of up to 256 frames (a launch carries ~7 us of fixed cost whatever
   // its size, so one 256-frame replay beats two of 128 by 3 %); two lanes when the batch needs several replays
   e->S = cfg->sub_batch > 0 ? cfg->sub_batch : (cfg->max_batch < 256 ? cfg->max_batch : 256);
@@ -1640,6 +1711,8 @@ void irmv_engine_destroy(irmv_engine *e) {
   cudaFree(e->slot_dev);
   cudaFree(e->d_stem_w); cudaFree(e->d_stem_b); cudaFree(e->d_stem_tab);
   if (e->d_raw_lut) cudaFree(e->d_raw_lut);
+  if (e->d_decode_lut) cudaFree(e->d_decode_lut);
+  if (e->slot8_dev) cudaFree(e->slot8_dev);
   if (e->batch_dev) cudaFree(e->batch_dev);
   for (int i = 1; i < kSets; ++i)
     if (e->sets[i].batch_dev) cudaFree(e->sets[i].batch_dev);
@@ -2028,9 +2101,10 @@ int irmv_engine_enable_armors(irmv_engine *e, const irmv_armor_params *prm) {
   return 0;
 }
 
-// The caller's [3][256] table (R, G, B sites) is expanded to [2][2][256] by sensor position parity (y & 1, x & 1), so
-// the kernels never look at the pattern.  The device table is allocated once; an update rewrites it in place after
-// the engine's queued work has finished, and the graphs read it through their captured pointer.
+// The caller's [3][T] table (R, G, B sites; T = 2^bits) is expanded to [2][2][T] by sensor position parity (y & 1,
+// x & 1), so the kernels never look at the pattern.  The device table is allocated once (at create for 10/12-bit
+// engines); an update rewrites it in place after the engine's queued work has finished, and the graphs read it
+// through their captured pointer.
 int irmv_engine_set_raw_lut(irmv_engine *e, const uint8_t *lut) {
   if (!e) { set_error("bad argument"); return 1; }
   if (e->cfg.chan_order < IRMV_CH_BAYER_RGGB || e->cfg.chan_order > IRMV_CH_BAYER_GBRG) {
@@ -2041,19 +2115,26 @@ int irmv_engine_set_raw_lut(irmv_engine *e, const uint8_t *lut) {
   IRMV_CUDA(cudaSetDevice(e->cfg.device));
   IRMV_CUDA(cudaDeviceSynchronize());
   const bool on = lut != nullptr;
+  const size_t T = (size_t)1 << e->raw_bits;       // table entries per site: 256, 1024 or 4096
+  // red site (red_y, red_x), as bayer_rgb (preprocess.cu) and gray_at (armors.cu)
+  const int co = e->cfg.chan_order;
+  const int red_y = (co == IRMV_CH_BAYER_BGGR || co == IRMV_CH_BAYER_GBRG) ? 1 : 0;
+  const int red_x = (co == IRMV_CH_BAYER_BGGR || co == IRMV_CH_BAYER_GRBG) ? 1 : 0;
+  std::vector<uint8_t> tab(4 * T);
+  for (int py = 0; py < 2; ++py)
+    for (int px = 0; px < 2; ++px) {
+      const int c = (py == red_y && px == red_x) ? 0 : (py != red_y && px != red_x) ? 2 : 1;
+      uint8_t *dst = tab.data() + (py * 2 + px) * T;
+      if (on) memcpy(dst, lut + c * T, T);
+      else for (size_t s = 0; s < T; ++s) dst[s] = (uint8_t)(s >> (e->raw_bits - 8));
+    }
+  if (e->raw_bits > 8) {    // the decode kernel applies the table; its graphs keep reading the same device table
+    IRMV_CUDA(cudaMemcpy(e->d_decode_lut, tab.data(), tab.size(), cudaMemcpyHostToDevice));
+    return 0;
+  }
   if (on) {
-    // red site (red_y, red_x), as bayer_rgb (preprocess.cu) and gray_at (armors.cu)
-    const int co = e->cfg.chan_order;
-    const int red_y = (co == IRMV_CH_BAYER_BGGR || co == IRMV_CH_BAYER_GBRG) ? 1 : 0;
-    const int red_x = (co == IRMV_CH_BAYER_BGGR || co == IRMV_CH_BAYER_GRBG) ? 1 : 0;
-    uint8_t tab[2][2][256];
-    for (int py = 0; py < 2; ++py)
-      for (int px = 0; px < 2; ++px) {
-        const int c = (py == red_y && px == red_x) ? 0 : (py != red_y && px != red_x) ? 2 : 1;
-        memcpy(tab[py][px], lut + c * 256, 256);
-      }
-    if (!e->d_raw_lut) IRMV_CUDA(dev_malloc((void **)&e->d_raw_lut, sizeof tab));
-    IRMV_CUDA(cudaMemcpy(e->d_raw_lut, tab, sizeof tab, cudaMemcpyHostToDevice));
+    if (!e->d_raw_lut) IRMV_CUDA(dev_malloc((void **)&e->d_raw_lut, tab.size()));
+    IRMV_CUDA(cudaMemcpy(e->d_raw_lut, tab.data(), tab.size(), cudaMemcpyHostToDevice));
   }
   if (on != e->raw_lut_on) {
     for (auto &ln : e->lanes) {           // the kernels the replay launches changed: drop captured graphs

@@ -53,7 +53,7 @@ class YoloEngine:
                  sub_batch: int = 0, num_lanes: int = 0, num_slots: int = 3, device: int = 0,
                  conv_impl: int = L.CONV_TCGEN05, score_thr: float = 0.25, iou_thr: float = 0.45,
                  max_det: int = 100, use_graph: bool = True, fused_stem: bool = True, fuse_tails: bool = True,
-                 fuse_units: bool = True, split_upsample_convs: bool = True):
+                 fuse_units: bool = True, split_upsample_convs: bool = True, raw_format: int = L.RAW_8):
         lib = L.lib()
         wpath = onnx_file_path if onnx_file_path.endswith(".irmw") else weights_path_for(onnx_file_path)
         if not os.path.exists(wpath):
@@ -75,6 +75,7 @@ class YoloEngine:
         cfg.reserved[1] = 0 if fuse_tails else 1
         cfg.reserved[2] = 0 if fuse_units else 1          # ShuffleNetV2 variant: one kernel per unit (default) or one per conv
         cfg.reserved[3] = 0 if split_upsample_convs else 1   # neck cv1 over concat(upsample(a), b): two raster launches or one gather launch
+        cfg.raw_format = raw_format
         self._cfg = cfg
         self._h = C.c_void_p()
         self._lib = lib
@@ -82,7 +83,17 @@ class YoloEngine:
         self.src_image_size = (cfg.src_width, cfg.src_height)
         self.enable_profiling = enable_profiling
         self.channels = 1 if chan_order >= L.CH_BAYER_RGGB else 3
-        self.frame_bytes = cfg.src_width * cfg.src_height * self.channels
+        self.raw_format = raw_format
+        W, H = cfg.src_width, cfg.src_height
+        # one frame as the engine takes it: dtype and shape (RAW_8: [H, W] Bayer or [H, W, 3] packed RGB)
+        if raw_format in (L.RAW_10, L.RAW_12):
+            self.frame_dtype, self.frame_shape = np.dtype(np.uint16), (H, W)
+        elif raw_format == L.RAW_12_PACKED:
+            self.frame_dtype, self.frame_shape = np.dtype(np.uint8), (H, W * 3 // 2)
+        else:
+            self.frame_dtype, self.frame_shape = np.dtype(np.uint8), (H, W) + ((3,) if self.channels == 3 else ())
+        self.raw_bits = {L.RAW_10: 10, L.RAW_12: 12, L.RAW_12_PACKED: 12}.get(raw_format, 8)
+        self.frame_bytes = int(np.prod(self.frame_shape)) * self.frame_dtype.itemsize
         self.max_batch, self.max_det = max_batch, max_det
         self._slot = 0
         self._out = (L.Bbox * (max_batch * max_det))()
@@ -91,13 +102,13 @@ class YoloEngine:
 
     # -- reference surface ---------------------------------------------------------------
     def get_src_image_buffer(self, slot: int = 0) -> np.ndarray:
-        """Pinned-host frame slot as a writable numpy view (reference returns uint8_t*)."""
+        """Pinned-host frame slot as a writable numpy view (reference returns uint8_t*): u8 [H, W, 3] or [H, W] for
+        8-bit sources, u16 [H, W] for RAW_10 / RAW_12, u8 [H, 3W/2] for RAW_12_PACKED."""
         p = self._lib.irmv_engine_src_buffer(self._h, slot)
         if not p:
             raise L.IrmvError("bad slot")
         buf = (C.c_uint8 * self.frame_bytes).from_address(p)
-        shape = (self.src_image_size[1], self.src_image_size[0]) + ((3,) if self.channels == 3 else ())
-        return np.frombuffer(buf, np.uint8).reshape(shape)
+        return np.frombuffer(buf, self.frame_dtype).reshape(self.frame_shape)
 
     def detect(self, slot: int = 0) -> List[bbox]:
         n = C.c_int(0)
@@ -126,10 +137,14 @@ class YoloEngine:
 
     # -- batch extension -----------------------------------------------------------------
     def detect_batch(self, frames: np.ndarray) -> List[List[bbox]]:
-        """frames u8 [n,H,W,3] (or [n,H,W] Bayer) in host memory."""
-        frames = np.ascontiguousarray(frames, np.uint8)
+        """frames u8 [n,H,W,3] (or [n,H,W] Bayer) in host memory; 10/12-bit engines: [n] frames of exactly
+        get_src_image_buffer()'s dtype and shape."""
+        if self.raw_format != L.RAW_8:
+            frames = self._raw_frames(frames)
+        else:
+            frames = np.ascontiguousarray(frames, np.uint8)
         n = frames.shape[0]
-        if frames[0].size != self.frame_bytes:
+        if frames[0].size != self.frame_bytes // self.frame_dtype.itemsize:
             raise ValueError("frame size does not match the engine's src_image_size")
         L.check(self._lib.irmv_engine_detect_batch(self._h, frames.ctypes.data, 0, n, self._out, self._counts),
                 "irmv_engine_detect_batch")
@@ -138,7 +153,7 @@ class YoloEngine:
     def detect_batch_arrays(self, frames: np.ndarray):
         """Same call as detect_batch, results as arrays (no per-detection Python objects):
         counts i32[n] and a structured view {xyxy f32[4], score f32, class_id i32}[n, max_det]."""
-        frames = np.ascontiguousarray(frames, np.uint8)
+        frames = self._raw_frames(frames) if self.raw_format != L.RAW_8 else np.ascontiguousarray(frames, np.uint8)
         n = frames.shape[0]
         L.check(self._lib.irmv_engine_detect_batch(self._h, frames.ctypes.data, 0, n, self._out, self._counts),
                 "irmv_engine_detect_batch")
@@ -151,15 +166,31 @@ class YoloEngine:
         """Queue H2D + pipeline + D2H for host frames and return a ticket; at most three batches in
         flight, collect in order.  `frames` must stay alive and unchanged until collected (pinned
         memory makes the copy asynchronous)."""
-        if not frames.flags.c_contiguous or frames.dtype != np.uint8:
+        if self.raw_format != L.RAW_8:
+            frames = self._raw_frames(frames, copy=False)
+        elif not frames.flags.c_contiguous or frames.dtype != np.uint8:
             raise ValueError("submit_batch needs a C-contiguous uint8 array")
         n = frames.shape[0]
-        if frames[0].size != self.frame_bytes:
+        if frames[0].size != self.frame_bytes // self.frame_dtype.itemsize:
             raise ValueError("frame size does not match the engine's src_image_size")
         t = C.c_int(0)
         L.check(self._lib.irmv_engine_submit_batch(self._h, frames.ctypes.data, n, C.byref(t)), "irmv_engine_submit_batch")
         self._ticket_n[t.value % 3] = n
         return t.value
+
+    def _raw_frames(self, frames: np.ndarray, copy: bool = True) -> np.ndarray:
+        """Host frames of a 10/12-bit engine: exactly [n] + frame_shape of frame_dtype, never cast (a cast would
+        truncate or reinterpret the samples).  copy=False: they must already be C-contiguous."""
+        frames = np.asarray(frames)
+        if frames.dtype != self.frame_dtype or frames.ndim != 1 + len(self.frame_shape) or \
+                tuple(frames.shape[1:]) != self.frame_shape or frames.shape[0] < 1:
+            raise ValueError(f"this engine takes {self.frame_dtype.name} frames of shape [n, "
+                             f"{', '.join(map(str, self.frame_shape))}], got {frames.dtype.name} {list(frames.shape)}")
+        if not frames.flags.c_contiguous:
+            if not copy:
+                raise ValueError("submit_batch needs a C-contiguous array")
+            frames = np.ascontiguousarray(frames)
+        return frames
 
     def collect_arrays(self, ticket: int, poses: bool = False):
         """Wait for a submitted batch: (counts i32[n], dets structured [n, max_det]) and, with
@@ -244,15 +275,18 @@ class YoloEngine:
         L.check(self._lib.irmv_engine_enable_armors(self._h, C.byref(prm)), "irmv_engine_enable_armors")
 
     def set_raw_lut(self, lut: Optional[np.ndarray]) -> None:
-        """Raw-domain colour stage of a Bayer engine: `lut` is a (3, 256) uint8 table (rows: red, green, blue
-        sites) that every raw sample goes through before the demosaic, or None to switch it off.  The engine
-        with table L on frames F returns what it returns without a table on raw_lut.apply_raw_lut(F, L)."""
+        """Raw-domain colour stage of a Bayer engine: `lut` is a (3, 2^b) uint8 table (rows: red, green, blue
+        sites; b = 8, 10 or 12 bits per raw sample) that every raw sample goes through before the demosaic, or None.
+        8-bit engines: None switches the table off, and the engine with table L on frames F returns what it returns
+        without a table on raw_lut.apply_raw_lut(F, L).  10/12-bit engines: None restores the default shift
+        s >> (b - 8); the engine returns what an 8-bit engine without a table returns on raw_lut.decode_raw(F, ...)."""
         if lut is None:
             L.check(self._lib.irmv_engine_set_raw_lut(self._h, None), "irmv_engine_set_raw_lut")
             return
         lut = np.asarray(lut)
-        if lut.shape != (3, 256) or lut.dtype != np.uint8:
-            raise ValueError("set_raw_lut needs a (3, 256) uint8 table or None")
+        n = 1 << self.raw_bits
+        if lut.shape != (3, n) or lut.dtype != np.uint8:
+            raise ValueError(f"set_raw_lut needs a (3, {n}) uint8 table or None")
         lut = np.ascontiguousarray(lut)
         L.check(self._lib.irmv_engine_set_raw_lut(self._h, lut.ctypes.data), "irmv_engine_set_raw_lut")
 

@@ -4,10 +4,14 @@ apply_raw_lut is the definition the engine's kernels are checked against: the en
 frames F returns, bit for bit, what it returns without a table on apply_raw_lut(F, L, pattern).
 make_raw_lut builds such a table from the black level, white-balance gains and gamma a caller would set
 on the camera's ISP.
+
+decode_raw is the same definition for 10- and 12-bit sources (raw_format RAW_10, RAW_12, RAW_12_PACKED): a b-bit
+engine with table T on frames F returns, bit for bit, what an otherwise identical 8-bit engine without a table
+returns on decode_raw(F, raw_format, T, pattern).
 """
 from __future__ import annotations
 
-from typing import Sequence
+from typing import Optional, Sequence
 
 import numpy as np
 
@@ -27,23 +31,79 @@ def site_colours(h: int, w: int, pattern: int) -> np.ndarray:
     return np.where(red, 0, np.where(blue, 2, 1)).astype(np.uint8)
 
 
+RAW_BITS = {L.RAW_8: 8, L.RAW_10: 10, L.RAW_12: 12, L.RAW_12_PACKED: 12}
+
+
 def apply_raw_lut(raw: np.ndarray, lut: np.ndarray, pattern: int) -> np.ndarray:
-    """raw u8 [..., H, W] Bayer mosaic(s) as the camera wrote them (before rot180), lut u8 [3, 256]:
-    sample s at sensor position (y, x) becomes lut[colour of (y, x)][s].  Returns a new array."""
-    raw = np.asarray(raw, np.uint8)
+    """raw [..., H, W] Bayer mosaic(s) as the camera wrote them (before rot180), lut u8 [3, 2^b] (b = 8, 10, 12):
+    sample s at sensor position (y, x) becomes lut[colour of (y, x)][s & (2^b - 1)].  With a (3, 256) table raw is
+    taken as u8; wider tables take unsigned integer samples (u16).  Returns a new u8 array."""
     lut = np.asarray(lut, np.uint8)
-    if lut.shape != (3, 256):
-        raise ValueError("lut must be (3, 256) uint8")
+    if lut.shape == (3, 256):
+        raw = np.asarray(raw, np.uint8)
+    elif lut.shape in ((3, 1 << 10), (3, 1 << 12)):
+        raw = np.asarray(raw)
+        if raw.dtype.kind != "u":
+            raise ValueError("samples for a 10/12-bit table must be unsigned integers")
+        raw = raw & np.asarray(lut.shape[1] - 1, raw.dtype)
+    else:
+        raise ValueError("lut must be (3, 256), (3, 1024) or (3, 4096) uint8")
     c = site_colours(raw.shape[-2], raw.shape[-1], pattern)
     return lut[c, raw]
 
 
-def make_raw_lut(black_level: int = 0, gains: Sequence[float] = (1.0, 1.0, 1.0), gamma: float = 1.0) -> np.ndarray:
-    """u8 [3, 256] table of the usual ISP chain per colour site: subtract the black level, rescale to the
-    full range, apply the channel's white-balance gain, clip, apply the tone curve x ** gamma, round half up."""
-    v = np.arange(256, dtype=np.float64)
-    x = np.clip(v - black_level, 0.0, None) / (255.0 - black_level)
-    out = np.empty((3, 256), np.uint8)
+def unpack_raw12_packed(packed: np.ndarray) -> np.ndarray:
+    """u8 [..., H, 3W/2] 12-bit packed rows -> u16 [..., H, W].  Two horizontally adjacent samples p0, p1 in three
+    bytes (GigE Vision BayerXX12Packed): B0 = p0[11:4], B1 = p1[3:0] << 4 | p0[3:0], B2 = p1[11:4]."""
+    packed = np.asarray(packed, np.uint8)
+    if packed.shape[-1] % 3:
+        raise ValueError("a 12-bit packed row holds a multiple of 3 bytes")
+    b = packed.reshape(packed.shape[:-1] + (-1, 3)).astype(np.uint16)
+    p0 = b[..., 0] << 4 | (b[..., 1] & 15)
+    p1 = b[..., 2] << 4 | b[..., 1] >> 4
+    return np.stack([p0, p1], -1).reshape(packed.shape[:-1] + (-1,))
+
+
+def pack_raw12_packed(raw: np.ndarray) -> np.ndarray:
+    """u16 [..., H, W] (W even; the low 12 bits of each sample) -> u8 [..., H, 3W/2], the inverse of
+    unpack_raw12_packed."""
+    raw = np.asarray(raw)
+    if raw.shape[-1] % 2:
+        raise ValueError("12-bit packed rows need an even width")
+    s = (raw.astype(np.uint16) & 0xFFF).reshape(raw.shape[:-1] + (-1, 2))
+    p0, p1 = s[..., 0], s[..., 1]
+    out = np.stack([p0 >> 4, (p1 & 15) << 4 | (p0 & 15), p1 >> 4], -1).astype(np.uint8)
+    return out.reshape(raw.shape[:-1] + (-1,))
+
+
+def default_raw_lut(bits: int) -> np.ndarray:
+    """u8 [3, 2^bits]: the table a b-bit engine runs with until set_raw_lut, s -> s >> (bits - 8)."""
+    return np.tile((np.arange(1 << bits) >> (bits - 8)).astype(np.uint8), (3, 1))
+
+
+def decode_raw(frames: np.ndarray, raw_format: int, lut: Optional[np.ndarray], pattern: int) -> np.ndarray:
+    """Frames as a raw_format engine takes them (u16 [..., H, W] for RAW_10 / RAW_12, u8 [..., H, 3W/2] for
+    RAW_12_PACKED) -> the u8 [..., H, W] mosaics an 8-bit engine without a table must see: unpack, mask each sample
+    to b bits, map it through lut[colour of its sensor site] (lut None: default_raw_lut(b))."""
+    bits = RAW_BITS[raw_format]
+    if bits == 8:
+        raise ValueError("decode_raw takes 10/12-bit formats; 8-bit frames go through apply_raw_lut")
+    raw = unpack_raw12_packed(frames) if raw_format == L.RAW_12_PACKED else np.asarray(frames, np.uint16)
+    lut = default_raw_lut(bits) if lut is None else np.asarray(lut, np.uint8)
+    if lut.shape != (3, 1 << bits):
+        raise ValueError(f"a {bits}-bit format takes a (3, {1 << bits}) table")
+    return apply_raw_lut(raw, lut, pattern)
+
+
+def make_raw_lut(black_level: int = 0, gains: Sequence[float] = (1.0, 1.0, 1.0), gamma: float = 1.0,
+                 bits: int = 8) -> np.ndarray:
+    """u8 [3, 2^bits] table of the usual ISP chain per colour site, from bits-bit samples to 8-bit values: subtract
+    the black level (in units of that bit depth), rescale to the full range 2^bits - 1 - black, apply the channel's
+    white-balance gain, clip, apply the tone curve x ** gamma, round half up."""
+    top = (1 << bits) - 1
+    v = np.arange(top + 1, dtype=np.float64)
+    x = np.clip(v - black_level, 0.0, None) / (float(top) - black_level)
+    out = np.empty((3, top + 1), np.uint8)
     for c in range(3):
         y = np.clip(x * float(gains[c]), 0.0, 1.0) ** float(gamma)
         out[c] = np.floor(y * 255.0 + 0.5).astype(np.uint8)
