@@ -199,6 +199,9 @@ long long irmv_debug_alloc_count(void);
  * kernel relies on that padding staying zero.  Counts the padding pixels of all activation tensors of the engine that
  * are not zero: 0 after any sequence of calls, anything else is a stray store (the memory check this pool allows). */
 int irmv_debug_check_padding(irmv_engine *e, long long *bad_pixels);
+/* Debug: CTAs per SM of the camera-case stem kernel as the engine launches it now (with its raw table when one is
+ * set), or 0 when its frames go to the generic stem kernel instead. */
+int irmv_debug_stem_ctas(irmv_engine *e, int *ctas);
 
 /* One frame from pinned slot `slot`: H2D + graph(preprocess, net, decode, NMS) + D2H + parse. */
 int irmv_engine_detect(irmv_engine *e, int slot, irmv_bbox *out, int cap, int *n);

@@ -66,6 +66,7 @@ SYMBOLS = {
     "irmv_engine_rotated_view": (C.c_int, [_P, C.c_int, C.POINTER(_P)]),
     "irmv_debug_alloc_count": (C.c_longlong, []),
     "irmv_debug_check_padding": (C.c_int, [C.c_void_p, C.POINTER(C.c_longlong)]),
+    "irmv_debug_stem_ctas": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "irmv_engine_fetch_armor_poses": (C.c_int, [_P, C.c_int, C.c_int, _P]),
     "irmv_engine_detect": (C.c_int, [_P, C.c_int, C.POINTER(Bbox), C.c_int, C.POINTER(C.c_int)]),
     "irmv_engine_detect_batch": (C.c_int, [_P, _P, C.c_int, C.c_int, C.POINTER(Bbox), C.POINTER(C.c_int)]),

@@ -85,8 +85,11 @@ cudaError_t launch_rotate(const PreprocessParams &p, cudaStream_t s);
 // fast_tab: device table block of stem_bayer2x_tables() (null: always the generic kernel).
 cudaError_t launch_stem(const PreprocessParams &p, const float *w, const float *bias, const uint32_t *fast_tab, __half *out,
                         long long out_pstride, __half *out2, long long out2_pstride, cudaStream_t s);
-// Camera-case stem (stem_bayer.cu): Bayer source of width 1280, reference resize, 8-bit intermediate.
+// Camera-case stem (stem_bayer.cu): Bayer or packed source of width 1280, reference resize, 8-bit intermediate,
+// shared memory within a block's limit; with p.raw_lut, only where the table keeps the CTAs per SM.
 bool stem_bayer2x_applies(const PreprocessParams &p);
+// CTAs per SM of the camera-case kernel for p (with its raw table if p.raw_lut), 0 where it does not apply
+int stem_bayer2x_ctas(const PreprocessParams &p);
 // w [16][9 taps][3], bias [16]; the tables depend on the source height, the Bayer pattern and the rotation
 std::vector<uint32_t> stem_bayer2x_tables(const float *w, const float *bias, int src_h, int chan_order, int rotate180);
 cudaError_t launch_stem_bayer2x(const PreprocessParams &p, int frame0, const uint32_t *tab, __half *out,

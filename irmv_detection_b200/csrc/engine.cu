@@ -1914,6 +1914,21 @@ int irmv_engine_rotated_image(irmv_engine *e, int slot, uint8_t *dst) {
 
 long long irmv_debug_alloc_count(void) { return g_allocs.load(); }
 
+int irmv_debug_stem_ctas(irmv_engine *e, int *ctas) {
+  IRMV_ABI_TRY
+  if (!e || !ctas) { set_error("null argument"); return 1; }
+  IRMV_CUDA(cudaSetDevice(e->cfg.device));
+  PreprocessParams pp{};
+  pp.src_w = e->cfg.src_width; pp.src_h = e->cfg.src_height;
+  pp.chan_order = e->cfg.chan_order; pp.rotate180 = e->cfg.rotate180;
+  pp.resize_mode = e->cfg.resize_mode; pp.quantize_u8 = e->cfg.quantize_u8;
+  pp.raw_lut = e->raw_lut_on ? e->d_raw_lut : nullptr;
+  const bool fused = e->fused_stem && e->cfg.conv_impl != IRMV_CONV_DIRECT;
+  *ctas = fused && e->d_stem_tab ? stem_bayer2x_ctas(pp) : 0;
+  return 0;
+  IRMV_ABI_CATCH
+}
+
 int irmv_debug_check_padding(irmv_engine *e, long long *bad_pixels) {
   IRMV_ABI_TRY
   if (!e || !bad_pixels) { set_error("null argument"); return 1; }

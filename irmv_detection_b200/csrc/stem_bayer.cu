@@ -360,33 +360,13 @@ cudaError_t launch_o(const StemBayerArgs &a, size_t smem, cudaStream_t s) {
   return cudaGetLastError();
 }
 
-// The table's 1 KB must not cost the kernel a CTA per SM (it is sized for two at the camera's 1024 rows, where
-// about 2.5 KB per CTA are left): refuse the launch rather than silently run at half the occupancy.
-template <bool ROT, int FMT, bool OUT1, bool OUT2>
-cudaError_t launch_lut(const StemBayerArgs &a, size_t smem, cudaStream_t s) {
-  auto on = stem_bayer2x_kernel<ROT, FMT, OUT1, OUT2, true>;
-  auto off = stem_bayer2x_kernel<ROT, FMT, OUT1, OUT2, false>;
-  cudaError_t e = cudaFuncSetAttribute(on, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem + 1024));
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(off, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  int ctas_on = 0, ctas_off = 0;
-  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_on, on, NTHREADS, smem + 1024);
-  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_off, off, NTHREADS, smem);
-  if (e != cudaSuccess) return e;
-  if (ctas_on < ctas_off) {
-    fprintf(stderr, "irmv: camera-case stem with a raw lookup table: %d CTAs per SM instead of %d (shared memory %zu B)\n",
-            ctas_on, ctas_off, smem + 1024);
-    return cudaErrorLaunchOutOfResources;
-  }
-  return launch_o<ROT, FMT, OUT1, OUT2, true>(a, smem + 1024, s);
-}
-
 template <bool ROT, int FMT>
 cudaError_t launch_t(const StemBayerArgs &a, size_t smem, cudaStream_t s) {
   if constexpr (FMT < FMT_RGB) {
-    if (a.raw_lut) {
-      if (a.out && a.out2) return launch_lut<ROT, FMT, true, true>(a, smem, s);
-      if (a.out2) return launch_lut<ROT, FMT, false, true>(a, smem, s);
-      if (a.out) return launch_lut<ROT, FMT, true, false>(a, smem, s);
+    if (a.raw_lut) {                                   // the table's 1 KB sits behind the lerp table
+      if (a.out && a.out2) return launch_o<ROT, FMT, true, true, true>(a, smem + 1024, s);
+      if (a.out2) return launch_o<ROT, FMT, false, true, true>(a, smem + 1024, s);
+      if (a.out) return launch_o<ROT, FMT, true, false, true>(a, smem + 1024, s);
       return cudaErrorInvalidValue;
     }
   } else {
@@ -421,14 +401,64 @@ int format_of(int chan_order, int rotate180) {
 // staged-row capacity of a strip for a source of height H (H / 640 = P / Q)
 int nr_max_for(int P, int Q, int fmt) { return (2 * orows_for(fmt) * P + Q - 1) / Q + (fmt >= FMT_RGB ? 4 : 6); }
 
+constexpr size_t kMaxSmem = 227 * 1024;  // dynamic shared memory a block may have on sm_100
+
+// dynamic shared memory of a launch without the raw table: tile + lerp table, then the staged rows
+size_t smem_for(int H, int fmt) {
+  const int g = gcd_i(H, kNet), P = H / g, Q = kNet / g;
+  const size_t lut_n = 2 * Q * 255 + Q + 1;
+  return (((size_t)(2 * orows_for(fmt) + 1) * PITCHW * 4 + lut_n * 2 + 15) & ~(size_t)15) +
+         (size_t)nr_max_for(P, Q, fmt) * row_pitch(fmt);
+}
+
+// CTAs per SM with `smem` bytes of dynamic shared memory.  Every instantiation of a format has the same static
+// shared memory, and __launch_bounds__(NTHREADS, 2) keeps the registers of two CTAs within an SM's file, so the
+// answer depends on the format, the table and smem only.
+template <int FMT, bool LUT>
+int ctas_per_sm(size_t smem) {
+  auto k = stem_bayer2x_kernel<false, FMT, true, false, LUT>;
+  int n = 0;
+  if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k, NTHREADS, smem) != cudaSuccess) {
+    (void)cudaGetLastError();            // a refused query must not surface as the next launch's error
+    return 0;
+  }
+  return n;
+}
+
+int ctas_for(int fmt, bool lut, size_t smem) {
+  switch (fmt) {
+    case FMT_BAYER: return lut ? ctas_per_sm<FMT_BAYER, true>(smem + 1024) : ctas_per_sm<FMT_BAYER, false>(smem);
+    case FMT_BAYER_REDCOL:
+      return lut ? ctas_per_sm<FMT_BAYER_REDCOL, true>(smem + 1024) : ctas_per_sm<FMT_BAYER_REDCOL, false>(smem);
+    case FMT_RGB: return lut ? 0 : ctas_per_sm<FMT_RGB, false>(smem);
+    default: return lut ? 0 : ctas_per_sm<FMT_BGR, false>(smem);
+  }
+}
+
 }  // namespace
 
 // The fast path applies to: 8-bit Bayer or packed u8x3 source of width 1280, height >= 640 with
-// H/640 = P/Q, Q <= 16, reference resize (corner-aligned stretch) and the 8-bit intermediate.
+// H/640 = P/Q, Q <= 16, reference resize (corner-aligned stretch) and the 8-bit intermediate, when its shared
+// memory fits a block: packed sources of 3400 rows and more stage rows three times as long and do not.  With a raw
+// table (p.raw_lut) its 1 KB must also keep the CTAs per SM of the launch without it (the kernel is sized for two at
+// the camera's 1024 rows, where about 2.5 KB per CTA are left); where it would cost one, stem_kernel runs instead,
+// at its full occupancy.  Called without a table at engine creation (no device query) and with it at every launch.
 bool stem_bayer2x_applies(const PreprocessParams &p) {
   if (p.chan_order < 0 || p.chan_order > 5 || p.src_w != SW || p.resize_mode != 0 || !p.quantize_u8 || p.src_h < kNet || p.src_h > 4096) return false;
   const int g = gcd_i(p.src_h, kNet);
-  return kNet / g <= 16;
+  if (kNet / g > 16) return false;
+  const int fmt = format_of(p.chan_order, p.rotate180);
+  const size_t smem = smem_for(p.src_h, fmt);
+  if (!p.raw_lut) return smem <= kMaxSmem;
+  if (fmt >= FMT_RGB || smem + 1024 > kMaxSmem) return false;
+  return ctas_for(fmt, true, smem) >= ctas_for(fmt, false, smem);
+}
+
+int stem_bayer2x_ctas(const PreprocessParams &p) {
+  if (!stem_bayer2x_applies(p)) return 0;
+  const int fmt = format_of(p.chan_order, p.rotate180);
+  return ctas_for(fmt, p.raw_lut != nullptr, smem_for(p.src_h, fmt));
 }
 
 // Host side of the table block (layout above): conv0 weights w[16][9 taps][3] and bias[16] as the engine
@@ -507,16 +537,14 @@ cudaError_t launch_stem_bayer2x(const PreprocessParams &p, int frame0, const uin
                                 long long out_ps, __half *out2, long long out2_ps, cudaStream_t s) {
   StemBayerArgs a{};
   a.src = p.src; a.src_indirect = p.src_indirect; a.n = p.n; a.H = p.src_h; a.frame0 = frame0; a.rev = p.rev_order;
-  const int g = gcd_i(p.src_h, kNet);
-  const int P = p.src_h / g, Q = kNet / g;
+  const int Q = kNet / gcd_i(p.src_h, kNet);
   const int fmt = format_of(p.chan_order, p.rotate180);
   a.Q = Q; a.lut_n = 2 * Q * 255 + Q + 1;
   a.tab_strip = TAB_LUT + (a.lut_n + 7) / 8 * 4;
   a.tab = tab; a.out = out; a.out_ps = out_ps; a.out2 = out2; a.out2_ps = out2_ps;
   a.raw_lut = p.raw_lut;
-  const size_t smem = (((size_t)(2 * orows_for(fmt) + 1) * PITCHW * 4 + (size_t)a.lut_n * 2 + 15) & ~(size_t)15) +
-                      (size_t)nr_max_for(P, Q, fmt) * row_pitch(fmt);
-  if (smem + (p.raw_lut ? 1024 : 0) > 227 * 1024) return cudaErrorInvalidValue;
+  const size_t smem = smem_for(p.src_h, fmt);
+  if (smem + (p.raw_lut ? 1024 : 0) > kMaxSmem) return cudaErrorInvalidValue;
   return p.rotate180 ? launch_f<true>(fmt, a, smem, s) : launch_f<false>(fmt, a, smem, s);
 }
 

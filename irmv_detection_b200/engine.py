@@ -302,6 +302,13 @@ class YoloEngine:
         L.check(self._lib.irmv_debug_check_padding(self._h, C.byref(bad)), "irmv_debug_check_padding")
         return int(bad.value)
 
+    def stem_camera_ctas(self) -> int:
+        """Debug: CTAs per SM of the camera-case stem kernel (csrc/stem_bayer.cu) as the engine launches it now, with
+        its raw table when one is set; 0 when the frames go to the generic stem kernel instead."""
+        n = C.c_int(-1)
+        L.check(self._lib.irmv_debug_stem_ctas(self._h, C.byref(n)), "irmv_debug_stem_ctas")
+        return int(n.value)
+
     def describe_ops(self):
         """Kernels of the network stage in issue order: dicts {kind, k, s, cin, cout, hw, raster, tail_cout}."""
         buf = C.create_string_buffer(16384)

@@ -527,15 +527,63 @@ def _stem_fast_path_emulation(raw, chan, rot):
     return out
 
 
-@pytest.mark.parametrize("H,chan,rot", [(1024, 2, True), (1024, 5, True), (1024, 3, False), (720, 4, True)])
+@pytest.mark.parametrize("rot", [True, False])
+@pytest.mark.parametrize("chan", [2, 3, 4, 5])
+@pytest.mark.parametrize("H", [640, 720, 800, 960, 1024, 1080, 1200, 1280])
 def test_stem_fast_path_arithmetic_matches_oracle(H, chan, rot):
     """The camera-case stem's packed-lane demosaic + integer lerp, restated in numpy, equals the oracle's
-    demosaic -> rot180 -> NPP-convention resize -> 8-bit rounding for every pixel."""
+    demosaic -> rot180 -> NPP-convention resize -> 8-bit rounding for every pixel, at every height of the GPU
+    geometry matrix (tests/test_gpu_stem_geometry.py), all four Bayer patterns, with and without rot180."""
     from oracle import preprocess_ref as PR
     raw = np.random.default_rng(H + chan).integers(0, 256, (H, 1280), dtype=np.uint8)
     x, _ = PR.preprocess(raw, chan, rot, True)
     ref = np.rint(x.transpose(1, 2, 0) * 255).astype(np.int64)
     assert np.array_equal(_stem_fast_path_emulation(raw, chan, rot), ref)
+
+
+def _probe_m0(xp, taps_of=lambda t: t):
+    """What a faithful engine stores in m0 for each probe file of oracle/stem_probe.py, from the padded input xp
+    [N, 3, 641, 641] (FP16 values): FP16(SiLU(read)).  taps_of(t) is the tap actually read for tap t."""
+    from oracle import stem_probe as SP
+    views = SP.tap_views(xp.astype(np.float64))
+    out = []
+    for taps in SP.TAP_FILES:
+        m0 = np.zeros(views.shape[:1] + (320, 320, 16), np.float16)
+        for i, t in enumerate(taps):
+            m0[..., 3 * i:3 * i + 3] = SP.silu(views[:, taps_of(t)]).transpose(0, 2, 3, 1).astype(np.float16)
+        out.append(m0)
+    return out
+
+
+def test_stem_probe_helper_catches_single_errors():
+    """The probe comparison of tests/test_gpu_stem_geometry.py (oracle/stem_probe.py) passes a faithful engine and
+    fails each single error a fused stem could make: one pixel off by one 8-bit step, tap (0, 0) read from (0, 1),
+    a non-zero top padding row, and on the float path one pixel off by two FP16 ulps."""
+    from oracle import stem_probe as SP
+    rng = np.random.default_rng(7)
+    codes = rng.integers(0, 256, (2, 3, 640, 640))
+    x16 = (codes / 255.0).astype(np.float16)
+    got = lambda xp, **kw: SP.engine_views(_probe_m0(xp, **kw))
+    assert SP.compare_codes(got(SP.pad_input(x16)), codes) is None
+    for f, c, y, x in ((0, 0, 0, 0), (1, 2, 639, 639), (1, 1, 331, 12), (0, 1, 7, 400)):
+        bad = codes.copy()
+        bad[f, c, y, x] = bad[f, c, y, x] + 1 if bad[f, c, y, x] < 255 else 254
+        msg = SP.compare_codes(got(SP.pad_input((bad / 255.0).astype(np.float16))), codes)
+        assert msg is not None and f"({f}, {c}, {y}, {x})" in msg, msg
+    msg = SP.compare_codes(got(SP.pad_input(x16), taps_of=lambda t: 1 if t == 0 else t), codes)
+    assert msg is not None and "tap (0, 0)" in msg, msg
+    top = SP.pad_input(x16)
+    top[:, :, 0, 1:] = np.float16(1 / 255)                     # top padding row, left padding column kept zero
+    msg = SP.compare_codes(got(top), codes)
+    assert msg is not None and ", -1, " in msg and "tap (0, " in msg, msg
+    # float path: values off the 8-bit grid, one pixel two FP16 ulps off at a value in [0.5, 1)
+    xf = rng.uniform(0, 1, (1, 3, 640, 640)).astype(np.float16)
+    xf[0, 1, 100, 200] = np.float16(0.75)
+    assert SP.float_deviation(got(SP.pad_input(xf)), xf)[0] <= SP.FLOAT_TOL
+    bad = xf.copy()
+    bad[0, 1, 100, 200] = np.float16(0.75 + 2 * 2.0 ** -11)
+    d, at = SP.float_deviation(got(SP.pad_input(bad)), xf)
+    assert d > SP.FLOAT_TOL and (at["frame"], at["channel"], at["y"], at["x"]) == (0, 1, 100, 200), (d, at)
 
 
 def test_shufflenet_variant_weights_and_oracle(base_image, tmp_path):
