@@ -81,7 +81,7 @@ cudaError_t launch_preprocess(const PreprocessParams &p, cudaStream_t s);
 // rotated packed-RGB frame only (what get_rotated_image() exposes, reference include/irmv_detection/yolo_engine.hpp:34)
 cudaError_t launch_rotate(const PreprocessParams &p, cudaStream_t s);
 // Fused preprocess + conv0 (3x3 s2, 3->16, SiLU): w = [16][9 taps][3] FP32, writes two planes.
-// out2 (optional): parity-split twin of the output (see ConvParams).
+// out2 (optional): parity-split twin of the output (see ConvParams); the camera-case kernel writes one of the two.
 // fast_tab: device table block of stem_bayer2x_tables() (null: always the generic kernel).
 cudaError_t launch_stem(const PreprocessParams &p, const float *w, const float *bias, const uint32_t *fast_tab, __half *out,
                         long long out_pstride, __half *out2, long long out2_pstride, cudaStream_t s);
@@ -168,12 +168,11 @@ struct ConvParams {
   ConvSeg tail_ext;        // channels that precede the intermediate in the tail's input concat (C2f.cv2 over
                            // [older chunks | the bottleneck output just computed]); c == 0: none
   int in_parity;           // 1: seg[0].ptr / pstride describe the parity twin of the input
-  __half *out2;            // parity twin of the output (written in addition to `out`); may be null
+  __half *out2;            // parity twin of the output (written in addition to `out` unless that is null); may be null
   long long out2_pstride;
   int rev_tiles;           // 1: process the tiles from the last to the first.  Consecutive layers alternate the
                            // direction, so a layer starts with the part of its input the producer wrote last --
                            // the part that is still in the 126 MB L2 (tensors of a 128-frame replay are 100-400 MB)
-  int sync_mode;           // tcgen05 producer hand-off: 0 = cp.async-tracked mbarrier, 1 = wait+fence
   long long *trace;        // debug: CTA 0 writes per-tile clock64 stamps [tile][8]; null in production
   int trace_cap;
   // Raster kernel, small replays: the same weights as `split_ways` slices of npad / split_ways output channels,

@@ -723,8 +723,7 @@ bool plan(const ConvParams &p_in, int num_sms, RArgs &a) {
   // Small replays: a launch with fewer 128-pixel tiles than a quarter of the SMs gives every tile to `split_ways`
   // CTAs, one per slice of output channels (ConvParams::w_raster_split).
   a.nsplit = 1;
-  static const bool split_env = !getenv("IRMV_NO_NSPLIT");
-  if (split_env && p.w_raster_split && p.split_ways > 1 && p.stride == 1 && !p.in_parity && !p.tail_w && !p.out2 && !p.out_runs &&
+  if (p.w_raster_split && p.split_ways > 1 && p.stride == 1 && !p.in_parity && !p.tail_w && !p.out2 && !p.out_runs &&
       !p.seg[0].runs && !p.res_up && p.out && p.cout == p.npad && p.npad % (16 * p.split_ways) == 0) {
     const long long m = (long long)p.B * (p.OH + 1) * (p.OW + 1) - (p.OW + 1);
     if ((m + 127) / 128 * p.split_ways <= num_sms) {
@@ -790,14 +789,11 @@ bool plan(const ConvParams &p_in, int num_sms, RArgs &a) {
   auto stage_bytes = [&](int R) { return (size_t)a.NP * plane_pixels(R) * 16; };
   int best_R = 0;
   a.b_stream = 0;
-  static const int rmax_env = getenv("IRMV_RMAX") ? atoi(getenv("IRMV_RMAX")) : 4;   // tuning knob
-  static const bool ext2_env = !getenv("IRMV_EXT1");
   for (int R = 4; R >= 1 && !best_R; R >>= 1) {
-    if (R > rmax_env) continue;
     if (2 * R * (p.npad + tnp) > 512) continue;
     long long tiles = (Mr + 128 * R - 1) / (128 * R);
     if (R > 1 && tiles < 2LL * num_sms) continue;    // keep every SM busy at small batch
-    for (ext_stages = (ext_c && ext2_env) ? 2 : 1; ext_stages >= 1; --ext_stages) {
+    for (ext_stages = ext_c ? 2 : 1; ext_stages >= 1; --ext_stages) {
       if (a.b_bytes + tail_bytes(R) + 2 * stage_bytes(R) + misc > (size_t)SMEM_BUDGET) continue;
       best_R = R;
       break;
@@ -806,7 +802,7 @@ bool plan(const ConvParams &p_in, int num_sms, RArgs &a) {
   if (ext_stages < 1) ext_stages = 1;
   a.ext_stages = ext_stages;
   if (!best_R && tail) return false;                 // a fused tail needs resident weights
-  if (!best_R && !getenv("IRMV_NO_BSTREAM")) {
+  if (!best_R) {
     // weights do not fit next to two activation stages: stream them chunk by chunk.  Larger tiles
     // amortise the weight traffic (all of the weights once per tile), so prefer the largest R that
     // still leaves one tile per SM.
@@ -853,7 +849,7 @@ bool plan(const ConvParams &p_in, int num_sms, RArgs &a) {
     // (shared memory and TMEM halves) run two: their phases interleave.
     const size_t half_budget = 112 * 1024;
     const size_t fixed = a.b_bytes + tail_bytes(a.R) + misc;
-    const bool two = !getenv("IRMV_ONE_CTA") && alloc <= 256 && fixed + 2 * (size_t)a.a_stage_bytes <= half_budget;
+    const bool two = alloc <= 256 && fixed + 2 * (size_t)a.a_stage_bytes <= half_budget;
     a.ctas_per_sm = two ? 2 : 1;
     const size_t budget = two ? half_budget : (size_t)SMEM_BUDGET;
     a.stages = (int)((budget - fixed) / a.a_stage_bytes);
@@ -892,7 +888,6 @@ cudaError_t launch_k(const RArgs &a, int grid, size_t smem, cudaStream_t s) {
     cudaError_t e = cudaFuncSetAttribute(conv_raster_kernel<R, NEPI, ACT, RES, TAIL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e != cudaSuccess) return e;
   }
-  static const bool pdl = !getenv("IRMV_NO_PDL");
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)grid);
   cfg.blockDim = dim3((NEPI + 2) * 32);
@@ -902,7 +897,7 @@ cudaError_t launch_k(const RArgs &a, int grid, size_t smem, cudaStream_t s) {
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, conv_raster_kernel<R, NEPI, ACT, RES, TAIL>, a);
 }
 

@@ -246,7 +246,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_tc_kernel(const __grid_const
     const int Hh = H >> 1, Wh = W >> 1;
     const int stages = a.stages, KB = a.KB;
     const int lag = (stages - 1) / 2 < 7 ? (stages - 1) / 2 : 7;   // own k-blocks in flight = lag + 1
-    const bool nozero = !(p.sync_mode & 2);
     int s = 0;                 // ring slot of the current k-block
     uint32_t ph = 0;           // its phase
     int par = 0;               // its parity (which group owns it)
@@ -274,7 +273,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_tc_kernel(const __grid_const
         const int my0 = (up0 ? half : full) * 8;           // halfs inside a plane
         const int my1 = two ? (up1 ? half : full) * 8 : 0;
         // the PR layout's zero row/column make every tap of a real output pixel readable
-        const uint32_t vb = __ballot_sync(0xffffffffu, m < M && nozero) >> (lane & 24);
+        const uint32_t vb = __ballot_sync(0xffffffffu, m < M) >> (lane & 24);
         const uint32_t mfull = k3 ? 0x1FFu : 1u;
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
@@ -346,7 +345,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_tc_kernel(const __grid_const
           __syncwarp();
           if (lane == 0) mbar_arrive(&bars->tmem_empty[acc]);
         }
-        if (!mok || c0 >= p.cout || (p.sync_mode & 16)) continue;
+        if (!mok || c0 >= p.cout) continue;
         float v[16];
 #pragma unroll
         for (int j = 0; j < 16; ++j) {
@@ -369,7 +368,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_tc_kernel(const __grid_const
         __half2 hv[8];
 #pragma unroll
         for (int t = 0; t < 8; ++t) hv[t] = __floats2half2_rn(v[2 * t], v[2 * t + 1]);
-        if (p.sync_mode & 8) continue;
         *reinterpret_cast<uint4 *>(orow + (size_t)pl * p.out_pstride) = *reinterpret_cast<uint4 *>(&hv[0]);
         if (c0 + 8 < p.cout)
           *reinterpret_cast<uint4 *>(orow + (size_t)(pl + 1) * p.out_pstride) = *reinterpret_cast<uint4 *>(&hv[4]);
@@ -403,7 +401,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) conv_tc_kernel(const __grid_const
           const uint64_t adesc = make_desc(smem_u32(sA + (size_t)s * A_STAGE));
           const uint64_t bdesc = make_desc(smem_u32(sB + (size_t)(a.b_resident ? kb : s) * b_block_bytes));
           const int nks = (kb == KB - 1) ? a.ksteps_last : 4;
-          if (!(p.sync_mode & 4))
           for (int ks = 0; ks < nks; ++ks)
             tc_mma_f16(tmem_d, adesc + (uint64_t)(ks * 2), bdesc + (uint64_t)(ks * 2), a.idesc,
                        (uint32_t)((kb | ks) != 0));
@@ -476,8 +473,7 @@ cudaError_t launch_conv_tc(const ConvParams &p_in, int num_sms, cudaStream_t s) 
   a.num_tiles = (a.M + BM - 1) / BM;
   a.nsplit = 1;
   a.npad_full = p.npad;
-  static const bool split_env = !getenv("IRMV_NO_NSPLIT");
-  if (split_env && p.npad >= 128 && p.npad % 64 == 0 && p.cout == p.npad && a.num_tiles * 4 <= num_sms) {
+  if (p.npad >= 128 && p.npad % 64 == 0 && p.cout == p.npad && a.num_tiles * 4 <= num_sms) {
     a.nsplit = 4;
     p.npad /= 4;
     p.cout /= 4;
@@ -509,7 +505,6 @@ cudaError_t launch_conv_tc(const ConvParams &p_in, int num_sms, cudaStream_t s) 
   }
   const int slots = num_sms / a.nsplit;
   const int grid = (a.num_tiles < slots ? a.num_tiles : slots) * a.nsplit;
-  static const bool pdl = !getenv("IRMV_NO_PDL") && !getenv("IRMV_TC_NO_PDL");
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)grid);
   cfg.blockDim = dim3(NTHREADS);
@@ -519,7 +514,7 @@ cudaError_t launch_conv_tc(const ConvParams &p_in, int num_sms, cudaStream_t s) 
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, conv_tc_kernel, a);
 }
 

@@ -354,9 +354,8 @@ struct Tensor {            // channel-blocked planar PR layout (common.cuh)
   __half *p = nullptr;     // pixel 0 of plane 0
   long long pstride = 0;   // halfs between planes
   int H = 0, W = 0, C = 0;
-  __half *pp = nullptr;    // parity-split twin (4 * C/8 planes of (H/2) x (W/2) rasters), or null
-  long long pp_stride = 0;
-  bool parity_only = false;  // the producer writes only the twin (every consumer reads the twin)
+  __half *pp = nullptr;    // parity-split twin (4 * C/8 planes of (H/2) x (W/2) rasters), or null;
+  long long pp_stride = 0; // when set, the producer writes only the twin and every consumer reads it
   std::vector<int> cmap;     // logical -> physical channel (ShuffleNetV2 stage buffers); empty = identity
 };
 
@@ -556,7 +555,7 @@ struct irmv_engine {
   long long next_ticket = 0;
   double profile_ms = 0.0, device_ms = 0.0;
   bool pnp_on = false;
-  bool fused_stem = true;               // preprocess + conv0 in one kernel (input never materialised)
+  bool fused_stem = true;               // preprocess + conv0 in one kernel (input never materialised); never with the direct kernel
   float *d_stem_w = nullptr, *d_stem_b = nullptr;
   uint32_t *d_stem_tab = nullptr;        // table block of the camera-case stem (stem_bayer.cu), or null
   uint8_t *d_raw_lut = nullptr;          // [2][2][256] raw-domain colour table (irmv_engine_set_raw_lut), allocated on first use
@@ -606,10 +605,9 @@ bool new_tensor(Lane &ln, int S, int H, int W, int C, Tensor &t, const char *tap
   return true;
 }
 
-// Parity-split twin of `t` (written by t's producer next to the normal layout, read by a
+// Parity-split twin of `t` (written by t's producer instead of the normal layout, read by a
 // stride-2 consumer running on the raster kernel; ConvParams in common.cuh).
-bool add_parity_twin(Lane &ln, int S, Tensor &t, bool only) {
-  t.parity_only = only;
+bool add_parity_twin(Lane &ln, int S, Tensor &t) {
   const size_t plane_px = ((size_t)kGuardFront + (size_t)pr_pixels(S, t.H / 2, t.W / 2) + kGuardBack + 7) & ~(size_t)7;
   t.pp_stride = (long long)plane_px * 8;
   __half *base = nullptr;
@@ -664,24 +662,22 @@ void add_conv(irmv_engine *e, Lane &ln, HostConv &hc, std::vector<SegRef> in, in
   p.res = res ? res->p + (long long)(res_coff / 8) * res->pstride : nullptr;
   p.res_pstride = res ? res->pstride : 0;
   p.res_up = res ? res_up : 0;
-  p.sync_mode = 0;
   p.trace = nullptr; p.trace_cap = 0;
   p.in_parity = 0;
   p.out2 = nullptr; p.out2_pstride = 0;
   if (out.pp && out_coff == 0 && hc.cout == out.C) {
     p.out2 = out.pp; p.out2_pstride = out.pp_stride;
-    if (out.parity_only) p.out = nullptr;
+    p.out = nullptr;
   }
-  if (hc.stride == 2 && p.nseg == 1 && in[0].t->pp && in[0].coff == 0 && in[0].c == in[0].t->C &&
-      !getenv("IRMV_NO_RASTER") && !getenv("IRMV_NO_S2_RASTER")) {
+  if (hc.stride == 2 && p.nseg == 1 && in[0].t->pp && in[0].coff == 0 && in[0].c == in[0].t->C) {
     ConvParams q = p;                       // try the raster kernel on the parity twin of the input
     q.in_parity = 1;
     q.seg[0].ptr = in[0].t->pp; q.seg[0].pstride = in[0].t->pp_stride;
     q.seg[1] = q.seg[0];
     if (conv_raster_fits(q)) p = q;
-    else if (in[0].t->parity_only) fprintf(stderr, "irmv: internal: stride-2 consumer of a parity-only tensor does not fit the raster kernel\n");
+    else fprintf(stderr, "irmv: internal: stride-2 consumer of a parity-only tensor does not fit the raster kernel\n");
   }
-  op.raster = conv_raster_fits(p) && !getenv("IRMV_NO_RASTER");
+  op.raster = conv_raster_fits(p);
   if (p.out2 && !op.raster) { p.out2 = nullptr; p.out = out.p; }   // conv0 as a stand-alone op: the stem kernel writes the twin
   ln.ops.push_back(op);
 }
@@ -689,14 +685,14 @@ void add_conv(irmv_engine *e, Lane &ln, HostConv &hc, std::vector<SegRef> in, in
 // C2f (ultralytics): cv1 -> split -> n bottlenecks chained on the last chunk -> cv2 over all chunks.
 // All chunks live in one buffer so split and concat are channel offsets.
 bool add_c2f(irmv_engine *e, Lane &ln, size_t &ci, std::vector<SegRef> in, int H, int W, int c2,
-             int n, bool shortcut, Tensor &out, const char *tap, int parity_out = 0) {   // 1: twin only, 2: both layouts
+             int n, bool shortcut, Tensor &out, const char *tap, bool parity_out = false) {   // out: the twin only
   const int c = c2 / 2;
   Tensor buf, tmp;
   if (!new_tensor(ln, e->S, H, W, (2 + n) * c, buf) || !new_tensor(ln, e->S, H, W, c, tmp) ||
       !new_tensor(ln, e->S, H, W, c2, out, tap))
     return false;
   if (parity_out) {
-    if (!add_parity_twin(ln, e->S, out, parity_out == 1)) return false;
+    if (!add_parity_twin(ln, e->S, out)) return false;
     if (tap) ln.taps[tap] = out;
   }
   // cv1 of the neck C2f blocks reads concat(upsample(a), b).  A 1x1 conv commutes with nearest upsampling:
@@ -734,7 +730,7 @@ bool add_c2f(irmv_engine *e, Lane &ln, size_t &ci, std::vector<SegRef> in, int H
 // disappears (m1 -> m2.cv1 and the Detect towers' 3x3 -> 1x1 pairs).  Only when nobody else reads
 // the intermediate and the fused operands fit (conv_raster_fits decides).
 void fuse_tails(irmv_engine *e, Lane &ln) {
-  if (e->cfg.conv_impl == IRMV_CONV_DIRECT || e->cfg.reserved[1] || getenv("IRMV_NO_TAIL")) return;
+  if (e->cfg.conv_impl == IRMV_CONV_DIRECT || e->cfg.reserved[1]) return;
   auto overlaps = [](const __half *a0, const __half *a1, const __half *b0, const __half *b1) { return a0 < b1 && b0 < a1; };
   for (size_t i = 0; i + 1 < ln.ops.size(); ++i) {
     Op &m = ln.ops[i];
@@ -798,15 +794,13 @@ bool build_lane(irmv_engine *e, Lane &ln) {
   if (!new_tensor(ln, S, kNet, kNet, kInC, ln.in8, "input")) return false;
   size_t ci = 0;
   Tensor t0, t1, x2, t3, x4, t5, x6, t7, x8, sp, x9, x12, x15, t16, x18, t19, x21;
-  // stride-2 3x3 layers whose operands fit run on the raster kernel from parity-split twins of
-  // their inputs (m1, m3, m5, m16); the producers write the twin next to the normal layout
-  const bool par = e->cfg.conv_impl != IRMV_CONV_DIRECT && !getenv("IRMV_NO_RASTER") && !getenv("IRMV_NO_S2_RASTER");
-  const bool fused = e->fused_stem && e->cfg.conv_impl != IRMV_CONV_DIRECT;
-  // x4 / x15 also feed stride-1 consumers, so their producers would write both layouts (m5, m16)
-  const bool par2 = par && getenv("IRMV_S2_DUAL");
+  // the stride-2 3x3 layers m1 and m3 run on the raster kernel from parity-split twins of their
+  // inputs, which their producers write instead of the normal layout.  (x4 / x15, the inputs of m5
+  // and m16, also feed stride-1 consumers: their producers would have to write both layouts.)
+  const bool par = e->cfg.conv_impl != IRMV_CONV_DIRECT;
   const bool shuffle = e->arch == kArchShuffleKpt;
   if (!new_tensor(ln, S, 320, 320, 16, t0, "m0")) return false;
-  if (!shuffle && par && fused && !add_parity_twin(ln, S, t0, true)) return false;
+  if (!shuffle && par && e->fused_stem && !add_parity_twin(ln, S, t0)) return false;
   ln.taps["m0"] = t0;
   add_conv(e, ln, *e->convs[ci++], {{&ln.in8, 0, kInC, 0}}, 640, 640, t0, 0);
   ln.ops.back().cp.out2 = nullptr;                 // conv0 as a stand-alone op never writes the twin
@@ -840,12 +834,11 @@ bool build_lane(irmv_engine *e, Lane &ln) {
         // depthwise conv reads a halo other CTAs may already have rewritten, so not in place)
         Tensor XB;
         if (!new_tensor(ln, S, oh, oh, st.cout, X) || (st.units && !new_tensor(ln, S, oh, oh, st.cout, XB))) return false;
-        static const int th_force = getenv("IRMV_UNIT_TH") ? atoi(getenv("IRMV_UNIT_TH")) : 0;
         auto pick_th = [&](ShuffleUnitParams q) {                          // most rows per tile that still leave two CTAs per SM
           for (int th : {8, 4, 2}) {
             if (oh % th) continue;
             q.TH = th;
-            if (th == th_force || (!th_force && shuffle_unit_ctas_per_sm(q) >= 2)) return th;
+            if (shuffle_unit_ctas_per_sm(q) >= 2) return th;
           }
           return 1;
         };
@@ -912,10 +905,10 @@ bool build_lane(irmv_engine *e, Lane &ln) {
   } else {
   if (!new_tensor(ln, S, 160, 160, 32, t1, "m1")) return false;
   add_conv(e, ln, *e->convs[ci++], {{&t0, 0, 16, 0}}, 320, 320, t1, 0);
-  if (!add_c2f(e, ln, ci, {{&t1, 0, 32, 0}}, 160, 160, 32, 1, true, x2, "m2", par ? 1 : 0)) return false;
+  if (!add_c2f(e, ln, ci, {{&t1, 0, 32, 0}}, 160, 160, 32, 1, true, x2, "m2", par)) return false;
   if (!new_tensor(ln, S, 80, 80, 64, t3, "m3")) return false;
   add_conv(e, ln, *e->convs[ci++], {{&x2, 0, 32, 0}}, 160, 160, t3, 0);
-  if (!add_c2f(e, ln, ci, {{&t3, 0, 64, 0}}, 80, 80, 64, 2, true, x4, "m4", par2 ? 2 : 0)) return false;
+  if (!add_c2f(e, ln, ci, {{&t3, 0, 64, 0}}, 80, 80, 64, 2, true, x4, "m4")) return false;
   if (!new_tensor(ln, S, 40, 40, 128, t5, "m5")) return false;
   add_conv(e, ln, *e->convs[ci++], {{&x4, 0, 64, 0}}, 80, 80, t5, 0);
   if (!add_c2f(e, ln, ci, {{&t5, 0, 128, 0}}, 40, 40, 128, 2, true, x6, "m6")) return false;
@@ -933,7 +926,7 @@ bool build_lane(irmv_engine *e, Lane &ln) {
   add_conv(e, ln, *e->convs[ci++], {{&sp, 0, 512, 0}}, 20, 20, x9, 0);
   // neck: upsample and concat happen in the consumers' gathers
   if (!add_c2f(e, ln, ci, {{&x9, 0, 256, 1}, {&x6, 0, 128, 0}}, 40, 40, 128, 1, false, x12, "m12")) return false;
-  if (!add_c2f(e, ln, ci, {{&x12, 0, 128, 1}, {&x4, 0, 64, 0}}, 80, 80, 64, 1, false, x15, "m15", par2 ? 2 : 0)) return false;
+  if (!add_c2f(e, ln, ci, {{&x12, 0, 128, 1}, {&x4, 0, 64, 0}}, 80, 80, 64, 1, false, x15, "m15")) return false;
   ln.ops.back().signal = 0;                        // P3 feature ready: its Detect / keypoint towers may start
   if (!new_tensor(ln, S, 40, 40, 64, t16, "m16")) return false;
   add_conv(e, ln, *e->convs[ci++], {{&x15, 0, 64, 0}}, 80, 80, t16, 0);
@@ -1055,29 +1048,27 @@ int issue_replay(irmv_engine *e, Lane &ln, int n, cudaStream_t st, int *launches
   pp.chan_order = e->cfg.chan_order; pp.rotate180 = e->cfg.rotate180;
   pp.resize_mode = e->cfg.resize_mode; pp.quantize_u8 = e->cfg.quantize_u8;
   pp.raw_lut = e->raw_lut_on ? e->d_raw_lut : nullptr;
-  const bool fused = e->fused_stem && e->cfg.conv_impl != IRMV_CONV_DIRECT;
-  if (fused) IRMV_CUDA(launch_stem(pp, e->d_stem_w, e->d_stem_b, e->d_stem_tab, ln.stem_out.parity_only ? nullptr : ln.stem_out.p, ln.stem_out.pstride, ln.stem_out.pp, ln.stem_out.pp_stride, st));
+  if (e->fused_stem) IRMV_CUDA(launch_stem(pp, e->d_stem_w, e->d_stem_b, e->d_stem_tab, ln.stem_out.pp ? nullptr : ln.stem_out.p, ln.stem_out.pstride, ln.stem_out.pp, ln.stem_out.pp_stride, st));
   else IRMV_CUDA(launch_preprocess(pp, st));
   cnt += 1 + (ln.rotated ? 1 : 0);
   if (mark(1)) return 1;
   op_mark();
   // Consecutive kernels walk their tiles in opposite directions (ConvParams::rev_tiles): a layer then
   // starts with the end of the tensor its producer has just finished writing, which is what the L2 still holds.
-  static const bool pingpong = !getenv("IRMV_NO_PINGPONG");
   // Branched schedule for small replays: at batch 1 a Detect tower launch occupies 4-52 of the 148 SMs and the
   // replay is a chain of ~57 launch latencies, so the towers of a scale run on side streams next to the rest of the
   // neck and next to each other (fork / join by events; inside a CUDA graph these become parallel branches).  Measured
   // (scripts/ab_small.py, device time of a replay, one stream -> branched): 1 frame 392 -> 346 us, 8 frames 548 -> 525,
   // 64 frames 1438 -> 1411 (the towers fill the other launches' partial last waves); at 128 / 256 frames every launch
   // fills the machine and the two schedules time the same, so those stay on one stream.
-  static const int branch_max = getenv("IRMV_BRANCH_MAX") ? atoi(getenv("IRMV_BRANCH_MAX")) : 64;
-  const bool branched = n <= branch_max && !stage_events && !op_events && e->cfg.conv_impl != IRMV_CONV_DIRECT;
+  constexpr int kBranchMax = 64;
+  const bool branched = n <= kBranchMax && !stage_events && !op_events && e->cfg.conv_impl != IRMV_CONV_DIRECT;
   unsigned side_used = 0;
   const cudaStream_t trunk = st;
   int seq = 0;
   bool first = true;
   for (auto &op : ln.ops) {
-    if (first && fused) { first = false; continue; }        // conv0 ran inside the stem kernel
+    if (first && e->fused_stem) { first = false; continue; }   // conv0 ran inside the stem kernel
     first = false;
     ++seq;
     st = trunk;
@@ -1088,19 +1079,19 @@ int issue_replay(irmv_engine *e, Lane &ln, int n, cudaStream_t st, int *launches
     if (op.kind == Op::CONV) {
       ConvParams p = op.cp;
       p.B = n;
-      p.rev_tiles = pingpong ? (seq & 1) : 0;
+      p.rev_tiles = seq & 1;
       if (e->cfg.conv_impl == IRMV_CONV_DIRECT) IRMV_CUDA(launch_conv_direct(p, st));
       else if (op.raster) IRMV_CUDA(launch_conv_raster(p, e->num_sms, st));
       else IRMV_CUDA(launch_conv_tc(p, e->num_sms, st));
     } else if (op.kind == Op::SHUF) {
       ShuffleUnitParams q = op.su;
       q.B = n;
-      q.rev = pingpong ? (seq & 1) : 0;
+      q.rev = seq & 1;
       IRMV_CUDA(launch_shuffle_unit(q, st));
     } else if (op.kind == Op::DW) {
       DwParams d = op.dw;
       d.B = n;
-      d.rev = pingpong ? (seq & 1) : 0;
+      d.rev = seq & 1;
       IRMV_CUDA(launch_dwconv3x3(d, st));
     } else {
       IRMV_CUDA(launch_sppf_pool(op.pool_buf, n, op.pH, op.pW, op.pStride, op.pC, st));
@@ -1217,8 +1208,8 @@ int enqueue(irmv_engine *e, const uint8_t *frames_dev, int n, const uint8_t *fra
   // Pipelined host batches (submit_batch) are replayed in chunks of at most 128 frames: a chunk starts as soon as its
   // own frames have landed, under the copy of the next one.  Measured on 256-frame batches (end to end, frames/s):
   // one 256-frame replay 40.7-40.8 k, two chunks of 128 41.3-41.4 k (0.977 of the H2D ceiling), four of 64 37.6 k.
-  static const int host_chunk = getenv("IRMV_HOST_CHUNK") ? atoi(getenv("IRMV_HOST_CHUNK")) : 128;
-  const int S = (frames_host && copy_stream && host_chunk > 0 && host_chunk < e->S) ? host_chunk : e->S;
+  constexpr int kHostChunk = 128;
+  const int S = (frames_host && copy_stream && kHostChunk < e->S) ? kHostChunk : e->S;
   const int chunks = (n + S - 1) / S;
   const int used = chunks < e->L ? chunks : e->L;
   unsigned fields = 1u << kNum | 1u << kBoxes | 1u << kScores | 1u << kClasses | 1u << kIndex;
@@ -1257,8 +1248,7 @@ int enqueue(irmv_engine *e, const uint8_t *frames_dev, int n, const uint8_t *fra
     IRMV_CUDA(cudaGetLastError());
     if (int rc = run_replay(e, ln, nf)) return rc;
     // results: the lane's block -> the slots of its frames in the pinned set
-    static const bool merge = !getenv("IRMV_NO_D2H_MERGE");   // A/B knob
-    const CopyPlan plan = plan_copies(e->lane_res, e->res, fields, (size_t)f0, (size_t)nf, merge);
+    const CopyPlan plan = plan_copies(e->lane_res, e->res, fields, (size_t)f0, (size_t)nf);
     for (int i = 0; i < plan.n; ++i) {
       const CopyRange &r = plan.r[i];
       e->d2h_bytes += r.bytes;
@@ -1425,10 +1415,10 @@ int irmv_engine_create(const char *weights_path, const irmv_engine_config *cfg, 
   if (e->arch == kArchYolov8n && fc.size() != 63 && fc.size() != 72) { set_error("weight file is not YOLOv8n nc=14"); return 4; }
   e->pose = e->arch == kArchShuffleKpt || fc.size() == 72;    // + keypoint branch (kpt_shape [4, 2])
   if (!check_specs(fc, e->pose, e->arch)) return 4;            // make_conv / build_lane index by the expected shapes
-  if (e->arch == kArchShuffleKpt && (cfg->conv_impl == IRMV_CONV_DIRECT || getenv("IRMV_NO_RASTER"))) {
+  if (e->arch == kArchShuffleKpt && cfg->conv_impl == IRMV_CONV_DIRECT) {
     set_error("the ShuffleNetV2 variant runs on the tcgen05 raster kernel only"); return 2;
   }
-  e->up_split = cfg->conv_impl != IRMV_CONV_DIRECT && cfg->reserved[3] == 0 && !getenv("IRMV_NO_RASTER") && !getenv("IRMV_NO_UP_SPLIT");
+  e->up_split = cfg->conv_impl != IRMV_CONV_DIRECT && cfg->reserved[3] == 0;
   // 63 reference convs -> 60 GEMMs (Detect box.0|cls.0 merged per scale)
   auto single = [&](size_t i, int cin_pad, std::vector<int> seg) {
     e->convs.emplace_back(new HostConv(make_conv({&fc[i]}, cin_pad, seg)));
@@ -1534,7 +1524,7 @@ int irmv_engine_create(const char *weights_path, const irmv_engine_config *cfg, 
       single(b + 1, 16, {16});
       single(b + 2, 16, {16});
     }
-  e->sh_fused = e->arch == kArchShuffleKpt && cfg->reserved[2] == 0 && !getenv("IRMV_NO_SHUFFLE_FUSE");
+  e->sh_fused = e->arch == kArchShuffleKpt && cfg->reserved[2] == 0;
   if (e->sh_fused) {
     // convs[1 .. 22] are the backbone's 1x1 convs (3 per down unit: b1.pw, b2.pw1, b2.pw2; 2 per basic unit),
     // dws[] its depthwise convs (2 per down unit: b1.dw, b2.dw; 1 per basic unit), both in execution order
@@ -1617,7 +1607,7 @@ int irmv_engine_create(const char *weights_path, const irmv_engine_config *cfg, 
     IRMV_CUDA(dev_malloc((void **)&e->d_stem_b, b.size() * 4));
     IRMV_CUDA(cudaMemcpy(e->d_stem_w, w.data(), w.size() * 4, cudaMemcpyHostToDevice));
     IRMV_CUDA(cudaMemcpy(e->d_stem_b, b.data(), b.size() * 4, cudaMemcpyHostToDevice));
-    e->fused_stem = cfg->reserved[0] == 0;
+    e->fused_stem = cfg->reserved[0] == 0 && cfg->conv_impl != IRMV_CONV_DIRECT;
     PreprocessParams probe{};
     probe.src_w = cfg->src_width; probe.src_h = cfg->src_height; probe.chan_order = cfg->chan_order;
     probe.resize_mode = cfg->resize_mode; probe.quantize_u8 = cfg->quantize_u8;
@@ -1923,8 +1913,7 @@ int irmv_debug_stem_ctas(irmv_engine *e, int *ctas) {
   pp.chan_order = e->cfg.chan_order; pp.rotate180 = e->cfg.rotate180;
   pp.resize_mode = e->cfg.resize_mode; pp.quantize_u8 = e->cfg.quantize_u8;
   pp.raw_lut = e->raw_lut_on ? e->d_raw_lut : nullptr;
-  const bool fused = e->fused_stem && e->cfg.conv_impl != IRMV_CONV_DIRECT;
-  *ctas = fused && e->d_stem_tab ? stem_bayer2x_ctas(pp) : 0;
+  *ctas = e->fused_stem && e->d_stem_tab ? stem_bayer2x_ctas(pp) : 0;
   return 0;
   IRMV_ABI_CATCH
 }
@@ -1972,7 +1961,7 @@ int irmv_engine_read_tensor(irmv_engine *e, const char *name, void *dst, int64_t
       const int planes = t.C / 8;
       std::vector<uint16_t> tmp(px * 8);
       uint16_t *o = static_cast<uint16_t *>(dst);
-      for (int pl = 0; pl < planes && !t.parity_only; ++pl) {
+      for (int pl = 0; pl < planes && !t.pp; ++pl) {
         IRMV_CUDA(cudaMemcpy(tmp.data(), t.p + (long long)pl * t.pstride, tmp.size() * 2, cudaMemcpyDeviceToHost));
         for (int b = 0; b < nb; ++b)
           for (int y = 0; y < t.H; ++y)
@@ -1987,7 +1976,7 @@ int irmv_engine_read_tensor(irmv_engine *e, const char *name, void *dst, int64_t
           for (int c = 0; c < t.C; ++c) o[q * t.C + c] = px[t.cmap[c]];
         }
       }
-      if (t.parity_only) {               // only the parity-split twin exists: planes [g][C/8] of (H/2) x (W/2)
+      if (t.pp) {                        // only the parity-split twin exists: planes [g][C/8] of (H/2) x (W/2)
         const size_t px2 = (size_t)pr_pixels(nb, t.H / 2, t.W / 2);
         tmp.resize(px2 * 8);
         for (int g = 0; g < 4; ++g)
@@ -2326,9 +2315,8 @@ int irmv_engine_describe_ops(irmv_engine *e, char *buf, int cap) {
   if (!e || !buf || cap < 1) return -1;
   std::string out;
   bool first = true;
-  const bool fused = e->fused_stem && e->cfg.conv_impl != IRMV_CONV_DIRECT;
   for (auto &o : e->lanes[0].ops) {
-    if (first && fused) { first = false; continue; }       // conv0 runs inside the stem kernel
+    if (first && e->fused_stem) { first = false; continue; }   // conv0 runs inside the stem kernel
     first = false;
     char line[160];
     if (o.kind == Op::POOL) snprintf(line, sizeof line, "pool\n");
@@ -2351,10 +2339,9 @@ int irmv_engine_describe_plans(irmv_engine *e, int nframes, char *buf, int cap) 
   if (!e || !buf || cap < 1 || nframes < 1) return -1;
   std::string out;
   bool first = true;
-  const bool fused = e->fused_stem && e->cfg.conv_impl != IRMV_CONV_DIRECT;
   const int n = nframes < e->S ? nframes : e->S;
   for (auto &o : e->lanes[0].ops) {
-    if (first && fused) { first = false; continue; }
+    if (first && e->fused_stem) { first = false; continue; }
     first = false;
     char line[200];
     if (o.kind == Op::POOL) { out += "pool\n"; continue; }
@@ -2392,7 +2379,6 @@ int irmv_engine_trace_conv(irmv_engine *e, int op_index, int nframes, long long 
   ConvParams p = op->cp;
   p.B = nframes < e->S ? nframes : e->S;
   p.trace = d; p.trace_cap = cap_tiles;
-  if (const char *dbg = getenv("IRMV_TC_DEBUG")) p.sync_mode = atoi(dbg);
   cudaDeviceSynchronize();
   cudaEventRecord(ln.stage_ev[0], ln.stream);
   if (op->raster) launch_conv_raster(p, e->num_sms, ln.stream); else launch_conv_tc(p, e->num_sms, ln.stream);

@@ -613,8 +613,7 @@ cudaError_t launch_stem(const PreprocessParams &p_in, const float *w, const floa
   PreprocessParams p = p_in;
   letterbox_geometry(p.src_w, p.src_h, p.resize_mode, &p.pad_x, &p.pad_y, &p.new_w, &p.new_h);
   if (p.n <= 0) return cudaSuccess;
-  static const bool no_fast = getenv("IRMV_NO_STEM_FAST") != nullptr;
-  if (!no_fast && fast_tab && stem_bayer2x_applies(p)) {
+  if (fast_tab && stem_bayer2x_applies(p)) {
     cudaError_t e = launch_stem_bayer2x(p, p.frame0, fast_tab, out, out_pstride, out2, out2_pstride, s);
     return e == cudaSuccess ? launch_rotate(p, s) : e;
   }

@@ -101,7 +101,7 @@ __device__ __forceinline__ Px3 unpack(const uint32_t *rowj) {
   return o;
 }
 
-// OUT1 / OUT2: write the normal layout / the parity-split twin (at least one of them).
+// OUT1 / OUT2: write the normal layout / the parity-split twin (exactly one of them).
 // LUT (Bayer formats only): the staged rows go through the raw-domain colour table before the demosaic; the
 // [2][2][256]-byte table sits in shared memory between the lerp table and the staged rows.
 template <bool ROT, int FMT, bool OUT1, bool OUT2, bool LUT>
@@ -362,20 +362,17 @@ cudaError_t launch_o(const StemBayerArgs &a, size_t smem, cudaStream_t s) {
 
 template <bool ROT, int FMT>
 cudaError_t launch_t(const StemBayerArgs &a, size_t smem, cudaStream_t s) {
+  if (!a.out == !a.out2) return cudaErrorInvalidValue;   // exactly one layout
   if constexpr (FMT < FMT_RGB) {
     if (a.raw_lut) {                                   // the table's 1 KB sits behind the lerp table
-      if (a.out && a.out2) return launch_o<ROT, FMT, true, true, true>(a, smem + 1024, s);
       if (a.out2) return launch_o<ROT, FMT, false, true, true>(a, smem + 1024, s);
-      if (a.out) return launch_o<ROT, FMT, true, false, true>(a, smem + 1024, s);
-      return cudaErrorInvalidValue;
+      return launch_o<ROT, FMT, true, false, true>(a, smem + 1024, s);
     }
   } else {
     if (a.raw_lut) return cudaErrorInvalidValue;       // the table is defined for Bayer sources only
   }
-  if (a.out && a.out2) return launch_o<ROT, FMT, true, true, false>(a, smem, s);
   if (a.out2) return launch_o<ROT, FMT, false, true, false>(a, smem, s);
-  if (a.out) return launch_o<ROT, FMT, true, false, false>(a, smem, s);
-  return cudaErrorInvalidValue;
+  return launch_o<ROT, FMT, true, false, false>(a, smem, s);
 }
 
 template <bool ROT>

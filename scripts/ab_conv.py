@@ -1,5 +1,5 @@
-"""A/B helper: conv-stage time of one replay (median of 7 eager stage profiles) for the current environment
-knobs (IRMV_MMA_GROUP, IRMV_LATE_PRODUCER, IRMV_RMAX, ...).  usage: python scripts/ab_conv.py [frames] [label]"""
+"""A/B helper: conv-stage and total device time of one replay of the bench workload (1280x1024 Bayer frames, PnP on;
+median of 7 eager stage profiles), for comparing two builds.  usage: python scripts/ab_conv.py [frames] [label]"""
 import os
 import statistics
 import sys

@@ -1,5 +1,5 @@
-"""A/B helper for small replays: median device time of a graph replay of n frames (n = 1, 2, 3, 4, 8) under the
-current environment knobs (IRMV_BRANCH_MAX, IRMV_NO_NSPLIT, ...).  usage: python scripts/ab_small.py [label]"""
+"""A/B helper for small replays: median device time of a graph replay of n frames of the bench workload (n = 1, 2, 3,
+4, 8, or the list in AB_SIZES), for comparing two builds.  usage: python scripts/ab_small.py [label]"""
 import os
 import statistics
 import sys

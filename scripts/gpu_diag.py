@@ -72,7 +72,7 @@ def main():
 
     oracle = Y.build(wpath)
 
-    def net(impl, sync_mode=None):
+    def net(impl):
         eng = irmv.YoloEngine(wpath, (1280, 1024), max_batch=3, sub_batch=3, conv_impl=impl, use_graph=False)
         t0 = time.time()
         dets = eng.detect_batch(fr)
