@@ -246,7 +246,8 @@ int irmv_engine_fetch_keypoints(irmv_engine *e, int ticket, int nframes, float *
 int irmv_armor_params_default(irmv_armor_params *p);
 /* Stage entry: nframes frames as the camera wrote them (the kernel reads the rotated view itself),
  * boxes[nframes*max_det] in source pixels with counts[nframes] valid entries per frame (what detect()
- * returns); out[nframes*max_det], slot-aligned with boxes.  prm == NULL: defaults. */
+ * returns); out[nframes*max_det], slot-aligned with boxes.  prm == NULL: defaults.  Sources up to
+ * 32766 x 32766 with 8 * (src_w + 2) * (src_h + 2) < 2^31; larger ones are refused (returns 2). */
 int irmv_extract_armors(const uint8_t *frames, int frames_on_device, int nframes, int src_w, int src_h, int chan_order,
                         int rotate180, const irmv_bbox *boxes, const int *counts, int max_det,
                         const irmv_armor_params *prm, int device, irmv_armor *out);
@@ -258,7 +259,8 @@ int irmv_extract_armors_last_profile(unsigned long long out[8]);
 /* Fuse the stage into the replay, between NMS and PnP: with irmv_engine_enable_pnp the pose stage then
  * solves on the armor corners (scaled by corner_sx/sy) instead of the box corners, and ok[] is 0 for
  * detections without an armor -- the whole of message_callback's per-frame work
- * (src/irm_detector.cpp:181-208) in one graph. */
+ * (src/irm_detector.cpp:181-208) in one graph.  Refuses (returns 2) an engine whose source size the
+ * stage does not take (see irmv_extract_armors). */
 int irmv_engine_enable_armors(irmv_engine *e, const irmv_armor_params *prm);
 /* out: nframes*max_det armors of the last detect/detect_batch/sync (ticket < 0) or of a collected
  * pipelined batch (its ticket). */

@@ -34,8 +34,11 @@ namespace {
 constexpr int kThreads = 256, kWarps = kThreads / 32;
 constexpr int kSmemWords = 2048;       // per bitmap: ROIs up to 64 K padded pixels keep their bitmaps in shared memory
 constexpr int kRows = 256;             // ... and up to this many rows (per-warp row-extreme arrays, hull)
-constexpr int kMaxRows = 1088;         // ROI height limit of the global-scratch path
-constexpr int kHullSmem = 2 * kRows + 2, kHullGlobal = 2 * kMaxRows + 2;   // a row adds at most two hull vertices
+constexpr int kHullSmem = 2 * kRows + 2;   // a row adds at most two hull vertices (global scratch: slot_hull_cap)
+// Coordinates are packed into 16 bits (x | y << 16 in the hull and the candidate list, short row extremes), and
+// cross3's products of ROI coordinate differences stay below 2^31 for sides up to kMaxSide; the border walk's step
+// cap 8 * (w + 2) * (h + 2) is an int
+constexpr int kMaxSide = 32766;
 constexpr int kCandCap = 64;         // ROIs with at most this many start candidates spread them over the warps
 // (large ROIs use a global scratch slot per CTA: with 64 shared slots behind locks the slots, not the SMs,
 // limited the stage when most boxes are large -- 15 ms per 6400 random-init boxes)
@@ -66,13 +69,18 @@ struct Shared {
   int cand[kCandCap];                  // x | y << 16, padded ROI coordinates
 };
 
-// words of one global scratch slot: two whole-frame bitmaps + the per-warp arrays
+// words of one global scratch slot: two whole-frame bitmaps + the per-warp arrays, sized by the source height
+// (an ROI has at most src_h rows; its border walk indexes rows 0 .. rh of the row-extreme arrays)
 __host__ __device__ inline size_t slot_bitmap_words(int src_w, int src_h) {
   return (((size_t)src_w + 2 + 31) / 32) * ((size_t)src_h + 2);
 }
-__host__ __device__ inline size_t slot_warp_words() { return (size_t)kMaxRows + kHullGlobal; }   // 2 short arrays + hull
+__host__ __device__ inline int slot_rows(int src_h) { return src_h + 2; }
+__host__ __device__ inline int slot_hull_cap(int src_h) { return 2 * slot_rows(src_h) + 2; }
+__host__ __device__ inline size_t slot_warp_words(int src_h) {     // rmin, rmax (shorts: one word per row) + hull
+  return (size_t)slot_rows(src_h) + slot_hull_cap(src_h);
+}
 __host__ __device__ inline size_t slot_words(int src_w, int src_h) {
-  return 2 * slot_bitmap_words(src_w, src_h) + kWarps * slot_warp_words() + 16;
+  return 2 * slot_bitmap_words(src_w, src_h) + kWarps * slot_warp_words(src_h) + 16;
 }
 
 __device__ __forceinline__ int reflect101(int i, int n) {
@@ -376,11 +384,11 @@ __device__ __forceinline__ void roi_body(Shared &sh, const ArmorParams &p, uint3
   if (LARGE) {
     const size_t bw = slot_bitmap_words(W, H);
     fg = slot; ext = slot + bw;
-    uint32_t *wbase = slot + 2 * bw + (size_t)warp * slot_warp_words();
+    uint32_t *wbase = slot + 2 * bw + (size_t)warp * slot_warp_words(H);
     wb.rmin = reinterpret_cast<short *>(wbase);
-    wb.rmax = wb.rmin + kMaxRows;
-    wb.hull = reinterpret_cast<int *>(wbase + kMaxRows);
-    wb.hull_cap = kHullGlobal;
+    wb.rmax = wb.rmin + slot_rows(H);
+    wb.hull = reinterpret_cast<int *>(wbase + slot_rows(H));
+    wb.hull_cap = slot_hull_cap(H);
   } else {
     fg = sh.fg; ext = sh.ext;
     wb.rmin = sh.rmin[warp]; wb.rmax = sh.rmax[warp]; wb.hull = sh.hull[warp]; wb.hull_cap = kHullSmem;
@@ -617,7 +625,7 @@ __global__ void __launch_bounds__(kThreads, 3) extract_armors_kernel(ArmorParams
     const float max_x = x2 < (float)W ? x2 : (float)W, max_y = y2 < (float)H ? y2 : (float)H;
     const int rx = (int)min_x, ry = (int)min_y;
     const int rw = (int)__fsub_rn(max_x, min_x), rh = (int)__fsub_rn(max_y, min_y);
-    if (!(min_x < max_x && min_y < max_y) || rw <= 0 || rh <= 0 || rh > kMaxRows - 2) {
+    if (!(min_x < max_x && min_y < max_y) || rw <= 0 || rh <= 0) {
       if (tid == 0) out->valid = 0;
       continue;
     }
@@ -673,8 +681,16 @@ size_t armors_scratch_total_words(int src_w, int src_h, int grid) { return 64 + 
 // armors_grid() runs 3 CTAs per SM: the table must leave room for them (228 KB per SM, 1 KB reserved per CTA)
 static_assert(3 * (sizeof(Shared) + 1024 + 1024) <= 228 * 1024, "raw lookup table costs the armor stage a CTA per SM");
 
+const char *armors_geometry_error(int src_w, int src_h) {
+  if (src_w < 1 || src_h < 1) return "extract_armors: the source must have at least one row and one column";
+  if (src_w > kMaxSide || src_h > kMaxSide)
+    return "extract_armors: source width and height must be at most 32766 (coordinates are packed into 16 bits)";
+  if (8 * ((long long)src_w + 2) * ((long long)src_h + 2) > 0x7fffffffLL)
+    return "extract_armors: 8 * (width + 2) * (height + 2) must stay below 2^31 (the border walk's step cap is an int)";
+  return nullptr;
+}
+
 cudaError_t launch_extract_armors(const ArmorParams &p, cudaStream_t s) {
-  if (p.src_h > kMaxRows - 2 || p.src_w > 32766) return cudaErrorInvalidValue;
   if (p.raw_lut && p.chan_order < 2) return cudaErrorInvalidValue;    // the table is defined for Bayer sources only
   auto kernel = p.raw_lut ? extract_armors_kernel<true> : extract_armors_kernel<false>;
   const size_t smem = sizeof(Shared) + (p.raw_lut ? 1024 : 0);

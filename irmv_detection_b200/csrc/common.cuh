@@ -314,6 +314,8 @@ struct ArmorParams {
   const uint8_t *raw_lut;               // [2][2][256] raw-domain colour stage of a Bayer source (PreprocessParams::raw_lut), or null
 };
 int armors_grid(int num_sms);
+// null when the stage takes src_w x src_h frames, else why not (checked where the stage is set up, not per launch)
+const char *armors_geometry_error(int src_w, int src_h);
 size_t armors_scratch_words_per_cta(int src_w, int src_h);
 size_t armors_scratch_total_words(int src_w, int src_h, int grid);   // allocate this many words (one slot per CTA of the grid)
 cudaError_t launch_extract_armors(const ArmorParams &p, cudaStream_t s);

@@ -2087,6 +2087,7 @@ int irmv_armor_params_default(irmv_armor_params *p) {
 
 int irmv_engine_enable_armors(irmv_engine *e, const irmv_armor_params *prm) {
   if (!e) { set_error("bad argument"); return 1; }
+  if (const char *why = armors_geometry_error(e->cfg.src_width, e->cfg.src_height)) { set_error(why); return 2; }
   if (prm) e->armor_prm = *prm; else irmv_armor_params_default(&e->armor_prm);
   IRMV_CUDA(cudaSetDevice(e->cfg.device));
   IRMV_CUDA(cudaDeviceSynchronize());
@@ -2195,6 +2196,7 @@ int irmv_extract_armors(const uint8_t *frames, int frames_on_device, int nframes
                         int rotate180, const irmv_bbox *boxes, const int *counts, int max_det,
                         const irmv_armor_params *prm, int device, irmv_armor *out) {
   if (!frames || !boxes || !counts || !out || nframes < 1 || max_det < 1 || src_w < 2 || src_h < 2) { set_error("bad argument"); return 1; }
+  if (const char *why = armors_geometry_error(src_w, src_h)) { set_error(why); return 2; }
   irmv_armor_params q;
   if (prm) q = *prm; else irmv_armor_params_default(&q);
   IRMV_CUDA(cudaSetDevice(device));

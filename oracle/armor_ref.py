@@ -401,6 +401,72 @@ def extract_armors_cv2(image: np.ndarray, boxes: np.ndarray, scores, classes, pr
     return out
 
 
+ARMOR_TOL_PX = 1e-2     # corner / centre agreement of the CUDA stage with cv2 (FP32 rectangle arithmetic on both sides)
+
+
+def check_armors(got, image, boxes, scores, classes, prm: ArmorParams = ArmorParams()):
+    """The GPU stage's armors of one frame against the reference's function written with the cv2 calls.
+
+    got: ARMOR_DTYPE[max_det] (irmv_detection_b200.ARMOR_DTYPE), slot-aligned with `boxes` [n, 4] (rotated-view
+    pixels); image: the rotated view.  Valid flags, size class, class and score must be identical and corners and
+    centre within ARMOR_TOL_PX; every slot from n on must be invalid.  A box may only differ where the restatement
+    `extract_armors` reports an ambiguous minimum-area rectangle (two different rectangles of equal area: OpenCV's pick
+    depends on rounding inside its calipers).  The restatement is pure Python and runs on the mismatched boxes only.
+    Returns (number of armors of the reference, indices of the excused boxes)."""
+    ref = {a.bbox_index: a for a in extract_armors_cv2(image, boxes, scores, classes, prm)}
+    bad = []
+    for i in range(len(boxes)):
+        g = got[i]
+        if bool(g["valid"]) != (i in ref):
+            bad.append(i)
+            continue
+        if i in ref:
+            r = ref[i]
+            if (int(g["size"]) != r.size or np.abs(g["pts"] - r.pts).max() > ARMOR_TOL_PX or
+                    np.abs(g["center"] - r.center).max() > ARMOR_TOL_PX):
+                bad.append(i)
+            else:
+                assert int(g["class_id"]) == r.class_id and abs(float(g["score"]) - r.score) < 1e-7, f"box {i}"
+    assert not got[len(boxes):]["valid"].any(), "an armor in a slot past the frame's detection count"
+    if bad:
+        amb = {}
+        sub = np.asarray(boxes)[bad]
+        extract_armors(image, sub, np.asarray(scores)[bad], np.asarray(classes)[bad], prm, ambiguous=amb)
+        not_excused = [bad[k] for k in range(len(bad)) if k not in amb]
+        assert not not_excused, f"armor mismatch on boxes {not_excused}"
+    return len(ref), bad
+
+
+def boxes_struct(boxes, scores, classes, max_det: int):
+    """One frame's detections as the stage takes them: BBOX_DTYPE [1, max_det], the first len(boxes) slots filled."""
+    from irmv_detection_b200 import BBOX_DTYPE
+    b = np.zeros((1, max_det), BBOX_DTYPE)
+    b["xyxy"][0, :len(boxes)] = boxes
+    b["score"][0, :len(boxes)] = scores
+    b["class_id"][0, :len(boxes)] = classes
+    return b
+
+
+def blob_scene(seed: int, h: int = 1024, w: int = 1280, n_blobs: int = 260):
+    """Speckle (sparse bright pixels and tiny components), filled rotated rectangles and rings (components inside a
+    ring are not external): with permissive light filters most contours with >= 5 vertices become lights, so contour
+    order, the vertex count and the external-only rule all decide the answer."""
+    import cv2
+    rng = np.random.default_rng(seed)
+    img = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
+    img[rng.random((h, w)) < 0.97] //= 3
+    for _ in range(n_blobs):
+        c = (float(rng.uniform(0, w)), float(rng.uniform(0, h)))
+        size = (float(rng.uniform(2, 14)), float(rng.uniform(4, 60)))
+        box = cv2.boxPoints((c, size, float(rng.uniform(-60, 60))))
+        v = int(rng.integers(150, 256))
+        if rng.random() < 0.3:
+            cv2.ellipse(img, (int(c[0]), int(c[1])), (int(size[1]), int(size[1] * 0.6) + 2), 0, 0, 360, (v, v, v), 2)
+        else:
+            cv2.fillConvexPoly(img, np.round(box).astype(np.int32), (v, v, v))
+    return img
+
+
 def synth_armor_scene(n_armors: int = 6, seed: int = 0, w: int = 1280, h: int = 1024, noise: bool = True):
     """A dark arena frame (rotated view) with bright light-bar pairs and the boxes a detector would put
     around them (generator: irmv_detection_b200/synth.py armor_scene)."""

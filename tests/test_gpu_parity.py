@@ -691,46 +691,6 @@ def test_fused_stem_input_pixels_exact(base_image, tmp_path, chan, rotate):
 
 
 # ------------------------------------------------------------------------- light bars -> armors
-ARMOR_TOL_PX = 1e-2     # corner / centre agreement with cv2 (FP32 rectangle arithmetic on both sides)
-
-
-def _check_armors(got, image, boxes, scores, classes, prm):
-    """got: ARMOR_DTYPE[max_det] of one frame.  Reference = the reference's function written with the
-    cv2 calls; a box may only differ where the restatement reports an ambiguous minimum-area rectangle
-    (two different rectangles of equal area: OpenCV's pick depends on rounding inside its calipers)."""
-    from oracle import armor_ref as A
-    ref = {a.bbox_index: a for a in A.extract_armors_cv2(image, boxes, scores, classes, prm)}
-    bad = []
-    for i in range(len(boxes)):
-        g = got[i]
-        if bool(g["valid"]) != (i in ref):
-            bad.append(i)
-            continue
-        if i in ref:
-            r = ref[i]
-            if (int(g["size"]) != r.size or np.abs(g["pts"] - r.pts).max() > ARMOR_TOL_PX or
-                    np.abs(g["center"] - r.center).max() > ARMOR_TOL_PX):
-                bad.append(i)
-            else:
-                assert int(g["class_id"]) == r.class_id and abs(float(g["score"]) - r.score) < 1e-7
-    assert not got[len(boxes):]["valid"].any()
-    if bad:
-        amb = {}
-        sub = np.asarray(boxes)[bad]
-        A.extract_armors(image, sub, np.asarray(scores)[bad], np.asarray(classes)[bad], prm, ambiguous=amb)
-        not_excused = [bad[k] for k in range(len(bad)) if k not in amb]
-        assert not not_excused, f"armor mismatch on boxes {not_excused}"
-    return len(ref), len(bad)
-
-
-def _boxes_struct(irmv, boxes, scores, classes, max_det):
-    b = np.zeros((1, max_det), irmv.BBOX_DTYPE)
-    b["xyxy"][0, :len(boxes)] = boxes
-    b["score"][0, :len(boxes)] = scores
-    b["class_id"][0, :len(boxes)] = classes
-    return b
-
-
 @pytest.mark.parametrize("seed,rotate", [(0, True), (1, True), (2, False)])
 def test_extract_armors_golden_scenes(seed, rotate):
     """Seeded light-bar scenes: armors of the CUDA stage vs the cv2 form of the reference's function and
@@ -740,32 +700,15 @@ def test_extract_armors_golden_scenes(seed, rotate):
     from oracle import armor_ref as A, preprocess_ref as PR
     img, boxes, scores, classes = A.synth_armor_scene(8, seed)
     frame = PR.rot180(img) if rotate else img                  # what the camera wrote
-    got = irmv.extract_armors(frame[None], _boxes_struct(irmv, boxes, scores, classes, 16), [len(boxes)],
+    got = irmv.extract_armors(frame[None], A.boxes_struct(boxes, scores, classes, 16), [len(boxes)],
                               rotate180=rotate)[0]
-    n_ref, n_bad = _check_armors(got, img, boxes, scores, classes, A.ArmorParams())
-    assert n_bad == 0
+    n_ref, excused = A.check_armors(got, img, boxes, scores, classes, A.ArmorParams())
+    assert not excused, excused
     g = np.load(os.path.join(os.path.dirname(__file__), "golden", "armor_golden.npz"))
     idx = np.nonzero(got["valid"])[0]
     assert idx.tolist() == g[f"index{seed}"].tolist()
     assert got["size"][idx].tolist() == g[f"size{seed}"].tolist()
-    assert np.abs(got["pts"][idx] - g[f"pts{seed}"]).max() < ARMOR_TOL_PX
-
-
-def _blob_scene(seed, h=1024, w=1280, n_blobs=260):
-    import cv2
-    rng = np.random.default_rng(seed)
-    img = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
-    img[rng.random((h, w)) < 0.97] //= 3                        # speckle: sparse bright pixels and tiny components
-    for _ in range(n_blobs):
-        c = (float(rng.uniform(0, w)), float(rng.uniform(0, h)))
-        size = (float(rng.uniform(2, 14)), float(rng.uniform(4, 60)))
-        box = cv2.boxPoints((c, size, float(rng.uniform(-60, 60))))
-        v = int(rng.integers(150, 256))
-        if rng.random() < 0.3:                                  # a ring: components inside it are not external
-            cv2.ellipse(img, (int(c[0]), int(c[1])), (int(size[1]), int(size[1] * 0.6) + 2), 0, 0, 360, (v, v, v), 2)
-        else:
-            cv2.fillConvexPoly(img, np.round(box).astype(np.int32), (v, v, v))
-    return img
+    assert np.abs(got["pts"][idx] - g[f"pts{seed}"]).max() < A.ARMOR_TOL_PX
 
 
 @pytest.mark.parametrize("seed,chan,rotate", [(3, 0, True), (4, 1, False), (5, 2, True), (6, 4, True)])
@@ -777,7 +720,7 @@ def test_extract_armors_stress_vs_cv2(seed, chan, rotate):
     import irmv_detection_b200 as irmv
     from oracle import armor_ref as A, preprocess_ref as PR
     rng = np.random.default_rng(100 + seed)
-    scene = _blob_scene(seed)
+    scene = A.blob_scene(seed)
     if chan >= 2:
         frame = PR.mosaic_from_rgb(PR.rot180(scene) if rotate else scene, chan)
     else:
@@ -798,12 +741,12 @@ def test_extract_armors_stress_vs_cv2(seed, chan, rotate):
     prm = A.ArmorParams(binary_threshold=kw["binary_threshold"], light_min_ratio=0.02, light_max_ratio=0.9,
                         light_max_angle=80.0, min_small_center_distance=0.1, max_small_center_distance=3.2,
                         min_large_center_distance=3.2, max_large_center_distance=50.0)
-    got = irmv.extract_armors(frame[None], _boxes_struct(irmv, boxes, scores, np.minimum(classes, 14), 100), [n],
+    got = irmv.extract_armors(frame[None], A.boxes_struct(boxes, scores, np.minimum(classes, 14), 100), [n],
                               chan_order=chan, rotate180=rotate, min_small_center_distance=0.1,
                               max_large_center_distance=50.0, **kw)[0]
-    n_ref, n_bad = _check_armors(got, image, boxes, scores, np.minimum(classes, 14), prm)
+    n_ref, excused = A.check_armors(got, image, boxes, scores, np.minimum(classes, 14), prm)
     assert n_ref >= 20, n_ref
-    assert n_bad <= 6, n_bad                                     # excused (ambiguous rectangle) boxes are rare
+    assert len(excused) <= 6, excused                            # excused (ambiguous rectangle) boxes are rare
 
 
 def test_engine_armor_stage_feeds_pnp(weights_seed0):
@@ -829,7 +772,7 @@ def test_engine_armor_stage_feeds_pnp(weights_seed0):
         assert np.array_equal(arm[f]["valid"][:k], alone[f]["valid"][:k])
         v = np.nonzero(arm[f]["valid"][:k])[0]
         assert np.array_equal(arm[f]["pts"][v], alone[f]["pts"][v])
-        _check_armors(arm[f], scenes[f], dets[f]["xyxy"][:k], dets[f]["score"][:k], dets[f]["class_id"][:k], A.ArmorParams())
+        A.check_armors(arm[f], scenes[f], dets[f]["xyxy"][:k], dets[f]["score"][:k], dets[f]["class_id"][:k], A.ArmorParams())
         assert not ok[f, :k][arm[f]["valid"][:k] == 0].any()
         if len(v):
             pts = arm[f]["pts"][v] * np.array([0.5, 480 / 1024], np.float32)
