@@ -281,6 +281,23 @@ int irmv_engine_fetch_armors(irmv_engine *e, int ticket, int nframes, irmv_armor
  * captured graphs stay. */
 int irmv_engine_set_raw_lut(irmv_engine *e, const uint8_t *lut);
 
+/* Colour-correction stage for Bayer sources: m = 3x3 int16 matrix (row-major, units of 1/1024: identity is 1024 * I)
+ * and tone_lut = [3][256] output tone table (R, G, B) or NULL (identity); m == NULL switches the stage off (the
+ * default), and then tone_lut must be NULL too.  Applied by every kernel that demosaics the raw frame (stem /
+ * preprocess, rotated view, fused armor stage) to every demosaiced pixel -- after the raw table (or the 10/12-bit
+ * decode), before rot180 and resize -- so it is the u8 RGB frame the network input, the rotated view and the armor
+ * stage's gray values are computed from:
+ *   v_c = sum_k m[c][k] * in_k,  out_c = tone_lut[c][clamp((v_c + 512) >> 10, 0, 255)]   (integer, arithmetic shift)
+ * The Bayer engine with matrix M and tone T on frames F returns what an otherwise identical IRMV_CH_PASSTHROUGH
+ * engine without it returns on the packed frames T(M(demosaic(F))).  A saturation gain is one such matrix; with the
+ * ISP order -- black level and gains in the raw table at gamma 1, then the matrix, then gamma in tone_lut -- the
+ * engine reproduces the camera ISP's colour chain apart from auto white balance.  Non-zero (irmv_last_error) for a
+ * packed RGB/BGR source (its ISP has already applied a matrix), for a tone table without a matrix, or while pipelined
+ * batches are in flight.  Works for every raw_format.  The first non-NULL call allocates the device block, later
+ * calls rewrite it in place (no allocation, the captured graphs stay); switching between off and on drops the
+ * captured graphs. */
+int irmv_engine_set_color_matrix(irmv_engine *e, const int16_t m[9], const uint8_t *tone_lut);
+
 /* Pipelined hand-off for host-resident batches -- the B200 form of the overlap the reference gets
  * from its TripleBuffer (camera thread fills the next slot while detect() runs on the previous one,
  * reference README.md:60-63, src/irm_detector.cpp:68-72).  submit queues H2D copy (dedicated copy

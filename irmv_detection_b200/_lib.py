@@ -90,6 +90,7 @@ SYMBOLS = {
     "irmv_engine_enable_armors": (C.c_int, [_P, C.POINTER(ArmorParams)]),
     "irmv_engine_fetch_armors": (C.c_int, [_P, C.c_int, C.c_int, _P]),
     "irmv_engine_set_raw_lut": (C.c_int, [_P, _P]),
+    "irmv_engine_set_color_matrix": (C.c_int, [_P, _P, _P]),
     "irmv_engine_profile_stages": (C.c_int, [_P, _P, C.c_int, C.POINTER(C.c_float * 5)]),
     "irmv_engine_submit_batch": (C.c_int, [_P, _P, C.c_int, C.POINTER(C.c_int)]),
     "irmv_engine_collect": (C.c_int, [_P, C.c_int, _P, _P, _P, _P, _P]),

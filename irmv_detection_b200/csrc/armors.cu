@@ -96,9 +96,11 @@ __device__ __forceinline__ int reflect101(int i, int n) {
 // LUT (Bayer only): every raw sample first goes through the raw-domain colour table lut[y & 1][x & 1][s]
 // (ArmorParams::raw_lut, staged in shared memory); reflect-101 keeps a mirrored neighbour on its colour site, so
 // the neighbours of (sx, sy) use the tables of parity (sx ^ 1) and (sy ^ 1).
-template <bool BAYER, bool LUT>
-__device__ __forceinline__ int gray_at(const uint8_t *__restrict__ frame, const uint8_t *lut, int W, int H, int red_y, int red_x,
-                                       int rot, int X, int Y) {
+// CCM (Bayer only): the demosaiced pixel then goes through the colour-correction block `ccm` (ArmorParams::ccm, staged
+// in shared memory) before the gray sum; memory channel 0 still takes the blue weight.
+template <bool BAYER, bool LUT, bool CCM>
+__device__ __forceinline__ int gray_at(const uint8_t *__restrict__ frame, const uint8_t *lut, const uint8_t *ccm, int W, int H,
+                                       int red_y, int red_x, int rot, int X, int Y) {
   const int sx = rot ? W - 1 - X : X, sy = rot ? H - 1 - Y : Y;
   int c0, c1, c2;
   if (BAYER) {
@@ -119,6 +121,7 @@ __device__ __forceinline__ int gray_at(const uint8_t *__restrict__ frame, const 
     c1 = (is_r || is_b) ? cross : c;
     c0 = is_r ? c : (is_b ? diag : (red_row ? horiz : vert));
     c2 = is_b ? c : (is_r ? diag : (red_row ? vert : horiz));
+    if (CCM) apply_ccm(ccm, c0, c1, c2);
   } else {
     const uint8_t *s = frame + ((size_t)sy * W + sx) * 3;
     c0 = s[0]; c1 = s[1]; c2 = s[2];
@@ -129,8 +132,8 @@ __device__ __forceinline__ int gray_at(const uint8_t *__restrict__ frame, const 
 // ROI -> 1-bit-per-pixel threshold bitmap, padded by one background pixel all round: a warp builds one
 // word per ballot, eight words per round with their loads issued together (clamped coordinates keep
 // the fetch branch-free).
-template <bool BAYER, bool LUT>
-__device__ __forceinline__ void build_bitmap(uint32_t *fg, const uint8_t *__restrict__ frame, const uint8_t *lut, int W, int H, int chan, int rot,
+template <bool BAYER, bool LUT, bool CCM>
+__device__ __forceinline__ void build_bitmap(uint32_t *fg, const uint8_t *__restrict__ frame, const uint8_t *lut, const uint8_t *ccm, int W, int H, int chan, int rot,
                                              int rx, int ry, int rw, int rh, int wpr, int words, int thr, int warp, int lane) {
   int red_y = 0, red_x = 0;
   if (chan == 3) { red_y = 1; red_x = 1; }
@@ -145,7 +148,7 @@ __device__ __forceinline__ void build_bitmap(uint32_t *fg, const uint8_t *__rest
       const int row = w / wpr, wi = w - row * wpr;
       const int x = wi * 32 + lane - 1, y = row - 1;
       const bool in = x >= 0 && x < rw && y >= 0 && y < rh;
-      g[u] = gray_at<BAYER, LUT>(frame, lut, W, H, red_y, red_x, rot, rx + min(max(x, 0), rw - 1), ry + min(max(y, 0), rh - 1));
+      g[u] = gray_at<BAYER, LUT, CCM>(frame, lut, ccm, W, H, red_y, red_x, rot, rx + min(max(x, 0), rw - 1), ry + min(max(y, 0), rh - 1));
       if (!in) g[u] = -1;
     }
 #pragma unroll
@@ -371,9 +374,11 @@ __device__ __forceinline__ void process_border(Shared &sh, const WarpBuf &wb, co
 
 // One detection: bitmap -> exterior flood -> border walks -> lights -> armor.  LARGE selects where
 // the per-ROI state lives, so that the small path compiles to shared-memory instructions.
-// LUT: Bayer frames go through the raw-domain colour table `lut` (shared memory)
-template <bool LARGE, bool LUT>
-__device__ __forceinline__ void roi_body(Shared &sh, const ArmorParams &p, uint32_t *slot, const uint8_t *frame, const uint8_t *lut, int W, int H,
+// LUT: Bayer frames go through the raw-domain colour table `lut` (shared memory); CCM: and through the
+// colour-correction block `ccm` (shared memory)
+template <bool LARGE, bool LUT, bool CCM>
+__device__ __forceinline__ void roi_body(Shared &sh, const ArmorParams &p, uint32_t *slot, const uint8_t *frame, const uint8_t *lut,
+                                         const uint8_t *ccm, int W, int H,
                                          bool bayer, int rx, int ry, int rw, int rh, float min_x, float min_y, int item,
                                          ArmorOut *out, int tid, int lane, int warp) {
   const int PW = rw + 2, PH = rh + 2, wpr = (PW + 31) >> 5, words = PH * wpr;
@@ -397,8 +402,8 @@ __device__ __forceinline__ void roi_body(Shared &sh, const ArmorParams &p, uint3
   int rounds = 0;
   if (p.prof && tid == 0) t0 = clock64();
   // 1. threshold bitmap
-  if (bayer) build_bitmap<true, LUT>(fg, frame, lut, W, H, p.chan_order, p.rotate180, rx, ry, rw, rh, wpr, words, p.binary_threshold, warp, lane);
-  else build_bitmap<false, false>(fg, frame, nullptr, W, H, p.chan_order, p.rotate180, rx, ry, rw, rh, wpr, words, p.binary_threshold, warp, lane);
+  if (bayer) build_bitmap<true, LUT, CCM>(fg, frame, lut, ccm, W, H, p.chan_order, p.rotate180, rx, ry, rw, rh, wpr, words, p.binary_threshold, warp, lane);
+  else build_bitmap<false, false, false>(fg, frame, nullptr, nullptr, W, H, p.chan_order, p.rotate180, rx, ry, rw, rh, wpr, words, p.binary_threshold, warp, lane);
   __syncthreads();
   if (p.prof && tid == 0) t1 = clock64();
   // 2. exterior background.  Seeds on the padding, spread along runs inside each word; then rounds of
@@ -594,14 +599,17 @@ __device__ __forceinline__ void roi_body(Shared &sh, const ArmorParams &p, uint3
 }
 
 // LUT: Bayer frames with a raw-domain colour table; the table (1 KB) follows Shared in dynamic shared memory
-// and is visible after the barrier that precedes the first ROI
-template <bool LUT>
+// and is visible after the barrier that precedes the first ROI.  CCM: Bayer frames with a colour-correction block
+// (kCcmBytes), staged behind the raw table's place the same way.
+template <bool LUT, bool CCM>
 __global__ void __launch_bounds__(kThreads, 3) extract_armors_kernel(ArmorParams p) {
   extern __shared__ __align__(16) uint8_t smem_raw[];
   Shared &sh = *reinterpret_cast<Shared *>(smem_raw);
   uint8_t *lut = smem_raw + sizeof(Shared);
+  uint8_t *ccm = lut + (LUT ? 1024 : 0);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   if (LUT) reinterpret_cast<uint32_t *>(lut)[tid] = reinterpret_cast<const uint32_t *>(p.raw_lut)[tid];   // kThreads == 256 words
+  if (CCM) stage_ccm(ccm, p.ccm, tid);
   const int W = p.src_w, H = p.src_h;
   const bool bayer = p.chan_order >= 2;
   const size_t frame_bytes = (size_t)W * H * (bayer ? 1 : 3);
@@ -638,10 +646,10 @@ __global__ void __launch_bounds__(kThreads, 3) extract_armors_kernel(ArmorParams
     __syncthreads();
     const uint8_t *frame = base + (size_t)f * frame_bytes;
     if (large) {
-      roi_body<true, LUT>(sh, p, p.scratch + (size_t)sh.slot * p.scratch_words_per_cta, frame, lut, W, H, bayer, rx, ry, rw, rh, min_x,
+      roi_body<true, LUT, CCM>(sh, p, p.scratch + (size_t)sh.slot * p.scratch_words_per_cta, frame, lut, ccm, W, H, bayer, rx, ry, rw, rh, min_x,
                      min_y, item, out, tid, lane, warp);
     } else {
-      roi_body<false, LUT>(sh, p, nullptr, frame, lut, W, H, bayer, rx, ry, rw, rh, min_x, min_y, item, out, tid, lane, warp);
+      roi_body<false, LUT, CCM>(sh, p, nullptr, frame, lut, ccm, W, H, bayer, rx, ry, rw, rh, min_x, min_y, item, out, tid, lane, warp);
     }
     __syncthreads();
   }
@@ -678,8 +686,8 @@ int armors_grid(int num_sms) { return num_sms * 3; }
 size_t armors_scratch_words_per_cta(int src_w, int src_h) { return slot_words(src_w, src_h); }
 size_t armors_scratch_total_words(int src_w, int src_h, int grid) { return 64 + (size_t)grid * slot_words(src_w, src_h); }
 
-// armors_grid() runs 3 CTAs per SM: the table must leave room for them (228 KB per SM, 1 KB reserved per CTA)
-static_assert(3 * (sizeof(Shared) + 1024 + 1024) <= 228 * 1024, "raw lookup table costs the armor stage a CTA per SM");
+// armors_grid() runs 3 CTAs per SM: the tables must leave room for them (228 KB per SM, 1 KB reserved per CTA)
+static_assert(3 * (sizeof(Shared) + 1024 + kCcmBytes + 1024) <= 228 * 1024, "colour tables cost the armor stage a CTA per SM");
 
 const char *armors_geometry_error(int src_w, int src_h) {
   if (src_w < 1 || src_h < 1) return "extract_armors: the source must have at least one row and one column";
@@ -691,9 +699,10 @@ const char *armors_geometry_error(int src_w, int src_h) {
 }
 
 cudaError_t launch_extract_armors(const ArmorParams &p, cudaStream_t s) {
-  if (p.raw_lut && p.chan_order < 2) return cudaErrorInvalidValue;    // the table is defined for Bayer sources only
-  auto kernel = p.raw_lut ? extract_armors_kernel<true> : extract_armors_kernel<false>;
-  const size_t smem = sizeof(Shared) + (p.raw_lut ? 1024 : 0);
+  if ((p.raw_lut || p.ccm) && p.chan_order < 2) return cudaErrorInvalidValue;   // the tables are defined for Bayer sources only
+  auto kernel = p.ccm ? (p.raw_lut ? extract_armors_kernel<true, true> : extract_armors_kernel<false, true>)
+                      : (p.raw_lut ? extract_armors_kernel<true, false> : extract_armors_kernel<false, false>);
+  const size_t smem = sizeof(Shared) + (p.raw_lut ? 1024 : 0) + (p.ccm ? kCcmBytes : 0);
   {   // per device and cheap: no process-wide "already configured" flag (several engines / devices per process)
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;

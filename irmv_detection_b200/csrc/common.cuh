@@ -60,7 +60,30 @@ struct PreprocessParams {
   // Raw-domain colour stage of a Bayer source (irmv_engine_set_raw_lut): [2][2][256] bytes, sample s at sensor
   // position (y, x) reads as raw_lut[y & 1][x & 1][s] before anything else uses it; null = off
   const uint8_t *raw_lut;
+  // Colour-correction stage of a Bayer source (irmv_engine_set_color_matrix): a kCcmBytes device block (layout
+  // below) applied to every demosaiced pixel, after the raw table and before rot180 / resize; null = off
+  const uint8_t *ccm;
 };
+// Device block of the colour-correction stage: int32 m[3][3] (row-major, units of 1/1024) at byte 0, u8 tone[3][256]
+// at byte kCcmTone.  A demosaiced pixel (R, G, B) becomes, per output channel c,
+//   tone[c][clamp((m[c][0] R + m[c][1] G + m[c][2] B + 512) >> 10, 0, 255)]
+// (raw_lut.apply_color_matrix is the definition).  Staged in shared memory by the kernels that read it per pixel.
+constexpr int kCcmTone = 48, kCcmBytes = kCcmTone + 3 * 256;
+__device__ __forceinline__ int ccm_channel(const int *m, const uint8_t *tone, int R, int G, int B) {
+  return tone[min(max((m[0] * R + m[1] * G + m[2] * B + 512) >> 10, 0), 255)];
+}
+__device__ __forceinline__ void apply_ccm(const uint8_t *ccm, int &R, int &G, int &B) {
+  const int *m = reinterpret_cast<const int *>(ccm);
+  const uint8_t *tone = ccm + kCcmTone;
+  const int r = R, g = G, b = B;
+  R = ccm_channel(m, tone, r, g, b);
+  G = ccm_channel(m + 3, tone + 256, r, g, b);
+  B = ccm_channel(m + 6, tone + 512, r, g, b);
+}
+// Copies the block to shared memory (dst 16-byte aligned, nthreads >= kCcmBytes / 4); visible after the next barrier.
+__device__ __forceinline__ void stage_ccm(uint8_t *dst, const uint8_t *ccm, int tid) {
+  if (tid < kCcmBytes / 4) reinterpret_cast<uint32_t *>(dst)[tid] = reinterpret_cast<const uint32_t *>(ccm)[tid];
+}
 // Resize geometry of a src_w x src_h frame.  LETTERBOX (resize_mode 1) follows ultralytics'
 // LetterBox: r = min(640/w, 640/h), new = round(size * r), centred, pad value 114, pixel-centre
 // bilinear resize.  (The reference itself stretches, src/yolo_engine.cpp:186-190; north_star and
@@ -312,6 +335,7 @@ struct ArmorParams {
   int grid;
   unsigned long long *prof;             // debug: cycles summed over ROIs {bitmap, flood, walks, armor, rois, flood rounds}; null in production
   const uint8_t *raw_lut;               // [2][2][256] raw-domain colour stage of a Bayer source (PreprocessParams::raw_lut), or null
+  const uint8_t *ccm;                   // colour-correction block of a Bayer source (PreprocessParams::ccm), or null
 };
 int armors_grid(int num_sms);
 // null when the stage takes src_w x src_h frames, else why not (checked where the stage is set up, not per launch)

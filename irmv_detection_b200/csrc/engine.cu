@@ -560,6 +560,8 @@ struct irmv_engine {
   uint32_t *d_stem_tab = nullptr;        // table block of the camera-case stem (stem_bayer.cu), or null
   uint8_t *d_raw_lut = nullptr;          // [2][2][256] raw-domain colour table (irmv_engine_set_raw_lut), allocated on first use
   bool raw_lut_on = false;               // the kernels that read the raw frame apply d_raw_lut
+  uint8_t *d_ccm = nullptr;              // colour-correction block (kCcmBytes, irmv_engine_set_color_matrix), allocated on first use
+  bool ccm_on = false;                   // the kernels that demosaic the raw frame apply d_ccm
   int raw_bits = 8;                      // bits per raw sample (cfg.raw_format); > 8: every replay decodes first
   uint8_t *d_decode_lut = nullptr;       // [2][2][1 << raw_bits] table of the decode kernel (raw_bits > 8), allocated at create
   uint8_t *slot8_dev = nullptr;          // decoded slot_dev, what refresh_rotated rotates (raw_bits > 8)
@@ -1048,6 +1050,7 @@ int issue_replay(irmv_engine *e, Lane &ln, int n, cudaStream_t st, int *launches
   pp.chan_order = e->cfg.chan_order; pp.rotate180 = e->cfg.rotate180;
   pp.resize_mode = e->cfg.resize_mode; pp.quantize_u8 = e->cfg.quantize_u8;
   pp.raw_lut = e->raw_lut_on ? e->d_raw_lut : nullptr;
+  pp.ccm = e->ccm_on ? e->d_ccm : nullptr;
   if (e->fused_stem) IRMV_CUDA(launch_stem(pp, e->d_stem_w, e->d_stem_b, e->d_stem_tab, ln.stem_out.pp ? nullptr : ln.stem_out.p, ln.stem_out.pstride, ln.stem_out.pp, ln.stem_out.pp_stride, st));
   else IRMV_CUDA(launch_preprocess(pp, st));
   cnt += 1 + (ln.rotated ? 1 : 0);
@@ -1146,7 +1149,7 @@ int issue_replay(irmv_engine *e, Lane &ln, int n, cudaStream_t st, int *launches
     ap.out = ln.armors; ap.slot_locks = reinterpret_cast<int *>(ln.armor_scratch); ap.scratch = ln.armor_scratch + 64;
     ap.scratch_words_per_cta = armors_scratch_words_per_cta(e->cfg.src_width, e->cfg.src_height);
     ap.grid = armors_grid(e->num_sms);
-    ap.raw_lut = pp.raw_lut;
+    ap.raw_lut = pp.raw_lut; ap.ccm = pp.ccm;
     IRMV_CUDA(launch_extract_armors(ap, st)); ++cnt;
     if (e->pnp_on) {
       const int total = n * e->cfg.max_det;
@@ -1321,6 +1324,7 @@ int refresh_rotated(irmv_engine *e, int slot) {
   pp.src_w = e->cfg.src_width; pp.src_h = e->cfg.src_height; pp.chan_order = e->cfg.chan_order;
   pp.rotate180 = e->cfg.rotate180;
   pp.raw_lut = e->raw_lut_on ? e->d_raw_lut : nullptr;
+  pp.ccm = e->ccm_on ? e->d_ccm : nullptr;
   IRMV_CUDA(launch_rotate(pp, e->main_stream));
   IRMV_CUDA(cudaMemcpyAsync(e->rot_host[slot], e->rot_dev, (size_t)e->cfg.src_width * e->cfg.src_height * 3,
                             cudaMemcpyDeviceToHost, e->main_stream));
@@ -1701,6 +1705,7 @@ void irmv_engine_destroy(irmv_engine *e) {
   cudaFree(e->slot_dev);
   cudaFree(e->d_stem_w); cudaFree(e->d_stem_b); cudaFree(e->d_stem_tab);
   if (e->d_raw_lut) cudaFree(e->d_raw_lut);
+  if (e->d_ccm) cudaFree(e->d_ccm);
   if (e->d_decode_lut) cudaFree(e->d_decode_lut);
   if (e->slot8_dev) cudaFree(e->slot8_dev);
   if (e->batch_dev) cudaFree(e->batch_dev);
@@ -1913,6 +1918,7 @@ int irmv_debug_stem_ctas(irmv_engine *e, int *ctas) {
   pp.chan_order = e->cfg.chan_order; pp.rotate180 = e->cfg.rotate180;
   pp.resize_mode = e->cfg.resize_mode; pp.quantize_u8 = e->cfg.quantize_u8;
   pp.raw_lut = e->raw_lut_on ? e->d_raw_lut : nullptr;
+  pp.ccm = e->ccm_on ? e->d_ccm : nullptr;
   *ctas = e->fused_stem && e->d_stem_tab ? stem_bayer2x_ctas(pp) : 0;
   return 0;
   IRMV_ABI_CATCH
@@ -2147,6 +2153,42 @@ int irmv_engine_set_raw_lut(irmv_engine *e, const uint8_t *lut) {
       ln.graphs.clear();
     }
     e->raw_lut_on = on;
+  }
+  return 0;
+}
+
+// The matrix is widened to int32 and stored with the tone table (identity when none is given) in one device block
+// (common.cuh, kCcmTone / kCcmBytes).  The block is allocated once; an update rewrites it in place after the engine's
+// queued work has finished, and the graphs read it through their captured pointer.
+int irmv_engine_set_color_matrix(irmv_engine *e, const int16_t *m, const uint8_t *tone_lut) {
+  if (!e) { set_error("bad argument"); return 1; }
+  if (e->cfg.chan_order < IRMV_CH_BAYER_RGGB || e->cfg.chan_order > IRMV_CH_BAYER_GBRG) {
+    set_error("irmv_engine_set_color_matrix: the colour-correction stage applies to Bayer sources only");
+    return 2;
+  }
+  if (!m && tone_lut) {
+    set_error("irmv_engine_set_color_matrix: a tone table needs a matrix (m == NULL switches the stage off)");
+    return 1;
+  }
+  if (pipeline_busy(e)) return 5;
+  IRMV_CUDA(cudaSetDevice(e->cfg.device));
+  IRMV_CUDA(cudaDeviceSynchronize());
+  const bool on = m != nullptr;
+  if (on) {
+    uint8_t blk[kCcmBytes] = {};
+    int32_t m32[9];
+    for (int i = 0; i < 9; ++i) m32[i] = m[i];
+    memcpy(blk, m32, sizeof m32);
+    for (int i = 0; i < 3 * 256; ++i) blk[kCcmTone + i] = tone_lut ? tone_lut[i] : (uint8_t)(i & 255);
+    if (!e->d_ccm) IRMV_CUDA(dev_malloc((void **)&e->d_ccm, kCcmBytes));
+    IRMV_CUDA(cudaMemcpy(e->d_ccm, blk, kCcmBytes, cudaMemcpyHostToDevice));
+  }
+  if (on != e->ccm_on) {
+    for (auto &ln : e->lanes) {           // the kernels the replay launches changed: drop captured graphs
+      for (auto &g : ln.graphs) cudaGraphExecDestroy(g.second);
+      ln.graphs.clear();
+    }
+    e->ccm_on = on;
   }
   return 0;
 }

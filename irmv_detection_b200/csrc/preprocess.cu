@@ -131,9 +131,11 @@ __device__ __forceinline__ float finish(float v, int quantize, const float *lut)
 
 // One network-input pixel (oy, ox): rot180 + resize taps + (demosaic | channel swap) + lerp +
 // 8-bit quantisation + /255, from the staged source window.  v = {R, G, B} as fed to the net.
+// CCM: every demosaiced pixel goes through the colour-correction block `ccm` (shared memory) before the lerp.
+template <bool CCM>
 __device__ __forceinline__ void sample_pixel(const Region &reg, const PreprocessParams &p, const Taps &ty,
                                              const Taps &tx, int red_y, int red_x, const float *lut,
-                                             float (&v)[3]) {
+                                             const uint8_t *ccm, float (&v)[3]) {
   const int H = p.src_h, W = p.src_w;
   const bool bayer = p.chan_order >= 2;
   const bool swap = (p.chan_order == 1);
@@ -155,6 +157,7 @@ __device__ __forceinline__ void sample_pixel(const Region &reg, const Preprocess
       int R, G, B;
       if (bayer) {
         bayer_rgb(reg, sy, sx, H, W, red_y, red_x, R, G, B);
+        if (CCM) apply_ccm(ccm, R, G, B);
       } else {
         R = rd(reg, sy, sx * 3 + 0);
         G = rd(reg, sy, sx * 3 + 1);
@@ -231,11 +234,14 @@ __device__ __forceinline__ void apply_raw_lut(const Region &r, const uint8_t *__
   }
 }
 
-// LUT: Bayer source with a raw-domain colour table (p.raw_lut)
-template <bool LUT>
+// LUT: Bayer source with a raw-domain colour table (p.raw_lut).  CCM: Bayer source with a colour-correction block
+// (p.ccm), staged behind the source window (rows_cap * pitch_s bytes)
+template <bool LUT, bool CCM>
 __global__ void __launch_bounds__(NT)
 preprocess_kernel(PreprocessParams p, int rows_cap, int pitch_s) {
   extern __shared__ __align__(16) uint8_t smem[];
+  uint8_t *ccm = smem + (size_t)rows_cap * pitch_s;
+  if (CCM) stage_ccm(ccm, p.ccm, threadIdx.x);
   const int n = blockIdx.z;
   const int oy0 = blockIdx.y * TH, ox0 = blockIdx.x * TW;
   const bool bayer = p.chan_order >= 2;
@@ -262,7 +268,6 @@ preprocess_kernel(PreprocessParams p, int rows_cap, int pitch_s) {
     apply_raw_lut(reg, p.raw_lut, NT);
     __syncthreads();
   }
-  (void)rows_cap;
 
   int red_y = 0, red_x = 0;
   if (p.chan_order == 3) { red_y = 1; red_x = 1; }       // BGGR
@@ -273,7 +278,7 @@ preprocess_kernel(PreprocessParams p, int rows_cap, int pitch_s) {
     int oy = oy0 + q / TW, ox = ox0 + q % TW;
     if (oy >= kNet || ox >= kNet) continue;
     float v[3];
-    if (ytap[q / TW].ok && xtap[q % TW].ok) sample_pixel(reg, p, ytap[q / TW], xtap[q % TW], red_y, red_x, lut, v);
+    if (ytap[q / TW].ok && xtap[q % TW].ok) sample_pixel<CCM>(reg, p, ytap[q / TW], xtap[q % TW], red_y, red_x, lut, ccm, v);
     else v[0] = v[1] = v[2] = lut[114];                 // letterbox padding: 114 / 255
     __half2 h01 = __halves2half2(__float2half_rn(v[0]), __float2half_rn(v[1]));
     __half2 h23 = __halves2half2(__float2half_rn(v[2]), __float2half_rn(0.0f));
@@ -302,11 +307,14 @@ __device__ __forceinline__ float silu_fast(float x) {
   return fmaf(h, t, h);
 }
 
-template <bool LUT>
+// LUT / CCM: as preprocess_kernel; the colour-correction block follows the source window (smem_win bytes)
+template <bool LUT, bool CCM>
 __global__ void __launch_bounds__(ST * ST)
 stem_kernel(PreprocessParams p, const float *__restrict__ w, const float *__restrict__ bias, __half *out,
-            long long out_pstride, __half *out2, long long out2_pstride, int pitch_s, int fast_x) {
+            long long out_pstride, __half *out2, long long out2_pstride, int pitch_s, int fast_x, int smem_win) {
   extern __shared__ __align__(16) uint8_t smem[];
+  uint8_t *ccm = smem + smem_win;
+  if (CCM) stage_ccm(ccm, p.ccm, threadIdx.x);
   __shared__ __half tile[3][SI][SI + 1];             // network-input tile, already rounded to FP16
   __shared__ uint32_t sbf[16][16];                   // conv0 weights as half2 {w[n][2j], w[n][2j+1]}, K padded to 32
   __shared__ float sbias[16];
@@ -406,6 +414,7 @@ stem_kernel(PreprocessParams p, const float *__restrict__ w, const float *__rest
           R = red_row ? horiz : vert;
           B = red_row ? vert : horiz;
         }
+        if (CCM) apply_ccm(ccm, R, G, B);
       };
       // v is a convex combination of 8-bit values: no clamp needed, floor(v + 0.5) is one F2I
       auto finish_h = [&](float v) -> __half {
@@ -440,7 +449,7 @@ stem_kernel(PreprocessParams p, const float *__restrict__ w, const float *__rest
       const int iy = iy_lo + r, ix = ix_lo + c;
       float v[3] = {0.f, 0.f, 0.f};
       if (iy >= 0 && iy < kNet && ix >= 0 && ix < kNet) {
-        if (ytap[r].ok && xtap[c].ok) sample_pixel(reg, p, ytap[r], xtap[c], red_y, red_x, lut, v);
+        if (ytap[r].ok && xtap[c].ok) sample_pixel<CCM>(reg, p, ytap[r], xtap[c], red_y, red_x, lut, ccm, v);
         else v[0] = v[1] = v[2] = lut[114];             // letterbox padding: 114 / 255
       }
       tile[0][r][c] = __float2half_rn(v[0]); tile[1][r][c] = __float2half_rn(v[1]); tile[2][r][c] = __float2half_rn(v[2]);
@@ -517,7 +526,8 @@ stem_kernel(PreprocessParams p, const float *__restrict__ w, const float *__rest
 // Optional: materialise the rotated RGB frame (what get_rotated_image() exposes in the reference,
 // include/irmv_detection/yolo_engine.hpp:34) for consumers of the rotated source image.
 // LUT: Bayer source with a raw-domain colour table (p.raw_lut), applied to each of the nine raw reads.
-template <bool LUT>
+// CCM: Bayer source with a colour-correction block (p.ccm), applied to the demosaiced pixel (read through L1).
+template <bool LUT, bool CCM>
 __global__ void rotate_kernel(PreprocessParams p) {
   const bool bayer = p.chan_order >= 2;
   const int H = p.src_h, W = p.src_w, bpp = bayer ? 1 : 3;
@@ -559,6 +569,7 @@ __global__ void rotate_kernel(PreprocessParams p) {
         R = on_red_row ? horiz : vert;
         B = on_red_row ? vert : horiz;
       }
+      if (CCM) apply_ccm(p.ccm, R, G, B);
       (void)reg;
     } else {
       const uint8_t *s = frame + ((size_t)sy * W + sx) * 3;
@@ -577,8 +588,13 @@ cudaError_t launch_rotate(const PreprocessParams &p, cudaStream_t s) {
   size_t total = (size_t)p.n * p.src_h * p.src_w;
   int blocks = (int)((total + 255) / 256);
   if (blocks > 148 * 16) blocks = 148 * 16;
-  if (p.raw_lut) rotate_kernel<true><<<blocks, 256, 0, s>>>(p);
-  else rotate_kernel<false><<<blocks, 256, 0, s>>>(p);
+  if (p.ccm) {
+    if (p.raw_lut) rotate_kernel<true, true><<<blocks, 256, 0, s>>>(p);
+    else rotate_kernel<false, true><<<blocks, 256, 0, s>>>(p);
+  } else {
+    if (p.raw_lut) rotate_kernel<true, false><<<blocks, 256, 0, s>>>(p);
+    else rotate_kernel<false, false><<<blocks, 256, 0, s>>>(p);
+  }
   return cudaGetLastError();
 }
 
@@ -594,8 +610,10 @@ cudaError_t launch_preprocess(const PreprocessParams &p_in, cudaStream_t s) {
   int pitch_s = ((cols_cap * bpp + 15) / 16 + 2) * 16;   // +1 chunk for the alignment shift
   size_t smem = (size_t)rows_cap * pitch_s;
   if (smem > 200 * 1024) return cudaErrorInvalidValue;
-  if (p.raw_lut && !bayer) return cudaErrorInvalidValue;       // the table is defined for Bayer sources only
-  auto kernel = p.raw_lut ? preprocess_kernel<true> : preprocess_kernel<false>;
+  if ((p.raw_lut || p.ccm) && !bayer) return cudaErrorInvalidValue;   // the tables are defined for Bayer sources only
+  auto kernel = p.ccm ? (p.raw_lut ? preprocess_kernel<true, true> : preprocess_kernel<false, true>)
+                      : (p.raw_lut ? preprocess_kernel<true, false> : preprocess_kernel<false, false>);
+  if (p.ccm) smem += kCcmBytes;
   if (smem > 48 * 1024) {                 // per device, cheap: no process-wide flag
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
@@ -618,15 +636,18 @@ cudaError_t launch_stem(const PreprocessParams &p_in, const float *w, const floa
     return e == cudaSuccess ? launch_rotate(p, s) : e;
   }
   const bool bayer = p.chan_order >= 2;
-  if (p.raw_lut && !bayer) return cudaErrorInvalidValue;
+  if ((p.raw_lut || p.ccm) && !bayer) return cudaErrorInvalidValue;
   const int bpp = bayer ? 1 : 3;
   const float sx = (float)p.src_w / p.new_w, sy = (float)p.src_h / p.new_h;
   int rows_cap = (int)(SI * sy) + 4 + (bayer ? 4 : 0);
   int cols_cap = (int)(SI * sx) + 4 + (bayer ? 4 : 0);
   int pitch_s = ((cols_cap * bpp + 15) / 16 + 2) * 16;
-  size_t smem = (size_t)rows_cap * pitch_s;
+  const int smem_win = rows_cap * pitch_s;
+  size_t smem = (size_t)smem_win;
   if (smem > 160 * 1024) return cudaErrorInvalidValue;
-  auto kernel = p.raw_lut ? stem_kernel<true> : stem_kernel<false>;
+  auto kernel = p.ccm ? (p.raw_lut ? stem_kernel<true, true> : stem_kernel<false, true>)
+                      : (p.raw_lut ? stem_kernel<true, false> : stem_kernel<false, false>);
+  if (p.ccm) smem += kCcmBytes;
   if (smem > 30 * 1024) {
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
@@ -634,7 +655,7 @@ cudaError_t launch_stem(const PreprocessParams &p_in, const float *w, const floa
   dim3 grid(kNet / 2 / ST, kNet / 2 / ST, p.n);
   // integer horizontal scale without half-pixel centres: every second x tap has weight exactly 0
   const int fast_x = (p.src_w % kNet == 0) && p.resize_mode == 0;
-  kernel<<<grid, ST * ST, smem, s>>>(p, w, bias, out, out_pstride, out2, out2_pstride, pitch_s, fast_x);
+  kernel<<<grid, ST * ST, smem, s>>>(p, w, bias, out, out_pstride, out2, out2_pstride, pitch_s, fast_x, smem_win);
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? launch_rotate(p, s) : e;
 }

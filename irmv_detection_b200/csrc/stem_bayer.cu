@@ -59,7 +59,14 @@ struct StemBayerArgs {
   __half *out; long long out_ps;         // normal layout (may be null)
   __half *out2; long long out2_ps;       // parity-split twin (may be null)
   const uint8_t *raw_lut;                // [2][2][256] raw-domain colour stage (PreprocessParams::raw_lut), LUT instantiations only
+  const uint8_t *ccm;                    // colour-correction block (PreprocessParams::ccm), LUT == LUT_COLOUR only
 };
+
+// Table modes of the Bayer instantiations (template parameter LUT): no table, the raw table, the raw table (when one
+// is set) and the colour-correction stage.  Dynamic shared memory each mode adds behind the lerp table:
+constexpr int LUT_NONE = 0, LUT_RAW = 1, LUT_COLOUR = 2;
+constexpr size_t lut_bytes(int lut) { return lut == LUT_NONE ? 0 : lut == LUT_RAW ? 1024 : 1024 + kCcmBytes; }
+int lut_mode(const PreprocessParams &p) { return p.ccm ? LUT_COLOUR : p.raw_lut ? LUT_RAW : LUT_NONE; }
 
 // Device table block (built once per engine, stem_bayer2x_tables):
 //   TAB_BFRAG  conv0 B fragments per lane [32][8]: weights * 0.5 as FP16 pairs, K ordered (ky, 3 px x 3 ch + pad)
@@ -102,9 +109,11 @@ __device__ __forceinline__ Px3 unpack(const uint32_t *rowj) {
 }
 
 // OUT1 / OUT2: write the normal layout / the parity-split twin (exactly one of them).
-// LUT (Bayer formats only): the staged rows go through the raw-domain colour table before the demosaic; the
-// [2][2][256]-byte table sits in shared memory between the lerp table and the staged rows.
-template <bool ROT, int FMT, bool OUT1, bool OUT2, bool LUT>
+// LUT (Bayer formats only): LUT_RAW: the staged rows go through the raw-domain colour table before the demosaic; the
+// [2][2][256]-byte table sits in shared memory between the lerp table and the staged rows.  LUT_COLOUR: the same
+// (when a.raw_lut is set), and every demosaiced pixel goes through the colour-correction stage before the vertical
+// lerp; its block (kCcmBytes) sits behind the raw table.
+template <bool ROT, int FMT, bool OUT1, bool OUT2, int LUT>
 __global__ void __launch_bounds__(NTHREADS, 2) stem_bayer2x_kernel(const __grid_constant__ StemBayerArgs a) {
   constexpr int OROWS = orows_for(FMT), NIR = 2 * OROWS + 1, RP = row_pitch(FMT), STRIP_WORDS = strip_words(OROWS);
   constexpr bool PACKED = FMT >= FMT_RGB, RED_COL = FMT == FMT_BAYER_REDCOL;
@@ -113,7 +122,8 @@ __global__ void __launch_bounds__(NTHREADS, 2) stem_bayer2x_kernel(const __grid_
   uint32_t *tile_w = reinterpret_cast<uint32_t *>(smem);                       // [NIR][PITCHW]
   uint8_t *lut = smem + (size_t)NIR * PITCHW * 4;                              // [lut_n] halves
   uint8_t *rlut = smem + (((size_t)NIR * PITCHW * 4 + (size_t)a.lut_n * 2 + 15) & ~(size_t)15);  // [2][2][256] (LUT)
-  uint8_t *raw = rlut + (LUT ? 1024 : 0);                                                        // [nr][RP]
+  uint8_t *ccm = rlut + 1024;                                                                    // (LUT_COLOUR)
+  uint8_t *raw = rlut + lut_bytes(LUT);                                                          // [nr][RP]
   __shared__ __align__(16) RowTab rowtab[NIR];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int H = a.H;
@@ -146,7 +156,9 @@ __global__ void __launch_bounds__(NTHREADS, 2) stem_bayer2x_kernel(const __grid_
     uint32_t *sl = reinterpret_cast<uint32_t *>(lut);
     for (int i = tid; i < (a.lut_n + 1) / 2; i += NTHREADS) sl[i] = gl[i];
   }
-  if (LUT && tid < 256) reinterpret_cast<uint32_t *>(rlut)[tid] = reinterpret_cast<const uint32_t *>(a.raw_lut)[tid];
+  const bool raw_lut = LUT == LUT_RAW || (LUT == LUT_COLOUR && a.raw_lut);
+  if (raw_lut && tid < 256) reinterpret_cast<uint32_t *>(rlut)[tid] = reinterpret_cast<const uint32_t *>(a.raw_lut)[tid];
+  if (LUT == LUT_COLOUR) stage_ccm(ccm, a.ccm, tid);
   if (tid < NIR) {
     reinterpret_cast<uint4 *>(rowtab)[tid] = reinterpret_cast<const uint4 *>(strip + 4)[tid];
     // conv padding of the tile: column 0 (ix = -1) and the pad half behind the last pixel
@@ -156,7 +168,7 @@ __global__ void __launch_bounds__(NTHREADS, 2) stem_bayer2x_kernel(const __grid_
   }
   asm volatile("cp.async.wait_all;" ::: "memory");
   __syncthreads();
-  if (LUT) {
+  if (raw_lut) {
     // raw-domain colour stage, in place: a sample of sensor row y, column x becomes rlut[y & 1][x & 1][s].  The
     // parity is that of the row and column actually read; reflect-101 keeps a mirrored sample on its colour site
     // (column -1 holds column 1, column SW holds column SW - 2).
@@ -246,8 +258,20 @@ __global__ void __launch_bounds__(NTHREADS, 2) stem_bayer2x_kernel(const __grid_
       }
       // site row: own colour at the centre, green = cross, the other colour = diagonal; green row on a
       // red row (RED_COL == false): R horizontal, B vertical; on a blue row: R vertical, B horizontal
-      const uint32_t RS = RED_COL ? cS : diag, BS = RED_COL ? diag : cS;
-      const uint32_t RG = RED_COL ? vert : horiz, BG = RED_COL ? horiz : vert;
+      uint32_t RS = RED_COL ? cS : diag, BS = RED_COL ? diag : cS;
+      uint32_t RG = RED_COL ? vert : horiz, BG = RED_COL ? horiz : vert;
+      if (LUT == LUT_COLOUR) {
+        // colour-correction stage on the four demosaiced pixels (two lanes of the site row and of the green row)
+        auto cc = [&](uint32_t &r, uint32_t &g, uint32_t &b) {
+          int r0 = (int)(r & 0xffffu), g0 = (int)(g & 0xffffu), b0 = (int)(b & 0xffffu);
+          int r1 = (int)(r >> 16), g1 = (int)(g >> 16), b1 = (int)(b >> 16);
+          apply_ccm(ccm, r0, g0, b0);
+          apply_ccm(ccm, r1, g1, b1);
+          r = (uint32_t)r0 | ((uint32_t)r1 << 16); g = (uint32_t)g0 | ((uint32_t)g1 << 16); b = (uint32_t)b0 | ((uint32_t)b1 << 16);
+        };
+        cc(RS, cross, BS);
+        cc(RG, cG, BG);
+      }
       xr = RS * wS + RG * wG + QQ;
       xg = cross * wS + cG * wG + QQ;
       xb = BS * wS + BG * wG + QQ;
@@ -351,7 +375,7 @@ __global__ void __launch_bounds__(NTHREADS, 2) stem_bayer2x_kernel(const __grid_
 }
 
 
-template <bool ROT, int FMT, bool OUT1, bool OUT2, bool LUT>
+template <bool ROT, int FMT, bool OUT1, bool OUT2, int LUT>
 cudaError_t launch_o(const StemBayerArgs &a, size_t smem, cudaStream_t s) {
   cudaError_t e = cudaFuncSetAttribute(stem_bayer2x_kernel<ROT, FMT, OUT1, OUT2, LUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
@@ -364,15 +388,19 @@ template <bool ROT, int FMT>
 cudaError_t launch_t(const StemBayerArgs &a, size_t smem, cudaStream_t s) {
   if (!a.out == !a.out2) return cudaErrorInvalidValue;   // exactly one layout
   if constexpr (FMT < FMT_RGB) {
+    if (a.ccm) {                                       // raw table (if any) and colour block behind the lerp table
+      if (a.out2) return launch_o<ROT, FMT, false, true, LUT_COLOUR>(a, smem + lut_bytes(LUT_COLOUR), s);
+      return launch_o<ROT, FMT, true, false, LUT_COLOUR>(a, smem + lut_bytes(LUT_COLOUR), s);
+    }
     if (a.raw_lut) {                                   // the table's 1 KB sits behind the lerp table
-      if (a.out2) return launch_o<ROT, FMT, false, true, true>(a, smem + 1024, s);
-      return launch_o<ROT, FMT, true, false, true>(a, smem + 1024, s);
+      if (a.out2) return launch_o<ROT, FMT, false, true, LUT_RAW>(a, smem + 1024, s);
+      return launch_o<ROT, FMT, true, false, LUT_RAW>(a, smem + 1024, s);
     }
   } else {
-    if (a.raw_lut) return cudaErrorInvalidValue;       // the table is defined for Bayer sources only
+    if (a.raw_lut || a.ccm) return cudaErrorInvalidValue;   // the tables are defined for Bayer sources only
   }
-  if (a.out2) return launch_o<ROT, FMT, false, true, false>(a, smem, s);
-  return launch_o<ROT, FMT, true, false, false>(a, smem, s);
+  if (a.out2) return launch_o<ROT, FMT, false, true, LUT_NONE>(a, smem, s);
+  return launch_o<ROT, FMT, true, false, LUT_NONE>(a, smem, s);
 }
 
 template <bool ROT>
@@ -400,7 +428,7 @@ int nr_max_for(int P, int Q, int fmt) { return (2 * orows_for(fmt) * P + Q - 1) 
 
 constexpr size_t kMaxSmem = 227 * 1024;  // dynamic shared memory a block may have on sm_100
 
-// dynamic shared memory of a launch without the raw table: tile + lerp table, then the staged rows
+// dynamic shared memory of a launch without the tables: tile + lerp table, then the staged rows
 size_t smem_for(int H, int fmt) {
   const int g = gcd_i(H, kNet), P = H / g, Q = kNet / g;
   const size_t lut_n = 2 * Q * 255 + Q + 1;
@@ -410,8 +438,8 @@ size_t smem_for(int H, int fmt) {
 
 // CTAs per SM with `smem` bytes of dynamic shared memory.  Every instantiation of a format has the same static
 // shared memory, and __launch_bounds__(NTHREADS, 2) keeps the registers of two CTAs within an SM's file, so the
-// answer depends on the format, the table and smem only.
-template <int FMT, bool LUT>
+// answer depends on the format, the table mode and smem only.
+template <int FMT, int LUT>
 int ctas_per_sm(size_t smem) {
   auto k = stem_bayer2x_kernel<false, FMT, true, false, LUT>;
   int n = 0;
@@ -423,13 +451,22 @@ int ctas_per_sm(size_t smem) {
   return n;
 }
 
-int ctas_for(int fmt, bool lut, size_t smem) {
+// CTAs per SM in table mode `lut`; smem is the dynamic shared memory without the tables
+template <int FMT>
+int ctas_bayer(int lut, size_t smem) {
+  switch (lut) {
+    case LUT_NONE: return ctas_per_sm<FMT, LUT_NONE>(smem);
+    case LUT_RAW: return ctas_per_sm<FMT, LUT_RAW>(smem + lut_bytes(LUT_RAW));
+    default: return ctas_per_sm<FMT, LUT_COLOUR>(smem + lut_bytes(LUT_COLOUR));
+  }
+}
+
+int ctas_for(int fmt, int lut, size_t smem) {
   switch (fmt) {
-    case FMT_BAYER: return lut ? ctas_per_sm<FMT_BAYER, true>(smem + 1024) : ctas_per_sm<FMT_BAYER, false>(smem);
-    case FMT_BAYER_REDCOL:
-      return lut ? ctas_per_sm<FMT_BAYER_REDCOL, true>(smem + 1024) : ctas_per_sm<FMT_BAYER_REDCOL, false>(smem);
-    case FMT_RGB: return lut ? 0 : ctas_per_sm<FMT_RGB, false>(smem);
-    default: return lut ? 0 : ctas_per_sm<FMT_BGR, false>(smem);
+    case FMT_BAYER: return ctas_bayer<FMT_BAYER>(lut, smem);
+    case FMT_BAYER_REDCOL: return ctas_bayer<FMT_BAYER_REDCOL>(lut, smem);
+    case FMT_RGB: return lut ? 0 : ctas_per_sm<FMT_RGB, LUT_NONE>(smem);
+    default: return lut ? 0 : ctas_per_sm<FMT_BGR, LUT_NONE>(smem);
   }
 }
 
@@ -438,24 +475,26 @@ int ctas_for(int fmt, bool lut, size_t smem) {
 // The fast path applies to: 8-bit Bayer or packed u8x3 source of width 1280, height >= 640 with
 // H/640 = P/Q, Q <= 16, reference resize (corner-aligned stretch) and the 8-bit intermediate, when its shared
 // memory fits a block: packed sources of 3400 rows and more stage rows three times as long and do not.  With a raw
-// table (p.raw_lut) its 1 KB must also keep the CTAs per SM of the launch without it (the kernel is sized for two at
-// the camera's 1024 rows, where about 2.5 KB per CTA are left); where it would cost one, stem_kernel runs instead,
-// at its full occupancy.  Called without a table at engine creation (no device query) and with it at every launch.
+// table (p.raw_lut, 1 KB) or the colour-correction stage (p.ccm, 1 KB + kCcmBytes) the tables must also keep the
+// CTAs per SM of the launch without them (the kernel is sized for two at the camera's 1024 rows, where about 2.5 KB
+// per CTA are left); where they would cost one, stem_kernel runs instead, at its full occupancy.  Called without
+// tables at engine creation (no device query) and with them at every launch.
 bool stem_bayer2x_applies(const PreprocessParams &p) {
   if (p.chan_order < 0 || p.chan_order > 5 || p.src_w != SW || p.resize_mode != 0 || !p.quantize_u8 || p.src_h < kNet || p.src_h > 4096) return false;
   const int g = gcd_i(p.src_h, kNet);
   if (kNet / g > 16) return false;
   const int fmt = format_of(p.chan_order, p.rotate180);
   const size_t smem = smem_for(p.src_h, fmt);
-  if (!p.raw_lut) return smem <= kMaxSmem;
-  if (fmt >= FMT_RGB || smem + 1024 > kMaxSmem) return false;
-  return ctas_for(fmt, true, smem) >= ctas_for(fmt, false, smem);
+  const int lut = lut_mode(p);
+  if (lut == LUT_NONE) return smem <= kMaxSmem;
+  if (fmt >= FMT_RGB || smem + lut_bytes(lut) > kMaxSmem) return false;
+  return ctas_for(fmt, lut, smem) >= ctas_for(fmt, LUT_NONE, smem);
 }
 
 int stem_bayer2x_ctas(const PreprocessParams &p) {
   if (!stem_bayer2x_applies(p)) return 0;
   const int fmt = format_of(p.chan_order, p.rotate180);
-  return ctas_for(fmt, p.raw_lut != nullptr, smem_for(p.src_h, fmt));
+  return ctas_for(fmt, lut_mode(p), smem_for(p.src_h, fmt));
 }
 
 // Host side of the table block (layout above): conv0 weights w[16][9 taps][3] and bias[16] as the engine
@@ -539,9 +578,9 @@ cudaError_t launch_stem_bayer2x(const PreprocessParams &p, int frame0, const uin
   a.Q = Q; a.lut_n = 2 * Q * 255 + Q + 1;
   a.tab_strip = TAB_LUT + (a.lut_n + 7) / 8 * 4;
   a.tab = tab; a.out = out; a.out_ps = out_ps; a.out2 = out2; a.out2_ps = out2_ps;
-  a.raw_lut = p.raw_lut;
+  a.raw_lut = p.raw_lut; a.ccm = p.ccm;
   const size_t smem = smem_for(p.src_h, fmt);
-  if (smem + (p.raw_lut ? 1024 : 0) > kMaxSmem) return cudaErrorInvalidValue;
+  if (smem + lut_bytes(lut_mode(p)) > kMaxSmem) return cudaErrorInvalidValue;
   return p.rotate180 ? launch_f<true>(fmt, a, smem, s) : launch_f<false>(fmt, a, smem, s);
 }
 

@@ -290,6 +290,23 @@ class YoloEngine:
         lut = np.ascontiguousarray(lut)
         L.check(self._lib.irmv_engine_set_raw_lut(self._h, lut.ctypes.data), "irmv_engine_set_raw_lut")
 
+    def set_color_matrix(self, m: Optional[np.ndarray], tone: Optional[np.ndarray] = None) -> None:
+        """Colour-correction stage of a Bayer engine: `m` is a (3, 3) int16 matrix in units of 1/1024 and `tone` a
+        (3, 256) uint8 output tone table or None (identity), applied to every demosaiced pixel after the raw table
+        (or the 10/12-bit decode) and before rot180 and resize; m None switches the stage off (tone must be None
+        then).  The engine with M and T on Bayer frames F returns what a PASSTHROUGH engine returns on the packed
+        frames raw_lut.apply_color_matrix(demosaic_bilinear(F), M, T).  raw_lut.color_matrix_q10 builds M from a
+        colour-correction matrix and a saturation gain; raw_lut.make_raw_lut(0, (1, 1, 1), gamma) is a tone table."""
+        from . import raw_lut as R
+        mp = tp = None
+        if m is not None:
+            m = np.ascontiguousarray(R._check_matrix(m))
+            mp = m.ctypes.data
+        if tone is not None:
+            tone = np.ascontiguousarray(R._check_tone(tone))
+            tp = tone.ctypes.data
+        L.check(self._lib.irmv_engine_set_color_matrix(self._h, mp, tp), "irmv_engine_set_color_matrix")
+
     def fetch_armors(self, n: int, ticket: int = -1) -> np.ndarray:
         """Armors of the last synchronous call (or of a collected ticket): structured [n, max_det]."""
         out = np.zeros((n, self.max_det), ARMOR_DTYPE)

@@ -8,6 +8,10 @@ on the camera's ISP.
 decode_raw is the same definition for 10- and 12-bit sources (raw_format RAW_10, RAW_12, RAW_12_PACKED): a b-bit
 engine with table T on frames F returns, bit for bit, what an otherwise identical 8-bit engine without a table
 returns on decode_raw(F, raw_format, T, pattern).
+
+apply_color_matrix is the definition of the colour-correction stage that follows the demosaic (set_color_matrix):
+a 3x3 integer matrix and an output tone table; color_matrix_q10 builds the matrix from a colour-correction matrix and
+a saturation gain.
 """
 from __future__ import annotations
 
@@ -99,7 +103,11 @@ def make_raw_lut(black_level: int = 0, gains: Sequence[float] = (1.0, 1.0, 1.0),
                  bits: int = 8) -> np.ndarray:
     """u8 [3, 2^bits] table of the usual ISP chain per colour site, from bits-bit samples to 8-bit values: subtract
     the black level (in units of that bit depth), rescale to the full range 2^bits - 1 - black, apply the channel's
-    white-balance gain, clip, apply the tone curve x ** gamma, round half up."""
+    white-balance gain, clip, apply the tone curve x ** gamma, round half up.
+
+    make_raw_lut(0, (1, 1, 1), gamma) is also the output tone table of the colour-correction stage
+    (apply_color_matrix, set_color_matrix): an ISP applies black level and gains before the matrix and gamma after
+    it, so the raw table then keeps gamma 1."""
     top = (1 << bits) - 1
     v = np.arange(top + 1, dtype=np.float64)
     x = np.clip(v - black_level, 0.0, None) / (float(top) - black_level)
@@ -108,3 +116,57 @@ def make_raw_lut(black_level: int = 0, gains: Sequence[float] = (1.0, 1.0, 1.0),
         y = np.clip(x * float(gains[c]), 0.0, 1.0) ** float(gamma)
         out[c] = np.floor(y * 255.0 + 0.5).astype(np.uint8)
     return out
+
+
+# BT.601 luma weights of R, G, B: the grey axis a saturation gain keeps fixed
+LUMA_BT601 = (0.299, 0.587, 0.114)
+
+
+def apply_color_matrix(rgb: np.ndarray, m: np.ndarray, tone: Optional[np.ndarray] = None) -> np.ndarray:
+    """Colour-correction stage of Bayer sources (YoloEngine.set_color_matrix, irmv_engine_set_color_matrix).
+    rgb u8 [..., 3] is the demosaiced frame (oracle.preprocess_ref.demosaic_bilinear, after the raw table or the
+    10/12-bit decode, before rot180 and resize); m is int16 [3, 3], row-major, in units of 1/1024; tone is u8
+    [3, 256] or None (identity).  For every pixel and output channel c:
+        v_c = sum_k m[c][k] * in_k                     (int32)
+        o_c = clamp(floor((v_c + 512) / 1024), 0, 255)
+        out_c = tone[c][o_c]
+    The engine with matrix M and tone T on Bayer frames F returns, bit for bit, what a PASSTHROUGH engine returns
+    on the packed frames apply_color_matrix(demosaic_bilinear(F), M, T).  Returns a new u8 array."""
+    rgb = np.asarray(rgb)
+    if rgb.dtype != np.uint8 or rgb.ndim < 1 or rgb.shape[-1] != 3:
+        raise ValueError("rgb must be uint8 [..., 3]")
+    m = _check_matrix(m)
+    tone = _check_tone(tone)
+    v = rgb.astype(np.int32) @ m.astype(np.int32).T
+    o = np.clip((v + 512) >> 10, 0, 255)
+    if tone is None:
+        return o.astype(np.uint8)
+    return tone[np.arange(3), o]
+
+
+def color_matrix_q10(ccm: Optional[np.ndarray] = None, saturation: float = 1.0) -> np.ndarray:
+    """int16 [3, 3] matrix of the colour-correction stage: rint(1024 * S @ ccm), clipped to the int16 range, with
+    ccm a float [3, 3] colour-correction matrix (None: identity) and S = s*I + (1 - s) * 1 * luma^T the saturation
+    gain s about the BT.601 grey axis (s = 0 maps every pixel to its luma, s > 1 pushes colours apart)."""
+    c = np.eye(3) if ccm is None else np.asarray(ccm, np.float64)
+    if c.shape != (3, 3):
+        raise ValueError("ccm must be 3 x 3")
+    s = float(saturation)
+    S = s * np.eye(3) + (1.0 - s) * np.outer(np.ones(3), LUMA_BT601)
+    return np.clip(np.rint(1024.0 * (S @ c)), -32768, 32767).astype(np.int16)
+
+
+def _check_matrix(m) -> np.ndarray:
+    m = np.asarray(m)
+    if m.shape != (3, 3) or m.dtype != np.int16:
+        raise ValueError("the colour matrix must be a (3, 3) int16 array")
+    return m
+
+
+def _check_tone(tone) -> Optional[np.ndarray]:
+    if tone is None:
+        return None
+    tone = np.asarray(tone)
+    if tone.shape != (3, 256) or tone.dtype != np.uint8:
+        raise ValueError("the tone table must be a (3, 256) uint8 array or None")
+    return tone
