@@ -514,6 +514,18 @@ __global__ void quads_from_kpts_kernel(const int32_t *num, const float *kpts, in
 
 using namespace irmv;
 
+// Camera and armor constants of the pose kernels, for the stand-alone solver and the engine's pose stage.
+// K row-major 3x3, D = (k1, k2, p1, p2, k3) (reference src/pnp_solver.cpp:10-15); armor half extents in
+// metres (reference include/irmv_detection/pnp_solver.hpp:30-33, src/pnp_solver.cpp:18-21).
+static PnpConsts pnp_consts(const double K[9], const double D[5]) {
+  PnpConsts c{};
+  c.fx = K[0]; c.cx = K[2]; c.fy = K[4]; c.cy = K[5];
+  c.k1 = D[0]; c.k2 = D[1]; c.p1 = D[2]; c.p2 = D[3]; c.k3 = D[4];
+  c.half_w[0] = 135.0 / 2.0 / 1000.0; c.half_h[0] = 55.0 / 2.0 / 1000.0;
+  c.half_w[1] = 225.0 / 2.0 / 1000.0; c.half_h[1] = 55.0 / 2.0 / 1000.0;
+  return c;
+}
+
 constexpr int kSets = 3;    // batches in flight in the pipelined hand-off
 
 struct irmv_engine {
@@ -2011,10 +2023,7 @@ int irmv_engine_read_kept_indices(irmv_engine *e, int frame, int32_t *idx, int c
 
 int irmv_engine_enable_pnp(irmv_engine *e, const double K[9], const double D[5], float corner_sx, float corner_sy) {
   if (!e || !K || !D) { set_error("bad argument"); return 1; }
-  e->pnp_c.fx = K[0]; e->pnp_c.cx = K[2]; e->pnp_c.fy = K[4]; e->pnp_c.cy = K[5];
-  e->pnp_c.k1 = D[0]; e->pnp_c.k2 = D[1]; e->pnp_c.p1 = D[2]; e->pnp_c.p2 = D[3]; e->pnp_c.k3 = D[4];
-  e->pnp_c.half_w[0] = 135.0 / 2.0 / 1000.0; e->pnp_c.half_h[0] = 55.0 / 2.0 / 1000.0;
-  e->pnp_c.half_w[1] = 225.0 / 2.0 / 1000.0; e->pnp_c.half_h[1] = 55.0 / 2.0 / 1000.0;
+  e->pnp_c = pnp_consts(K, D);
   // boxes are in network pixels: first to the source frame (parse_output's scale), then to the calibration frame
   {
     int pad_x, pad_y, new_w, new_h;
@@ -2599,12 +2608,7 @@ int irmv_pnp_create(const double K[9], const double D[5], int device, irmv_pnp *
   IRMV_CUDA(cudaSetDevice(device));
   std::unique_ptr<irmv_pnp> p(new irmv_pnp);
   p->device = device;
-  // reference src/pnp_solver.cpp:10-15: K row-major 3x3, D first five coefficients
-  p->c.fx = K[0]; p->c.cx = K[2]; p->c.fy = K[4]; p->c.cy = K[5];
-  p->c.k1 = D[0]; p->c.k2 = D[1]; p->c.p1 = D[2]; p->c.p2 = D[3]; p->c.k3 = D[4];
-  // reference include/irmv_detection/pnp_solver.hpp:30-33 (mm) and src/pnp_solver.cpp:18-21
-  p->c.half_w[0] = 135.0 / 2.0 / 1000.0; p->c.half_h[0] = 55.0 / 2.0 / 1000.0;
-  p->c.half_w[1] = 225.0 / 2.0 / 1000.0; p->c.half_h[1] = 55.0 / 2.0 / 1000.0;
+  p->c = pnp_consts(K, D);
   IRMV_CUDA(cudaStreamCreateWithFlags(&p->stream, cudaStreamNonBlocking));
   IRMV_CUDA(cudaEventCreate(&p->ev0));
   IRMV_CUDA(cudaEventCreate(&p->ev1));

@@ -2,10 +2,10 @@
 // Replaces the per-armor CPU cv::solvePnP(..., SOLVEPNP_IPPE) call of the reference
 // (reference src/pnp_solver.cpp:36-52) and, optionally, the Rodrigues -> tf2 quaternion step of
 // the caller (reference src/irm_detector.cpp:218-226).  Algorithm = oracle/pnp_ref.py:
-// undistort (5 fixed-point iterations, result rounded to FP32 like cv::undistortPoints with
-// Point2f input), exact rectangle->quad homography, IPPE two-rotation solve, linear-LSQ
-// translation, sort by normalised reprojection RMSE, rot2vec.  No LM refinement (the
-// reference's call has none, SURVEY.md section 0.6).
+// undistort (5 fixed-point iterations, stopping at the initial guess where icdist < 0, result
+// rounded to FP32 like cv::undistortPoints with Point2f input), exact rectangle->quad
+// homography, IPPE two-rotation solve, linear-LSQ translation, sort by normalised reprojection
+// RMSE, rot2vec.  No LM refinement (the reference's call has none, SURVEY.md section 0.6).
 //
 // 80 algorithmic bytes per armor (32 in, 48 out) against ~2.5 kFLOP of dependent FP64 math:
 // the kernel is FP64-latency bound, so the mapping is one armor per thread with enough
@@ -90,7 +90,8 @@ __global__ void __launch_bounds__(128) pnp_kernel(PnpConsts C, const float *__re
     for (int it = 0; it < 5; ++it) {
       double r2 = x * x + y * y;
       double icd = 1.0 / (1.0 + ((C.k3 * r2 + C.k2) * r2 + C.k1) * r2);
-      if (icd < 0.0) { x = x0; y = y0; continue; }
+      // past the radius where the radial polynomial can be inverted: OpenCV stops and keeps (x0, y0)
+      if (icd < 0.0) { x = x0; y = y0; break; }
       double dx = 2.0 * C.p1 * x * y + C.p2 * (r2 + 2.0 * x * x);
       double dy = C.p1 * (r2 + 2.0 * y * y) + 2.0 * C.p2 * x * y;
       x = (x0 - dx) * icd;

@@ -57,9 +57,14 @@ def armor_object_points(large: bool = False) -> np.ndarray:
     return np.array([[0, hw, -hh], [0, hw, hh], [0, -hw, hh], [0, -hw, -hh]], np.float64)
 
 
-def armor_quads(n: int, seed: int = 0, noise_px: float = 0.5, K=K_CAMERA, D=D_CAMERA, img_w: int = 640, img_h: int = 480):
-    """SURVEY.md section 8d config 5 input: seeded armor poses (0.5-8 m, yaw +-60, pitch +-30, roll +-15 degrees)
-    projected through K/D with N(0, noise_px) pixel noise, kept inside the image: f32 [n, 4, 2].
+def armor_quads(n: int, seed: int = 0, noise_px: float = 0.5, K=K_CAMERA, D=D_CAMERA, img_w: int = 640, img_h: int = 480,
+                dist=(0.5, 8.0), yaw: float = 60.0, pitch: float = 30.0, roll: float = 15.0, margin: float = 0.15,
+                large: bool = False):
+    """SURVEY.md section 8d config 5 input: seeded armor poses (distance uniform in `dist` metres, yaw, pitch and roll
+    uniform in +-`yaw`, +-`pitch`, +-`roll` degrees) projected through K/D with N(0, noise_px) pixel noise, kept inside
+    the image: f32 [n, 4, 2].  The armor centre aims at a pixel drawn at least `margin` (a fraction of the frame)
+    from each edge; `large` selects the large armor.  The defaults are the survey's envelope, and the same seed
+    gives the same quads as before these arguments existed.
 
     Model frame is x-forward/y-left/z-up; the camera looks along +z, so the base rotation maps model x ->
     camera z, model y -> camera -x, model z -> camera -y."""
@@ -68,22 +73,23 @@ def armor_quads(n: int, seed: int = 0, noise_px: float = 0.5, K=K_CAMERA, D=D_CA
     Km = np.asarray(K, np.float64).reshape(3, 3)
     Dm = np.asarray(D, np.float64).reshape(1, 5)
     base = np.array([[0.0, -1.0, 0.0], [0.0, 0.0, -1.0], [1.0, 0.0, 0.0]])
-    obj = armor_object_points(False)
+    obj = armor_object_points(large)
     out = np.empty((n, 4, 2), np.float32)
     i = 0
     while i < n:
-        dist = rng.uniform(0.5, 8.0)
-        yaw, pitch, roll = np.deg2rad(rng.uniform(-60, 60)), np.deg2rad(rng.uniform(-30, 30)), np.deg2rad(rng.uniform(-15, 15))
-        cy, sy = np.cos(yaw), np.sin(yaw)
-        cp, sp = np.cos(pitch), np.sin(pitch)
-        cr, sr = np.cos(roll), np.sin(roll)
+        d = rng.uniform(dist[0], dist[1])
+        ya, pi, ro = (np.deg2rad(rng.uniform(-yaw, yaw)), np.deg2rad(rng.uniform(-pitch, pitch)),
+                      np.deg2rad(rng.uniform(-roll, roll)))
+        cy, sy = np.cos(ya), np.sin(ya)
+        cp, sp = np.cos(pi), np.sin(pi)
+        cr, sr = np.cos(ro), np.sin(ro)
         Ry = np.array([[cy, 0, sy], [0, 1, 0], [-sy, 0, cy]])
         Rx = np.array([[1, 0, 0], [0, cp, -sp], [0, sp, cp]])
         Rz = np.array([[cr, -sr, 0], [sr, cr, 0], [0, 0, 1]])
         R = Rz @ Rx @ Ry @ base
-        u = rng.uniform(0.15, 0.85) * img_w
-        v = rng.uniform(0.15, 0.85) * img_h
-        t = np.array([(u - Km[0, 2]) / Km[0, 0] * dist, (v - Km[1, 2]) / Km[1, 1] * dist, dist])
+        u = rng.uniform(margin, 1.0 - margin) * img_w
+        v = rng.uniform(margin, 1.0 - margin) * img_h
+        t = np.array([(u - Km[0, 2]) / Km[0, 0] * d, (v - Km[1, 2]) / Km[1, 1] * d, d])
         rvec, _ = cv2.Rodrigues(R)
         p, _ = cv2.projectPoints(obj, rvec, t, Km, Dm)
         p = p.reshape(4, 2) + rng.normal(0.0, noise_px, (4, 2))

@@ -10,17 +10,20 @@ the binary oracle in this image is cv2 4.13.0 (`solve_cv2`).  `solve_ippe` resta
 published algorithm (Collins & Bartoli, "Infinitesimal Plane-based Pose Estimation", IJCV 2014,
 as implemented in OpenCV modules/calib3d/src/ippe.cpp and undistort.dispatch.cpp):
   1. undistortPoints: normalise with K, then exactly 5 fixed-point iterations of the
-     plumb-bob inverse (TermCriteria default count 5), result rounded to FP32 (the output
+     plumb-bob inverse (TermCriteria default count 5); a point whose icdist turns negative
+     stops at once with its initial guess, as OpenCV's does; result rounded to FP32 (the output
      array takes the Point2f input depth -- measured: without that rounding the restatement is
-     5e-6 off cv2, with it 6e-11);
+     5e-6 off cv2, with it 6e-11).  After the rounding it equals cv2.undistortPoints bit for bit
+     on every pixel grid of CAMERAS (tests/test_pnp_ref_cameras.py);
   2. canonical object frame (centred, planar, z = 0) -- constant per armor size;
   3. exact homography canonical plane -> normalised image from the 4 correspondences;
   4. IPPE: Jacobian of the homography at the origin -> two rotations; translation by linear LSQ;
   5. back to the model frame, order the two poses by reprojection RMSE in normalised
      coordinates, return the lower;
   6. rotation matrix -> rvec with IPPE's rot2vec (axis from the skew part, angle = acos).
-It is pinned against cv2.solvePnP on seeded quads in tests/test_oracle_cpu.py (<=1e-9 relative)
-and on the survey's known-answer vector (SURVEY.md section 8c).
+It is pinned against cv2.solvePnP on seeded quads in tests/test_oracle_cpu.py (<=1e-9 relative),
+on the survey's known-answer vector (SURVEY.md section 8c), and across CAMERAS x both armor sizes x
+both ENVELOPES x noise in tests/test_pnp_ref_cameras.py (rotation matrices and relative translations).
 
 Only tests/, __graft_entry__.smoke() and bench.py's CPU-baseline legs may import this module.
 """
@@ -35,6 +38,41 @@ D_DEFAULT = np.array([-0.405274, 0.126058, -0.026939, -0.006503, 0.0])
 # /root/reference/include/irmv_detection/pnp_solver.hpp:30-33 (mm)
 SMALL_W, SMALL_H, LARGE_W, LARGE_H = 135.0, 55.0, 225.0, 55.0
 
+# The cameras the pose stage is checked with: name -> (K[9], D[5], (width, height)).  Only "wide" takes
+# undistortPoints' icdist < 0 exit (pixels beyond ~500 px from its centre); tests/test_pnp_ref_cameras.py
+# pins which camera does.
+CAMERAS = {
+    "default": (K_DEFAULT, D_DEFAULT, (640, 480)),
+    "k3_tangential": (np.array([1200.0, 0.0, 640.0, 0.0, 1180.0, 512.0, 0.0, 0.0, 1.0]),
+                      np.array([-0.3, 0.15, 0.001, -0.002, -0.05]), (1280, 1024)),
+    "pincushion": (np.array([1200.0, 0.0, 640.0, 0.0, 1200.0, 512.0, 0.0, 0.0, 1.0]),
+                   np.array([0.25, 0.05, 0.0, 0.0, 0.01]), (1280, 1024)),
+    "strong_barrel": (np.array([1400.0, 0.0, 640.0, 0.0, 1400.0, 512.0, 0.0, 0.0, 1.0]),
+                      np.array([-0.45, 0.0, 0.0, 0.0, 0.0]), (1280, 1024)),
+    "wide": (np.array([800.0, 0.0, 640.0, 0.0, 800.0, 512.0, 0.0, 0.0, 1.0]),
+             np.array([-0.5, 0.0, 0.0, 0.0, 0.0]), (1280, 1024)),
+    "no_distortion": (np.array([1500.0, 0.0, 700.0, 0.0, 1500.0, 480.0, 0.0, 0.0, 1.0]), np.zeros(5), (1280, 1024)),
+    "anisotropic_offcentre": (np.array([1100.0, 0.0, 702.3, 0.0, 1045.7, 431.9, 0.0, 0.0, 1.0]),
+                              np.array([-0.21, 0.09, 0.0015, 0.0008, -0.02]), (1280, 1024)),
+    "telephoto": (np.array([3000.0, 0.0, 960.0, 0.0, 3000.0, 600.0, 0.0, 0.0, 1.0]),
+                  np.array([-0.08, 0.4, 0.0005, -0.0003, -1.2]), (1920, 1200)),
+}
+
+# Pose envelopes of synth.armor_quads: the survey's (its defaults) and a wide one -- grazing yaw, any roll,
+# 0.3-25 m, armor centres up to 2 % from the frame edge.
+ENVELOPES = {
+    "survey": {},
+    "wide": dict(dist=(0.3, 25.0), yaw=85.0, roll=180.0, margin=0.02),
+}
+
+
+def camera_quads(camera: str, n: int, seed: int, large: bool = False, envelope: str = "survey",
+                 noise_px: float = 0.5) -> np.ndarray:
+    """synth.armor_quads through CAMERAS[camera] on its own frame, poses drawn from ENVELOPES[envelope]."""
+    from irmv_detection_b200 import synth
+    K, D, (w, h) = CAMERAS[camera]
+    return synth.armor_quads(n, seed, noise_px, K, D, w, h, large=large, **ENVELOPES[envelope])
+
 
 def object_points(large: bool = False) -> np.ndarray:
     """/root/reference/src/pnp_solver.cpp:17-33: LB, LT, RT, RB; x forward, y left, z up (m)."""
@@ -43,25 +81,29 @@ def object_points(large: bool = False) -> np.ndarray:
     return np.array([[0, hy, -hz], [0, hy, hz], [0, -hy, hz], [0, -hy, -hz]], np.float64)
 
 
-def undistort_points(pts: np.ndarray, K=K_DEFAULT, D=D_DEFAULT, iters: int = 5) -> np.ndarray:
-    """pts f64[...,2] pixel -> normalised undistorted coordinates (cv::undistortPoints, no R/P)."""
+def undistort_points(pts: np.ndarray, K=K_DEFAULT, D=D_DEFAULT, iters: int = 5, with_stop: bool = False):
+    """pts f64[...,2] pixel -> normalised undistorted coordinates (cv::undistortPoints, no R/P).
+
+    Like OpenCV, a point whose icdist turns negative in an iteration (an iterate beyond the radius where the
+    radial polynomial can be inverted) leaves the loop at once and keeps its initial guess (x0, y0).
+    with_stop=True also returns the bool[...] mask of those points."""
     fx, fy, cx, cy = K[0], K[4], K[2], K[5]
     k1, k2, p1, p2, k3 = D[:5]
     x0 = (pts[..., 0] - cx) / fx
     y0 = (pts[..., 1] - cy) / fy
     x, y = x0.copy(), y0.copy()
+    stop = np.zeros(x0.shape, bool)
     for _ in range(iters):
         r2 = x * x + y * y
-        icdist = 1.0 / (1.0 + ((k3 * r2 + k2) * r2 + k1) * r2)
-        # OpenCV: a negative icdist aborts the iteration with the initial guess
-        bad = icdist < 0
+        with np.errstate(divide="ignore", invalid="ignore"):
+            icdist = 1.0 / (1.0 + ((k3 * r2 + k2) * r2 + k1) * r2)
+        stop |= icdist < 0
         dx = 2.0 * p1 * x * y + p2 * (r2 + 2.0 * x * x)
         dy = p1 * (r2 + 2.0 * y * y) + 2.0 * p2 * x * y
-        xn = (x0 - dx) * icdist
-        yn = (y0 - dy) * icdist
-        x = np.where(bad, x0, xn)
-        y = np.where(bad, y0, yn)
-    return np.stack((x, y), -1)
+        x = np.where(stop, x0, (x0 - dx) * icdist)
+        y = np.where(stop, y0, (y0 - dy) * icdist)
+    xy = np.stack((x, y), -1)
+    return (xy, stop) if with_stop else xy
 
 
 def _homography_rect_to_quad(a: float, b: float, q: np.ndarray) -> np.ndarray:
@@ -193,9 +235,10 @@ def rot2vec(R: np.ndarray) -> np.ndarray:
     return r
 
 
-def solve_ippe(img_pts: np.ndarray, K=K_DEFAULT, D=D_DEFAULT, large: bool = False,
-               both: bool = False):
-    """img_pts f32/f64[n,4,2] (LB,LT,RT,RB px) -> rvec f64[n,3], tvec f64[n,3]."""
+def ippe_solutions(img_pts: np.ndarray, K=K_DEFAULT, D=D_DEFAULT, large: bool = False) -> dict:
+    """Both IPPE poses of img_pts f32/f64[n,4,2] (LB,LT,RT,RB px), in OpenCV's order: the first is the one
+    cv::solvePnP returns.  Keys: R1, R2 f64[n,3,3] rotation matrices (model -> camera), r1, r2 their rvecs,
+    t1, t2 f64[n,3], e1, e2 f64[n] reprojection RMSE in normalised coordinates."""
     pts = np.asarray(img_pts, np.float32).astype(np.float64).reshape(-1, 4, 2)
     # cv::undistortPoints writes its result in the input depth (CV_32FC2 for Point2f input,
     # /root/reference/src/pnp_solver.cpp:37-44), so IPPE sees FP32-rounded normalised points.
@@ -217,15 +260,54 @@ def solve_ippe(img_pts: np.ndarray, K=K_DEFAULT, D=D_DEFAULT, large: bool = Fals
         sols.append((Rm, t, err))
     first = sols[0][2].astype(np.float32) < sols[1][2].astype(np.float32)   # OpenCV compares floats
     # OpenCV: if (err1 < err2) keep order else swap  (ties -> second)
-    R1 = np.where(first[:, None, None], sols[0][0], sols[1][0])
-    t1 = np.where(first[:, None], sols[0][1], sols[1][1])
+    out = {}
+    for k, (i, j) in (("1", (0, 1)), ("2", (1, 0))):
+        out["R" + k] = np.where(first[:, None, None], sols[i][0], sols[j][0])
+        out["t" + k] = np.where(first[:, None], sols[i][1], sols[j][1])
+        out["e" + k] = np.where(first, sols[i][2], sols[j][2])
+        out["r" + k] = rot2vec(out["R" + k])
+    return out
+
+
+def solve_ippe(img_pts: np.ndarray, K=K_DEFAULT, D=D_DEFAULT, large: bool = False,
+               both: bool = False):
+    """img_pts f32/f64[n,4,2] (LB,LT,RT,RB px) -> rvec f64[n,3], tvec f64[n,3]; both=True:
+    (r1, t1, r2, t2, e1, e2), see ippe_solutions."""
+    s = ippe_solutions(img_pts, K, D, large)
     if not both:
-        return rot2vec(R1), t1
-    R2 = np.where(first[:, None, None], sols[1][0], sols[0][0])
-    t2 = np.where(first[:, None], sols[1][1], sols[0][1])
-    e1 = np.where(first, sols[0][2], sols[1][2])
-    e2 = np.where(first, sols[1][2], sols[0][2])
-    return rot2vec(R1), t1, rot2vec(R2), t2, e1, e2
+        return s["r1"], s["t1"]
+    return s["r1"], s["t1"], s["r2"], s["t2"], s["e1"], s["e2"]
+
+
+def rotation_error(R: np.ndarray, R_ref: np.ndarray) -> np.ndarray:
+    """||R - R_ref||_F per pose (f64[n,3,3] each), scaled by sin(theta_ref) past a quarter turn: near a
+    half turn rot2vec (OpenCV's, the kernel's and ours) keeps only eps / sin(theta) of its precision, so
+    the Rodrigues matrix of a returned rvec fixes the rotation no better than that."""
+    d = np.linalg.norm(R - R_ref, axis=(1, 2))
+    c = np.clip((np.trace(R_ref, axis1=1, axis2=2) - 1.0) / 2.0, -1.0, 1.0)
+    return d * np.where(c < 0, np.sqrt(1.0 - c * c), 1.0)
+
+
+def tf2_quaternion(R: np.ndarray) -> np.ndarray:
+    """tf2::Matrix3x3::getRotation (x, y, z, w) of each R f64[n,3,3] (reference src/irm_detector.cpp:218-226)."""
+    out = np.empty((R.shape[0], 4))
+    for n, m in enumerate(R):
+        tr = m[0, 0] + m[1, 1] + m[2, 2]
+        q = np.zeros(4)
+        if tr > 0:
+            s = np.sqrt(tr + 1.0)
+            q[3] = s * 0.5
+            s = 0.5 / s
+            q[0], q[1], q[2] = (m[2, 1] - m[1, 2]) * s, (m[0, 2] - m[2, 0]) * s, (m[1, 0] - m[0, 1]) * s
+        else:
+            i = (2 if m[1, 1] < m[2, 2] else 1) if m[0, 0] < m[1, 1] else (2 if m[0, 0] < m[2, 2] else 0)
+            j, k = (i + 1) % 3, (i + 2) % 3
+            s = np.sqrt(m[i, i] - m[j, j] - m[k, k] + 1.0)
+            q[i] = s * 0.5
+            s = 0.5 / s
+            q[3], q[j], q[k] = (m[k, j] - m[j, k]) * s, (m[j, i] + m[i, j]) * s, (m[k, i] + m[i, k]) * s
+        out[n] = q
+    return out
 
 
 def solve_cv2(img_pts: np.ndarray, K=K_DEFAULT, D=D_DEFAULT, large: bool = False):
