@@ -291,12 +291,49 @@ int irmv_engine_set_raw_lut(irmv_engine *e, const uint8_t *lut);
  * The Bayer engine with matrix M and tone T on frames F returns what an otherwise identical IRMV_CH_PASSTHROUGH
  * engine without it returns on the packed frames T(M(demosaic(F))).  A saturation gain is one such matrix; with the
  * ISP order -- black level and gains in the raw table at gamma 1, then the matrix, then gamma in tone_lut -- the
- * engine reproduces the camera ISP's colour chain apart from auto white balance.  Non-zero (irmv_last_error) for a
+ * engine reproduces the camera ISP's colour chain (auto white balance: irmv_engine_set_auto_white_balance).  Non-zero (irmv_last_error) for a
  * packed RGB/BGR source (its ISP has already applied a matrix), for a tone table without a matrix, or while pipelined
  * batches are in flight.  Works for every raw_format.  The first non-NULL call allocates the device block, later
  * calls rewrite it in place (no allocation, the captured graphs stay); switching between off and on drops the
  * captured graphs. */
 int irmv_engine_set_color_matrix(irmv_engine *e, const int16_t m[9], const uint8_t *tone_lut);
+
+/* Automatic white balance for Bayer sources, per frame and stateless: the gains applied to a frame are a function of
+ * that frame alone (raw_lut.awb_statistics / awb_gains / awb_matrix are the definition).  The input is the 8-bit
+ * mosaic the demosaic reads (IRMV_RAW_8: after the raw table; 10/12-bit: the decoded mosaic), in sensor coordinates.
+ * Quad (i, j) covers rows 2i, 2i+1 and columns 2j, 2j+1 (i < H/2, j < W/2); it is clipped if a sample is > clip_level,
+ * else dark if a sample is < dark_level, else counted.  Over the counted quads SR = sum R, SG = sum (Gr + Gb),
+ * SB = sum B; with A = (2 SR, SG, 2 SB) the Q10 gains are g_c = min((1024 max(A) + A_c / 2) / A_c, gain_max_q10), so
+ * the brightest channel keeps 1024.  A frame with counted < min_quads or an empty channel keeps (1024, 1024, 1024)
+ * and valid = 0.  The gains are applied by the colour-correction stage: frame F is demosaiced with
+ *   M_F[r][k] = clamp_int16((M[r][k] * g_k + 512) >> 10)   (M = the set_color_matrix matrix, or 1024 * I)
+ * and the tone table T of set_color_matrix (or identity).  So set_color_matrix(M_F, T) with AWB off reproduces what
+ * AWB did to F exactly: fetch the gains, compose them and switch AWB off to lock the white balance.  ISP order: the
+ * raw table takes black level only, then AWB, then the matrix, then tone. */
+typedef struct irmv_awb_params {
+  int32_t dark_level;    /* quads with a sample below this are not counted (default 8)    */
+  int32_t clip_level;    /* quads with a sample above this are not counted (default 250)  */
+  int32_t min_quads;     /* fewer counted quads: gains 1, valid 0 (default 4096)          */
+  int32_t gain_max_q10;  /* upper clamp of every gain, >= 1024 (default 4096)             */
+} irmv_awb_params;
+typedef struct irmv_awb {            /* one per frame, what was applied to that frame */
+  uint64_t sum[3];                   /* SR, SG (both green sites), SB over counted quads */
+  uint32_t counted, dark, clipped;   /* quads; dark/clipped are what a host exposure loop needs */
+  int32_t valid;
+  int32_t gain_q10[3];
+  int32_t reserved;
+} irmv_awb;
+int irmv_awb_params_default(irmv_awb_params *p);
+/* p == NULL switches the stage off (the default).  Refused: a packed RGB/BGR source (returns 2), parameters outside
+ * 0 <= dark_level <= clip_level <= 255, min_quads >= 1, 1024 <= gain_max_q10 <= 32767 (returns 1), pipelined
+ * batches in flight (returns 5).  Every replay then runs one statistics kernel first and every kernel that demosaics
+ * the raw frame reads its frame's own block.  The first call that switches it on allocates; later calls rewrite the
+ * parameters in place (no allocation, the captured graphs stay), and so does a set_color_matrix update; switching
+ * between off and on drops the captured graphs.  Per-frame calls allocate nothing. */
+int irmv_engine_set_auto_white_balance(irmv_engine *e, const irmv_awb_params *p);
+/* out: nframes records of the last detect/detect_batch/sync (ticket < 0) or of a collected pipelined batch (its
+ * ticket).  An error with the stage off or for a call that ran without it. */
+int irmv_engine_fetch_white_balance(irmv_engine *e, int ticket, int nframes, irmv_awb *out);
 
 /* Pipelined hand-off for host-resident batches -- the B200 form of the overlap the reference gets
  * from its TripleBuffer (camera thread fills the next slot while detect() runs on the previous one,

@@ -40,6 +40,11 @@ class ArmorParams(C.Structure):
                 ("max_large_center_distance", C.c_double)]
 
 
+class AwbParams(C.Structure):
+    _fields_ = [("dark_level", C.c_int32), ("clip_level", C.c_int32), ("min_quads", C.c_int32),
+                ("gain_max_q10", C.c_int32)]
+
+
 class EngineConfig(C.Structure):
     _fields_ = [
         ("src_width", C.c_int32), ("src_height", C.c_int32), ("chan_order", C.c_int32),
@@ -91,6 +96,9 @@ SYMBOLS = {
     "irmv_engine_fetch_armors": (C.c_int, [_P, C.c_int, C.c_int, _P]),
     "irmv_engine_set_raw_lut": (C.c_int, [_P, _P]),
     "irmv_engine_set_color_matrix": (C.c_int, [_P, _P, _P]),
+    "irmv_awb_params_default": (C.c_int, [C.POINTER(AwbParams)]),
+    "irmv_engine_set_auto_white_balance": (C.c_int, [_P, C.POINTER(AwbParams)]),
+    "irmv_engine_fetch_white_balance": (C.c_int, [_P, C.c_int, C.c_int, _P]),
     "irmv_engine_profile_stages": (C.c_int, [_P, _P, C.c_int, C.POINTER(C.c_float * 5)]),
     "irmv_engine_submit_batch": (C.c_int, [_P, _P, C.c_int, C.POINTER(C.c_int)]),
     "irmv_engine_collect": (C.c_int, [_P, C.c_int, _P, _P, _P, _P, _P]),

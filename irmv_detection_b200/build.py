@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libirmv_b200.so")
-SOURCES = ["engine.cu", "preprocess.cu", "stem_bayer.cu", "conv_direct.cu", "conv_tc.cu", "conv_raster.cu", "dwconv.cu", "shuffle_unit.cu", "decode_nms.cu", "pnp.cu", "armors.cu", "raw_decode.cu"]
+SOURCES = ["engine.cu", "preprocess.cu", "stem_bayer.cu", "conv_direct.cu", "conv_tc.cu", "conv_raster.cu", "dwconv.cu", "shuffle_unit.cu", "decode_nms.cu", "pnp.cu", "armors.cu", "raw_decode.cu", "awb.cu"]
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
     "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr",

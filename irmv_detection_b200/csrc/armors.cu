@@ -600,8 +600,10 @@ __device__ __forceinline__ void roi_body(Shared &sh, const ArmorParams &p, uint3
 
 // LUT: Bayer frames with a raw-domain colour table; the table (1 KB) follows Shared in dynamic shared memory
 // and is visible after the barrier that precedes the first ROI.  CCM: Bayer frames with a colour-correction block
-// (kCcmBytes), staged behind the raw table's place the same way.
-template <bool LUT, bool CCM>
+// (kCcmBytes), staged behind the raw table's place the same way.  FRAME_CCM (with CCM): one block per frame
+// (p.ccm_stride, auto white balance), staged again before every ROI -- a separate instantiation, so that the
+// engine-wide one keeps its registers and spills.
+template <bool LUT, bool CCM, bool FRAME_CCM = false>
 __global__ void __launch_bounds__(kThreads, 3) extract_armors_kernel(ArmorParams p) {
   extern __shared__ __align__(16) uint8_t smem_raw[];
   Shared &sh = *reinterpret_cast<Shared *>(smem_raw);
@@ -609,7 +611,7 @@ __global__ void __launch_bounds__(kThreads, 3) extract_armors_kernel(ArmorParams
   uint8_t *ccm = lut + (LUT ? 1024 : 0);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   if (LUT) reinterpret_cast<uint32_t *>(lut)[tid] = reinterpret_cast<const uint32_t *>(p.raw_lut)[tid];   // kThreads == 256 words
-  if (CCM) stage_ccm(ccm, p.ccm, tid);
+  if (CCM && !FRAME_CCM) stage_ccm(ccm, p.ccm, tid);
   const int W = p.src_w, H = p.src_h;
   const bool bayer = p.chan_order >= 2;
   const size_t frame_bytes = (size_t)W * H * (bayer ? 1 : 3);
@@ -639,6 +641,8 @@ __global__ void __launch_bounds__(kThreads, 3) extract_armors_kernel(ArmorParams
     }
     const int words_roi = (rh + 2) * ((rw + 2 + 31) >> 5);
     const bool large = words_roi > kSmemWords || rh > kRows;
+    // the previous ROI is done with the block (barrier at the end of the loop), the barrier below publishes this one
+    if (FRAME_CCM) stage_ccm(ccm, p.ccm + (size_t)f * p.ccm_stride, tid);
     if (tid == 0) {
       sh.nbest = 0; sh.lock = 0; sh.slot = -1; sh.ncand = 0;
       if (large) sh.slot = blockIdx.x;   // this CTA's own global scratch slot
@@ -700,7 +704,8 @@ const char *armors_geometry_error(int src_w, int src_h) {
 
 cudaError_t launch_extract_armors(const ArmorParams &p, cudaStream_t s) {
   if ((p.raw_lut || p.ccm) && p.chan_order < 2) return cudaErrorInvalidValue;   // the tables are defined for Bayer sources only
-  auto kernel = p.ccm ? (p.raw_lut ? extract_armors_kernel<true, true> : extract_armors_kernel<false, true>)
+  auto kernel = p.ccm && p.ccm_stride ? (p.raw_lut ? extract_armors_kernel<true, true, true> : extract_armors_kernel<false, true, true>)
+              : p.ccm ? (p.raw_lut ? extract_armors_kernel<true, true> : extract_armors_kernel<false, true>)
                       : (p.raw_lut ? extract_armors_kernel<true, false> : extract_armors_kernel<false, false>);
   const size_t smem = sizeof(Shared) + (p.raw_lut ? 1024 : 0) + (p.ccm ? kCcmBytes : 0);
   {   // per device and cheap: no process-wide "already configured" flag (several engines / devices per process)

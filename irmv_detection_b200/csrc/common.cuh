@@ -63,6 +63,9 @@ struct PreprocessParams {
   // Colour-correction stage of a Bayer source (irmv_engine_set_color_matrix): a kCcmBytes device block (layout
   // below) applied to every demosaiced pixel, after the raw table and before rot180 / resize; null = off
   const uint8_t *ccm;
+  // Bytes between the colour-correction blocks of consecutive frames: 0 = one block for every frame (the user's
+  // matrix), kCcmBytes = one block per source frame (auto white balance, awb.cu); frame f reads ccm + f * ccm_stride
+  int ccm_stride;
 };
 // Device block of the colour-correction stage: int32 m[3][3] (row-major, units of 1/1024) at byte 0, u8 tone[3][256]
 // at byte kCcmTone.  A demosaiced pixel (R, G, B) becomes, per output channel c,
@@ -132,6 +135,35 @@ struct RawDecodeParams {
   int packed;                          // 1: 12-bit packed (src_w even)
 };
 cudaError_t launch_raw_decode(const RawDecodeParams &p, int num_sms, cudaStream_t s);
+
+// ---------------------------------------------------------------- auto white balance (awb.cu)
+// Per frame: statistics over the 2x2 quads of the 8-bit mosaic, grey-world gains, and the frame's colour-correction
+// block = the base block's matrix times diag(gains) plus its tone table (raw_lut.awb_statistics / awb_gains /
+// awb_matrix are the definition).
+struct AwbAcc {                        // per-frame accumulators; zero before a launch, left zero after it
+  unsigned long long sum[3];           // SR, SG (both green sites), SB over the counted quads
+  unsigned int counted, dark, clipped;
+  unsigned int ctas_done;              // CTAs of the frame that have added their sums
+};
+struct AwbRecord {                     // == irmv_awb (include/irmv_cabi.h, static_assert in engine.cu)
+  unsigned long long sum[3];
+  unsigned int counted, dark, clipped;
+  int valid;
+  int gain_q10[3];
+  int reserved;
+};
+struct AwbParams {
+  const uint8_t *src;                  // [n][H][W] 8-bit mosaics; used when src_indirect == null
+  const uint8_t *const *src_indirect;  // device word holding the frame base pointer (batch path)
+  int n, src_w, src_h, chan_order;
+  const uint8_t *raw_lut;              // [2][2][256] raw-domain colour table (PreprocessParams::raw_lut), or null
+  const int *cfg;                      // device {dark_level, clip_level, min_quads, gain_max_q10} (irmv_awb_params)
+  const uint8_t *base;                 // kCcmBytes block: the user's matrix and tone table, or the identity
+  AwbAcc *acc;                         // [n]
+  uint8_t *ccm;                        // [n][kCcmBytes] out: the block frame f is demosaiced with
+  AwbRecord *rec;                      // [n] out
+};
+cudaError_t launch_awb(const AwbParams &p, cudaStream_t s);
 
 // ---------------------------------------------------------------- convolution
 struct ConvSeg {
@@ -336,6 +368,7 @@ struct ArmorParams {
   unsigned long long *prof;             // debug: cycles summed over ROIs {bitmap, flood, walks, armor, rois, flood rounds}; null in production
   const uint8_t *raw_lut;               // [2][2][256] raw-domain colour stage of a Bayer source (PreprocessParams::raw_lut), or null
   const uint8_t *ccm;                   // colour-correction block of a Bayer source (PreprocessParams::ccm), or null
+  int ccm_stride;                       // PreprocessParams::ccm_stride
 };
 int armors_grid(int num_sms);
 // null when the stage takes src_w x src_h frames, else why not (checked where the stage is set up, not per launch)

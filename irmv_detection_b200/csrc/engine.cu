@@ -409,6 +409,12 @@ struct Lane {
   float *kpts = nullptr;                   // [S*max_det][8] decoded keypoints of the kept detections, network pixels
   ArmorOut *armors = nullptr;              // [S*max_det], allocated by irmv_engine_enable_armors
   uint32_t *armor_scratch = nullptr;       // per-CTA bitmaps of ROIs that do not fit in shared memory
+  // auto white balance (awb.cu), allocated by the first irmv_engine_set_auto_white_balance: per frame of a replay,
+  // the accumulators, the colour-correction block the frame is demosaiced with, and the record fetch_white_balance
+  // returns (copied to the result set beside, not inside, the result block)
+  AwbAcc *awb_acc = nullptr;               // [S]
+  uint8_t *awb_ccm = nullptr;              // [S][kCcmBytes]
+  AwbRecord *awb_rec = nullptr;            // [S]
   cudaEvent_t stage_ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
 };
 
@@ -528,6 +534,15 @@ static PnpConsts pnp_consts(const double K[9], const double D[5]) {
 
 constexpr int kSets = 3;    // batches in flight in the pipelined hand-off
 
+// Engine-wide device block of auto white balance.
+struct AwbDevice {
+  int cfg[4];                              // irmv_awb_params in AwbParams::cfg order
+  alignas(16) uint8_t identity[kCcmBytes]; // base block without a user matrix: 1024 * I, identity tone
+  AwbAcc acc;                              // refresh_rotated's single frame: accumulators, block and record
+  alignas(16) uint8_t ccm[kCcmBytes];
+  AwbRecord rec;
+};
+
 struct irmv_engine {
   irmv_engine_config cfg{};
   int nc = IRMV_NUM_CLASSES;
@@ -562,6 +577,8 @@ struct irmv_engine {
     int n = 0;
     long long ticket = -1;                // ticket whose results the set holds (-1: a synchronous call / nothing)
     bool in_flight = false;               // submitted and not yet collected
+    AwbRecord *awb_host = nullptr;        // pinned [max_batch] auto white balance records (allocated with the stage)
+    bool awb = false;                     // the set's call ran with auto white balance: awb_host holds its records
   } sets[kSets];
   cudaStream_t copy_stream = nullptr;
   long long next_ticket = 0;
@@ -574,6 +591,8 @@ struct irmv_engine {
   bool raw_lut_on = false;               // the kernels that read the raw frame apply d_raw_lut
   uint8_t *d_ccm = nullptr;              // colour-correction block (kCcmBytes, irmv_engine_set_color_matrix), allocated on first use
   bool ccm_on = false;                   // the kernels that demosaic the raw frame apply d_ccm
+  AwbDevice *d_awb = nullptr;            // auto white balance parameters and blocks (irmv_engine_set_auto_white_balance)
+  bool awb_on = false;                   // every replay measures each frame and demosaics it with its own block
   int raw_bits = 8;                      // bits per raw sample (cfg.raw_format); > 8: every replay decodes first
   uint8_t *d_decode_lut = nullptr;       // [2][2][1 << raw_bits] table of the decode kernel (raw_bits > 8), allocated at create
   uint8_t *slot8_dev = nullptr;          // decoded slot_dev, what refresh_rotated rotates (raw_bits > 8)
@@ -1027,6 +1046,18 @@ bool build_lane(irmv_engine *e, Lane &ln) {
   return true;
 }
 
+// Auto white balance of n 8-bit mosaics: the parameters, the raw table and the base block the gains compose with
+// (the user's colour-correction block, else the identity).  The caller sets the per-frame outputs.
+AwbParams awb_params(const irmv_engine *e, const uint8_t *src, const uint8_t *const *src_indirect, int n) {
+  AwbParams a{};
+  a.src = src; a.src_indirect = src_indirect;
+  a.n = n; a.src_w = e->cfg.src_width; a.src_h = e->cfg.src_height; a.chan_order = e->cfg.chan_order;
+  a.raw_lut = e->raw_lut_on ? e->d_raw_lut : nullptr;
+  a.cfg = e->d_awb->cfg;
+  a.base = e->ccm_on ? e->d_ccm : e->d_awb->identity;
+  return a;
+}
+
 // Enqueue one replay (n frames) of the whole pipeline on the lane stream.  With `stage_events`
 // the lane's events are recorded between stages (profiling pass, never inside a graph).
 int issue_replay(irmv_engine *e, Lane &ln, int n, cudaStream_t st, int *launches,
@@ -1056,13 +1087,20 @@ int issue_replay(irmv_engine *e, Lane &ln, int n, cudaStream_t st, int *launches
     IRMV_CUDA(launch_raw_decode(d, e->num_sms, st)); ++cnt;
     src = ln.raw8; src_indirect = nullptr;
   }
+  // auto white balance: each frame's gains and colour block, before anything demosaics it (preprocess stage too)
+  if (e->awb_on) {
+    AwbParams a = awb_params(e, src, src_indirect, n);
+    a.acc = ln.awb_acc; a.ccm = ln.awb_ccm; a.rec = ln.awb_rec;
+    IRMV_CUDA(launch_awb(a, st)); ++cnt;
+  }
   PreprocessParams pp{};
   pp.src = src; pp.src_indirect = src_indirect; pp.dst = ln.in8.p; pp.rotated = ln.rotated;
   pp.n = n; pp.src_w = e->cfg.src_width; pp.src_h = e->cfg.src_height; pp.frame0 = 0;
   pp.chan_order = e->cfg.chan_order; pp.rotate180 = e->cfg.rotate180;
   pp.resize_mode = e->cfg.resize_mode; pp.quantize_u8 = e->cfg.quantize_u8;
   pp.raw_lut = e->raw_lut_on ? e->d_raw_lut : nullptr;
-  pp.ccm = e->ccm_on ? e->d_ccm : nullptr;
+  pp.ccm = e->awb_on ? ln.awb_ccm : e->ccm_on ? e->d_ccm : nullptr;
+  pp.ccm_stride = e->awb_on ? kCcmBytes : 0;
   if (e->fused_stem) IRMV_CUDA(launch_stem(pp, e->d_stem_w, e->d_stem_b, e->d_stem_tab, ln.stem_out.pp ? nullptr : ln.stem_out.p, ln.stem_out.pstride, ln.stem_out.pp, ln.stem_out.pp_stride, st));
   else IRMV_CUDA(launch_preprocess(pp, st));
   cnt += 1 + (ln.rotated ? 1 : 0);
@@ -1161,7 +1199,7 @@ int issue_replay(irmv_engine *e, Lane &ln, int n, cudaStream_t st, int *launches
     ap.out = ln.armors; ap.slot_locks = reinterpret_cast<int *>(ln.armor_scratch); ap.scratch = ln.armor_scratch + 64;
     ap.scratch_words_per_cta = armors_scratch_words_per_cta(e->cfg.src_width, e->cfg.src_height);
     ap.grid = armors_grid(e->num_sms);
-    ap.raw_lut = pp.raw_lut; ap.ccm = pp.ccm;
+    ap.raw_lut = pp.raw_lut; ap.ccm = pp.ccm; ap.ccm_stride = pp.ccm_stride;
     IRMV_CUDA(launch_extract_armors(ap, st)); ++cnt;
     if (e->pnp_on) {
       const int total = n * e->cfg.max_det;
@@ -1269,7 +1307,12 @@ int enqueue(irmv_engine *e, const uint8_t *frames_dev, int n, const uint8_t *fra
       e->d2h_bytes += r.bytes;
       IRMV_CUDA(cudaMemcpyAsync(rs.res_host + r.host_off, ln.results + r.dev_off, r.bytes, cudaMemcpyDeviceToHost, ln.stream));
     }
+    if (e->awb_on) {                     // the auto white balance records live beside the result block (result_layout.h)
+      e->d2h_bytes += (size_t)nf * sizeof(AwbRecord);
+      IRMV_CUDA(cudaMemcpyAsync(rs.awb_host + f0, ln.awb_rec, (size_t)nf * sizeof(AwbRecord), cudaMemcpyDeviceToHost, ln.stream));
+    }
   }
+  rs.awb = e->awb_on;
   for (int l = 0; l < used; ++l) {
     IRMV_CUDA(cudaEventRecord(e->lanes[l].done, e->lanes[l].stream));
     IRMV_CUDA(cudaStreamWaitEvent(e->main_stream, e->lanes[l].done, 0));
@@ -1337,6 +1380,12 @@ int refresh_rotated(irmv_engine *e, int slot) {
   pp.rotate180 = e->cfg.rotate180;
   pp.raw_lut = e->raw_lut_on ? e->d_raw_lut : nullptr;
   pp.ccm = e->ccm_on ? e->d_ccm : nullptr;
+  if (e->awb_on) {   // the frame's gains again (a function of the frame alone): the lanes may hold another batch by now
+    AwbParams a = awb_params(e, pp.src, nullptr, 1);
+    a.acc = &e->d_awb->acc; a.ccm = e->d_awb->ccm; a.rec = &e->d_awb->rec;
+    IRMV_CUDA(launch_awb(a, e->main_stream));
+    pp.ccm = e->d_awb->ccm;
+  }
   IRMV_CUDA(launch_rotate(pp, e->main_stream));
   IRMV_CUDA(cudaMemcpyAsync(e->rot_host[slot], e->rot_dev, (size_t)e->cfg.src_width * e->cfg.src_height * 3,
                             cudaMemcpyDeviceToHost, e->main_stream));
@@ -1718,6 +1767,7 @@ void irmv_engine_destroy(irmv_engine *e) {
   cudaFree(e->d_stem_w); cudaFree(e->d_stem_b); cudaFree(e->d_stem_tab);
   if (e->d_raw_lut) cudaFree(e->d_raw_lut);
   if (e->d_ccm) cudaFree(e->d_ccm);
+  if (e->d_awb) cudaFree(e->d_awb);
   if (e->d_decode_lut) cudaFree(e->d_decode_lut);
   if (e->slot8_dev) cudaFree(e->slot8_dev);
   if (e->batch_dev) cudaFree(e->batch_dev);
@@ -1725,6 +1775,7 @@ void irmv_engine_destroy(irmv_engine *e) {
     if (e->sets[i].batch_dev) cudaFree(e->sets[i].batch_dev);
   for (auto &st : e->sets) {
     if (st.res_host) cudaFreeHost(st.res_host);
+    if (st.awb_host) cudaFreeHost(st.awb_host);
     if (st.done) cudaEventDestroy(st.done);
     for (auto ev : st.h2d) cudaEventDestroy(ev);
   }
@@ -1930,7 +1981,7 @@ int irmv_debug_stem_ctas(irmv_engine *e, int *ctas) {
   pp.chan_order = e->cfg.chan_order; pp.rotate180 = e->cfg.rotate180;
   pp.resize_mode = e->cfg.resize_mode; pp.quantize_u8 = e->cfg.quantize_u8;
   pp.raw_lut = e->raw_lut_on ? e->d_raw_lut : nullptr;
-  pp.ccm = e->ccm_on ? e->d_ccm : nullptr;
+  pp.ccm = e->awb_on ? e->lanes[0].awb_ccm : e->ccm_on ? e->d_ccm : nullptr;
   *ctas = e->fused_stem && e->d_stem_tab ? stem_bayer2x_ctas(pp) : 0;
   return 0;
   IRMV_ABI_CATCH
@@ -2050,17 +2101,22 @@ int irmv_engine_fetch_poses(irmv_engine *e, int nframes, double *rvecs, double *
   return 0;
 }
 
-// Result block of a finished call: ticket < 0 = the last synchronous call (set 0), else a collected
+// Result set of a finished call: ticket < 0 = the last synchronous call (set 0), else a collected
 // pipelined batch whose set has not been reused yet.
-static const uint8_t *result_block(irmv_engine *e, int ticket) {
+static const irmv_engine::Set *result_set(irmv_engine *e, int ticket) {
   if (ticket < 0) {
     if (e->sets[0].ticket != -1) { set_error("set 0 holds a pipelined batch: pass its ticket"); return nullptr; }
-    return e->sets[0].res_host;
+    return &e->sets[0];
   }
   const irmv_engine::Set &rs = e->sets[ticket % kSets];
   if (!rs.res_host || rs.ticket != ticket) { set_error("this ticket's results are gone (never submitted, or its result set was reused)"); return nullptr; }
   if (rs.in_flight) { set_error("collect the ticket first"); return nullptr; }
-  return rs.res_host;
+  return &rs;
+}
+
+static const uint8_t *result_block(irmv_engine *e, int ticket) {
+  const irmv_engine::Set *rs = result_set(e, ticket);
+  return rs ? rs->res_host : nullptr;
 }
 
 static_assert(sizeof(irmv_pose) == 88, "irmv_pose layout");
@@ -2199,6 +2255,78 @@ int irmv_engine_set_color_matrix(irmv_engine *e, const int16_t *m, const uint8_t
     }
     e->ccm_on = on;
   }
+  return 0;
+}
+
+int irmv_awb_params_default(irmv_awb_params *p) {
+  if (!p) return 1;
+  p->dark_level = 8; p->clip_level = 250; p->min_quads = 4096; p->gain_max_q10 = 4096;
+  return 0;
+}
+
+static_assert(sizeof(AwbRecord) == sizeof(irmv_awb) && sizeof(irmv_awb) == 56, "AwbRecord mirrors irmv_awb");
+
+// The parameters live in one device block (AwbDevice) with the identity base block and refresh_rotated's single-frame
+// buffers; each lane gets its per-frame accumulators, blocks and records, and each result set a pinned record array.
+// All of it is allocated by the first call that switches the stage on; later calls rewrite the parameters in place
+// after the engine's queued work has finished, and the graphs read them through their captured pointer.
+int irmv_engine_set_auto_white_balance(irmv_engine *e, const irmv_awb_params *p) {
+  if (!e) { set_error("bad argument"); return 1; }
+  if (e->cfg.chan_order < IRMV_CH_BAYER_RGGB || e->cfg.chan_order > IRMV_CH_BAYER_GBRG) {
+    set_error("irmv_engine_set_auto_white_balance: auto white balance applies to Bayer sources only");
+    return 2;
+  }
+  if (p && !(0 <= p->dark_level && p->dark_level <= p->clip_level && p->clip_level <= 255 && p->min_quads >= 1 &&
+             p->gain_max_q10 >= 1024 && p->gain_max_q10 <= 32767)) {
+    set_error("irmv_engine_set_auto_white_balance: needs 0 <= dark_level <= clip_level <= 255, min_quads >= 1 and "
+              "1024 <= gain_max_q10 <= 32767");
+    return 1;
+  }
+  if (pipeline_busy(e)) return 5;
+  IRMV_CUDA(cudaSetDevice(e->cfg.device));
+  IRMV_CUDA(cudaDeviceSynchronize());
+  const bool on = p != nullptr;
+  if (on) {
+    if (!e->d_awb) {
+      IRMV_CUDA(dev_malloc((void **)&e->d_awb, sizeof(AwbDevice)));
+      IRMV_CUDA(cudaMemset(e->d_awb, 0, sizeof(AwbDevice)));
+      uint8_t ident[kCcmBytes] = {};
+      const int32_t m32[9] = {1024, 0, 0, 0, 1024, 0, 0, 0, 1024};
+      memcpy(ident, m32, sizeof m32);
+      for (int i = 0; i < 3 * 256; ++i) ident[kCcmTone + i] = (uint8_t)(i & 255);
+      IRMV_CUDA(cudaMemcpy(e->d_awb->identity, ident, kCcmBytes, cudaMemcpyHostToDevice));
+    }
+    const size_t S = (size_t)e->S;
+    for (auto &ln : e->lanes)             // (lane_alloc zeroes: the accumulators start at zero)
+      if ((!ln.awb_acc && !lane_alloc(ln, (void **)&ln.awb_acc, S * sizeof(AwbAcc))) ||
+          (!ln.awb_ccm && !lane_alloc(ln, (void **)&ln.awb_ccm, S * kCcmBytes)) ||
+          (!ln.awb_rec && !lane_alloc(ln, (void **)&ln.awb_rec, S * sizeof(AwbRecord))))
+        return 3;
+    for (auto &st : e->sets)
+      if (!st.awb_host) {
+        IRMV_CUDA(host_malloc((void **)&st.awb_host, (size_t)e->cfg.max_batch * sizeof(AwbRecord)));
+        memset(st.awb_host, 0, (size_t)e->cfg.max_batch * sizeof(AwbRecord));
+      }
+    const int32_t cfg[4] = {p->dark_level, p->clip_level, p->min_quads, p->gain_max_q10};
+    IRMV_CUDA(cudaMemcpy(e->d_awb->cfg, cfg, sizeof cfg, cudaMemcpyHostToDevice));
+  }
+  if (on != e->awb_on) {
+    for (auto &ln : e->lanes) {           // the kernels the replay launches changed: drop captured graphs
+      for (auto &g : ln.graphs) cudaGraphExecDestroy(g.second);
+      ln.graphs.clear();
+    }
+    e->awb_on = on;
+  }
+  return 0;
+}
+
+int irmv_engine_fetch_white_balance(irmv_engine *e, int ticket, int nframes, irmv_awb *out) {
+  if (!e || !out || nframes < 1 || nframes > e->cfg.max_batch) { set_error("bad argument"); return 1; }
+  if (!e->awb_on) { set_error("auto white balance not enabled"); return 2; }
+  const irmv_engine::Set *rs = result_set(e, ticket);
+  if (!rs) return 2;
+  if (!rs->awb) { set_error("this call ran without auto white balance"); return 2; }
+  memcpy(out, rs->awb_host, (size_t)nframes * sizeof(irmv_awb));
   return 0;
 }
 

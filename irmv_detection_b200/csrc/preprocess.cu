@@ -235,14 +235,14 @@ __device__ __forceinline__ void apply_raw_lut(const Region &r, const uint8_t *__
 }
 
 // LUT: Bayer source with a raw-domain colour table (p.raw_lut).  CCM: Bayer source with a colour-correction block
-// (p.ccm), staged behind the source window (rows_cap * pitch_s bytes)
+// (p.ccm; the frame's own block when p.ccm_stride is set), staged behind the source window (rows_cap * pitch_s bytes)
 template <bool LUT, bool CCM>
 __global__ void __launch_bounds__(NT)
 preprocess_kernel(PreprocessParams p, int rows_cap, int pitch_s) {
   extern __shared__ __align__(16) uint8_t smem[];
   uint8_t *ccm = smem + (size_t)rows_cap * pitch_s;
-  if (CCM) stage_ccm(ccm, p.ccm, threadIdx.x);
   const int n = blockIdx.z;
+  if (CCM) stage_ccm(ccm, p.ccm + (size_t)(p.frame0 + n) * p.ccm_stride, threadIdx.x);
   const int oy0 = blockIdx.y * TH, ox0 = blockIdx.x * TW;
   const bool bayer = p.chan_order >= 2;
   const int bpp = bayer ? 1 : 3;
@@ -314,7 +314,7 @@ stem_kernel(PreprocessParams p, const float *__restrict__ w, const float *__rest
             long long out_pstride, __half *out2, long long out2_pstride, int pitch_s, int fast_x, int smem_win) {
   extern __shared__ __align__(16) uint8_t smem[];
   uint8_t *ccm = smem + smem_win;
-  if (CCM) stage_ccm(ccm, p.ccm, threadIdx.x);
+  if (CCM) stage_ccm(ccm, p.ccm + (size_t)(p.frame0 + blockIdx.z) * p.ccm_stride, threadIdx.x);
   __shared__ __half tile[3][SI][SI + 1];             // network-input tile, already rounded to FP16
   __shared__ uint32_t sbf[16][16];                   // conv0 weights as half2 {w[n][2j], w[n][2j+1]}, K padded to 32
   __shared__ float sbias[16];
@@ -569,7 +569,7 @@ __global__ void rotate_kernel(PreprocessParams p) {
         R = on_red_row ? horiz : vert;
         B = on_red_row ? vert : horiz;
       }
-      if (CCM) apply_ccm(p.ccm, R, G, B);
+      if (CCM) apply_ccm(p.ccm + (size_t)(p.frame0 + n) * p.ccm_stride, R, G, B);
       (void)reg;
     } else {
       const uint8_t *s = frame + ((size_t)sy * W + sx) * 3;

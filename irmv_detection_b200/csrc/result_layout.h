@@ -7,6 +7,10 @@
 namespace irmv {
 
 // In memory order.  Each field is `frames` consecutive per-frame arrays.
+// The auto white balance record (irmv_awb, one per frame, not per detection) is deliberately not a field: every
+// field but kNum scales with max_det, and with the stage off the copy plans must stay what they are.  It lives in its
+// own per-lane device array and per-set pinned array beside this block, copied by one extra cudaMemcpyAsync per
+// replay or chunk only while the stage is on (engine.cu, enqueue).
 enum ResultField { kNum, kBoxes, kScores, kClasses, kIndex, kRvec, kTvec, kOk, kArmors, kKpts, kQuat, kDist, kNumResultFields };
 
 struct ResultFieldSpec { size_t frame_fixed, per_det, align; };   // bytes per frame = frame_fixed + per_det * max_det

@@ -60,6 +60,7 @@ struct StemBayerArgs {
   __half *out2; long long out2_ps;       // parity-split twin (may be null)
   const uint8_t *raw_lut;                // [2][2][256] raw-domain colour stage (PreprocessParams::raw_lut), LUT instantiations only
   const uint8_t *ccm;                    // colour-correction block (PreprocessParams::ccm), LUT == LUT_COLOUR only
+  int ccm_stride;                        // PreprocessParams::ccm_stride
 };
 
 // Table modes of the Bayer instantiations (template parameter LUT): no table, the raw table, the raw table (when one
@@ -158,7 +159,7 @@ __global__ void __launch_bounds__(NTHREADS, 2) stem_bayer2x_kernel(const __grid_
   }
   const bool raw_lut = LUT == LUT_RAW || (LUT == LUT_COLOUR && a.raw_lut);
   if (raw_lut && tid < 256) reinterpret_cast<uint32_t *>(rlut)[tid] = reinterpret_cast<const uint32_t *>(a.raw_lut)[tid];
-  if (LUT == LUT_COLOUR) stage_ccm(ccm, a.ccm, tid);
+  if (LUT == LUT_COLOUR) stage_ccm(ccm, a.ccm + (size_t)(a.frame0 + n) * a.ccm_stride, tid);
   if (tid < NIR) {
     reinterpret_cast<uint4 *>(rowtab)[tid] = reinterpret_cast<const uint4 *>(strip + 4)[tid];
     // conv padding of the tile: column 0 (ix = -1) and the pad half behind the last pixel
@@ -578,7 +579,7 @@ cudaError_t launch_stem_bayer2x(const PreprocessParams &p, int frame0, const uin
   a.Q = Q; a.lut_n = 2 * Q * 255 + Q + 1;
   a.tab_strip = TAB_LUT + (a.lut_n + 7) / 8 * 4;
   a.tab = tab; a.out = out; a.out_ps = out_ps; a.out2 = out2; a.out2_ps = out2_ps;
-  a.raw_lut = p.raw_lut; a.ccm = p.ccm;
+  a.raw_lut = p.raw_lut; a.ccm = p.ccm; a.ccm_stride = p.ccm_stride;
   const size_t smem = smem_for(p.src_h, fmt);
   if (smem + lut_bytes(lut_mode(p)) > kMaxSmem) return cudaErrorInvalidValue;
   return p.rotate180 ? launch_f<true>(fmt, a, smem, s) : launch_f<false>(fmt, a, smem, s);

@@ -307,6 +307,29 @@ class YoloEngine:
             tp = tone.ctypes.data
         L.check(self._lib.irmv_engine_set_color_matrix(self._h, mp, tp), "irmv_engine_set_color_matrix")
 
+    def set_auto_white_balance(self, params: Optional[dict] = None) -> None:
+        """Automatic white balance of a Bayer engine, per frame: `params` is None (off, the default) or a dict
+        overriding raw_lut.AWB_DEFAULTS (dark_level, clip_level, min_quads, gain_max_q10).  Every frame is then
+        demosaiced with the colour-correction matrix raw_lut.awb_matrix(g, M) and the tone table T of
+        set_color_matrix (M = 1024 * I and identity tone when none is set), g = raw_lut.awb_gains of
+        raw_lut.awb_statistics of the frame's 8-bit mosaic.  fetch_white_balance returns what was applied; with AWB
+        off, set_color_matrix(raw_lut.awb_matrix(g, M), T) reproduces it exactly (locks the white balance)."""
+        if params is None:
+            L.check(self._lib.irmv_engine_set_auto_white_balance(self._h, None), "irmv_engine_set_auto_white_balance")
+            return
+        from . import raw_lut as R
+        p = R.awb_params(params)
+        prm = L.AwbParams(p["dark_level"], p["clip_level"], p["min_quads"], p["gain_max_q10"])
+        L.check(self._lib.irmv_engine_set_auto_white_balance(self._h, C.byref(prm)), "irmv_engine_set_auto_white_balance")
+
+    def fetch_white_balance(self, n: int, ticket: int = -1) -> np.ndarray:
+        """Auto white balance records of the last synchronous call (or of a collected ticket): structured AWB_DTYPE
+        [n] (sum = SR, SG, SB over the counted quads; counted, dark, clipped quads; valid; gain_q10)."""
+        out = np.zeros(n, AWB_DTYPE)
+        L.check(self._lib.irmv_engine_fetch_white_balance(self._h, ticket, n, out.ctypes.data),
+                "irmv_engine_fetch_white_balance")
+        return out
+
     def fetch_armors(self, n: int, ticket: int = -1) -> np.ndarray:
         """Armors of the last synchronous call (or of a collected ticket): structured [n, max_det]."""
         out = np.zeros((n, self.max_det), ARMOR_DTYPE)
@@ -472,6 +495,8 @@ ARMOR_DTYPE = np.dtype([("pts", np.float32, (4, 2)), ("center", np.float32, 2), 
                         ("class_id", np.int32), ("size", np.int32), ("valid", np.int32)])
 POSE_DTYPE = np.dtype([("position", np.float64, 3), ("orientation", np.float64, 4), ("rvec", np.float64, 3),
                        ("distance_to_image_center", np.float32), ("ok", np.int32)])
+AWB_DTYPE = np.dtype([("sum", np.uint64, 3), ("counted", np.uint32), ("dark", np.uint32), ("clipped", np.uint32),
+                      ("valid", np.int32), ("gain_q10", np.int32, 3), ("reserved", np.int32)])   # == irmv_awb
 BBOX_DTYPE = np.dtype([("xyxy", np.float32, 4), ("score", np.float32), ("class_id", np.int32)])
 
 

@@ -12,6 +12,10 @@ returns on decode_raw(F, raw_format, T, pattern).
 apply_color_matrix is the definition of the colour-correction stage that follows the demosaic (set_color_matrix):
 a 3x3 integer matrix and an output tone table; color_matrix_q10 builds the matrix from a colour-correction matrix and
 a saturation gain.
+
+awb_statistics, awb_gains and awb_matrix are the definition of automatic white balance (set_auto_white_balance):
+per frame, grey-world gains from the unclipped, not-too-dark 2x2 quads of the 8-bit mosaic, applied as a diagonal
+matrix composed with the colour-correction stage's matrix.
 """
 from __future__ import annotations
 
@@ -170,3 +174,86 @@ def _check_tone(tone) -> Optional[np.ndarray]:
     if tone.shape != (3, 256) or tone.dtype != np.uint8:
         raise ValueError("the tone table must be a (3, 256) uint8 array or None")
     return tone
+
+
+# Automatic white balance (YoloEngine.set_auto_white_balance, irmv_engine_set_auto_white_balance, irmv_awb_params)
+AWB_DEFAULTS = {"dark_level": 8, "clip_level": 250, "min_quads": 4096, "gain_max_q10": 4096}
+
+
+def awb_params(params: Optional[dict] = None) -> dict:
+    """AWB_DEFAULTS updated with `params`, checked as the engine checks them: 0 <= dark_level <= clip_level <= 255,
+    min_quads >= 1, 1024 <= gain_max_q10 <= 32767."""
+    p = dict(AWB_DEFAULTS)
+    if params:
+        unknown = set(params) - set(p)
+        if unknown:
+            raise ValueError(f"unknown auto white balance parameters: {sorted(unknown)}")
+        p.update({k: int(v) for k, v in params.items()})
+    if not 0 <= p["dark_level"] <= p["clip_level"] <= 255:
+        raise ValueError("auto white balance needs 0 <= dark_level <= clip_level <= 255")
+    if p["min_quads"] < 1:
+        raise ValueError("auto white balance needs min_quads >= 1")
+    if not 1024 <= p["gain_max_q10"] <= 32767:
+        raise ValueError("auto white balance needs 1024 <= gain_max_q10 <= 32767")
+    return p
+
+
+def awb_statistics(mosaic8: np.ndarray, pattern: int, params: Optional[dict] = None) -> dict:
+    """Statistics of one frame.  mosaic8 is the u8 [H, W] mosaic the demosaic reads (RAW_8: after the raw table when
+    one is set, apply_raw_lut; 10/12-bit: decode_raw), in sensor coordinates (before rot180).  Quad (i, j) covers rows
+    2i, 2i + 1 and columns 2j, 2j + 1 (i < H // 2, j < W // 2: an odd last row or column is not used); its samples are
+    R, Gr, Gb, B under `pattern`.  A quad is clipped if a sample is > clip_level, else dark if a sample is
+    < dark_level, else counted.  Returns {"sum": (SR, SG, SB), "counted", "dark", "clipped"}: SR = sum of R,
+    SG = sum of Gr + Gb, SB = sum of B over the counted quads (Python ints)."""
+    p = awb_params(params)
+    m = np.asarray(mosaic8)
+    if m.dtype != np.uint8 or m.ndim != 2:
+        raise ValueError("mosaic8 must be a uint8 [H, W] mosaic")
+    h2, w2 = m.shape[0] // 2, m.shape[1] // 2
+    q = m[:2 * h2, :2 * w2].reshape(h2, 2, w2, 2).astype(np.int64)
+    s = [[q[:, py, :, px] for px in range(2)] for py in range(2)]
+    ry, rx = RED_SITE[pattern]
+    r, b = s[ry][rx], s[1 - ry][1 - rx]
+    g = s[ry][1 - rx] + s[1 - ry][rx]
+    hi = np.maximum(np.maximum(s[0][0], s[0][1]), np.maximum(s[1][0], s[1][1]))
+    lo = np.minimum(np.minimum(s[0][0], s[0][1]), np.minimum(s[1][0], s[1][1]))
+    clipped = hi > p["clip_level"]
+    dark = ~clipped & (lo < p["dark_level"])
+    counted = ~clipped & ~dark
+    return {"sum": (int(r[counted].sum()), int(g[counted].sum()), int(b[counted].sum())),
+            "counted": int(counted.sum()), "dark": int(dark.sum()), "clipped": int(clipped.sum())}
+
+
+def awb_gains(stats: dict, params: Optional[dict] = None) -> tuple:
+    """Q10 gains (gR, gG, gB) and validity of a frame from its statistics.  With the comparable channel sums
+    A = (2 SR, SG, 2 SB) and Amax = max(A): g_c = min((1024 Amax + A_c // 2) // A_c, gain_max_q10), so the brightest
+    channel gets exactly 1024 and no gain is below 1024.  A frame with fewer than min_quads counted quads or an
+    empty channel is invalid: gains (1024, 1024, 1024).  Returns ((gR, gG, gB), valid)."""
+    p = awb_params(params)
+    sr, sg, sb = (int(v) for v in stats["sum"])
+    a = (2 * sr, sg, 2 * sb)
+    if stats["counted"] < p["min_quads"] or min(a) == 0:
+        return (1024, 1024, 1024), False
+    amax = max(a)
+    return tuple(min((1024 * amax + c // 2) // c, p["gain_max_q10"]) for c in a), True
+
+
+def awb_matrix(gains: Sequence[int], m: Optional[np.ndarray] = None) -> np.ndarray:
+    """int16 [3, 3] matrix the colour-correction stage applies to a frame with AWB gains g under the user's matrix m
+    (None: 1024 * I): M_F[r][k] = clamp_int16((m[r][k] * g_k + 512) >> 10) (arithmetic shift).  With AWB off,
+    set_color_matrix(awb_matrix(g, m), tone) reproduces exactly what AWB with gains g produced: that locks the white
+    balance."""
+    mm = (1024 * np.eye(3)).astype(np.int16) if m is None else _check_matrix(m)
+    g = np.asarray(gains, np.int64)
+    if g.shape != (3,):
+        raise ValueError("gains must be three Q10 integers")
+    v = (mm.astype(np.int64) * g[None, :] + 512) >> 10
+    return np.clip(v, -32768, 32767).astype(np.int16)
+
+
+def awb_record(mosaic8: np.ndarray, pattern: int, params: Optional[dict] = None) -> dict:
+    """What the engine reports for one frame (irmv_awb, YoloEngine.fetch_white_balance): the statistics of
+    awb_statistics, the gains of awb_gains and their validity."""
+    st = awb_statistics(mosaic8, pattern, params)
+    g, valid = awb_gains(st, params)
+    return {**st, "valid": int(valid), "gain_q10": g}
